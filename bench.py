@@ -2,6 +2,7 @@
 """bench.py — MUrB all-pairs gravity hot path on B200: billion body-interactions/s (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--bodies n] [--scheme galaxy|random]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one computeOneIteration(): the N^2 force pass + the MUrB integrator (+ the position all-gather for N > 1),
@@ -13,6 +14,9 @@ i.e. one iteration of `murb -n <bodies> -i <steps> --nv --im gpu+b200 --gf`.
 public C-ABI with pinned HOST buffers: upload (H2D) + step + download (D2H) inside the timed region, every step.
 `--impl reference` times the reference's own CPU path (cpu+omp, compiled from /root/reference into oracle/_ref) on the
 host cores: on the configuration itself when it finishes in ~25 s (n = 200 000 does), else on a bounded sample of it.
+`--dump-outputs DIR` writes what the last timed step computed, as float32 DIR/<name>.npy: the state a caller receives
+(qx qy qz vx vy vz after the step) and the accelerations of its force pass (ax ay az).  The inputs are the seeded
+reference generator's, so two builds run with the same arguments can be compared array for array.
 
 Outside the timed region every line also carries: `parity` (a force pass on the final positions checked against the fp64
 all-pairs oracle on targets straddling every slice boundary), and on one GPU `roofline_1m` (the N = 1 000 000 force
@@ -378,6 +382,33 @@ def parity_check(b200nb, ctx, bodies, n, world, rank, scheme):
     return out
 
 
+DUMP_NAMES = ("qx", "qy", "qz", "vx", "vy", "vz", "ax", "ay", "az")
+DUMP_MAX_BODIES = 1 << 20   # 9 float32 arrays of 2^20 bodies: 36 MiB, under the 64 MiB a dump may take
+
+
+def dump_sample(n):
+    """Bodies --dump-outputs writes: all of them up to DUMP_MAX_BODIES, else a fixed seeded sample (sorted, the same in
+    every run with the same n)."""
+    if n <= DUMP_MAX_BODIES:
+        return None
+    return np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_BODIES, replace=False))
+
+
+def outputs_of_last_step(ctx, n):
+    """The state after the last step and the accelerations of that step's force pass (downloads are collective)."""
+    state = ctx.download_state()
+    out = {k: state[k] for k in ("qx", "qy", "qz", "vx", "vy", "vz")}
+    out.update(zip(("ax", "ay", "az"), ctx.download_accel()))
+    idx = dump_sample(n)
+    return {k: out[k] if idx is None else out[k][idx] for k in DUMP_NAMES}
+
+
+def write_outputs(path, arrays):
+    os.makedirs(path, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), np.ascontiguousarray(v, dtype=np.float32))
+
+
 def timed_steps_single_gpu(b200nb, scheme, n, steps, warmup):
     """`steps` flushed, event-timed computeOneIteration() of an n-body system on the current device (one GPU)."""
     names = ("qx", "qy", "qz", "m", "vx", "vy", "vz")
@@ -523,6 +554,10 @@ def run_b200_arm(args, rank, world, local_rank):
     launches = ctx.launch_count - launches0
     force_ms, force_launches = ctx.profile_get()
     ctx.profile_enable(False)
+    if args.dump_outputs:
+        last = outputs_of_last_step(ctx, n)
+        if rank == 0:
+            write_outputs(args.dump_outputs, last)
     dev_ms = reduce_max(dev_ms)
     force_ms = reduce_max(force_ms)
     interactions_per_step = float(n) * float(n)
@@ -654,7 +689,12 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-scaling-base", action="store_true", help="skip the 1-GPU run of the strong-scaling workload")
     ap.add_argument("--no-side-legs", action="store_true", help="skip roofline_1m and prior_art (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the state and accelerations of the last timed step as float32 DIR/<name>.npy "
+                         f"(a fixed seeded sample of {DUMP_MAX_BODIES} bodies above that size)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the GPU path computed: use it with --impl b200")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -667,6 +707,8 @@ def main():
         args.bodies = 200000 if args.gpus <= 1 else STRONG_SCALING_BODIES
     if args.steps is None:
         args.steps = 200 if args.gpus <= 1 else 5
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference_arm(args, rank, world)

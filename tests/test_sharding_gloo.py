@@ -23,7 +23,8 @@ def _free_port():
 def _worker(rank, world, port, n, steps, out_dir):
     sys.path.insert(0, os.path.join(REPO, "nbody-eurohpc_b200"))
     sys.path.insert(0, os.path.join(REPO, "tests"))
-    os.environ.update(RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(rank), MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
+    os.environ.update(RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(rank), MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port),
+                      CUDA_VISIBLE_DEVICES="")  # a CPU-only job: ranks must not bind GPUs, which a host may have fewer of
     from b200nb import dist as bdist, slice_length
     d = bdist.init_process_group("gloo")
     token = bdist.broadcast_bytes(d, bytes(range(128)) if rank == 0 else None)
