@@ -135,6 +135,30 @@ enum {
 };
 int b200nb_metrics(b200nb_ctx *ctx, double *out);
 
+/* ---- the gravitational field ----------------------------------------------------------------------------------
+ * The reference has no counterpart: it only ever asks for the acceleration of each body.  Same G, softening and G*m
+ * fold as the force pass:
+ *   field at a point p, over ALL bodies:  a(p) = sum_j G m_j (q_j - p) / (|q_j - p|^2 + soft^2)^(3/2),
+ *                                         phi(p) = -sum_j G m_j / (|q_j - p|^2 + soft^2)^(1/2);
+ *   per-body potential, self pair excluded by INDEX (a body at the same position as another still counts it):
+ *                                         phi_i = -sum_{j != i} G m_j / (|r_ij|^2 + soft^2)^(1/2),
+ * so b200nb_energy == sum_i m_i |v_i|^2 / 2 + (1/2) sum_i m_i phi_i, and the density-centre weight of b200nb_metrics is
+ * w_i = -m_i phi_i.  fp32 pair terms, hierarchical sums finished in fp64 (same accuracy design as the force pass).
+ * A result depends only on its point (or body) and the current bodies: bit-identical whatever the other points of
+ * the call, their number, the shard or rank count, and on reruns.  Neither call changes the simulation state
+ * (positions, velocities, the accelerations of b200nb_download_accel, the leapfrog's stored a(x_n), cached step graphs);
+ * both are ordered after a preceding asynchronous b200nb_step and join the devices before returning.  Device scratch is
+ * bounded (points go through in fixed-size batches), grow-only, owned by the context and counted in
+ * b200nb_allocated_bytes. */
+
+/* Acceleration and potential at n_points arbitrary points (host SoA).  Any output pointer may be NULL.  Joins the
+ * devices.  Collective when n_ranks > 1: every rank passes the same points and receives every result.
+ * n_points == 0 is a no-op; NULL point arrays otherwise give B200NB_EINVAL; B200NB_ESTATE before an upload. */
+int b200nb_field(b200nb_ctx *ctx, uint64_t n_points, const float *px, const float *py, const float *pz,
+                 float *ax, float *ay, float *az, float *phi);
+/* Per-body potential of the current positions, self pair excluded, all n_bodies values.  Collective when n_ranks > 1. */
+int b200nb_potential(b200nb_ctx *ctx, float *phi);
+
 /* Joins every device and communication stream.  main.cpp:353-371 only synchronises the current device, so the glue
  * calls this when more than one device is in use. */
 int b200nb_sync(b200nb_ctx *ctx);

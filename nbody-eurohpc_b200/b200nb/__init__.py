@@ -77,6 +77,8 @@ def lib() -> ctypes.CDLL:
         "b200nb_integrate_host_accel": (c_int, [ctx, _FP, _FP, _FP, c_float]),
         "b200nb_energy": (c_int, [ctx, POINTER(c_double)]),
         "b200nb_metrics": (c_int, [ctx, POINTER(c_double)]),
+        "b200nb_field": (c_int, [ctx, c_uint64] + [_FP] * 7),
+        "b200nb_potential": (c_int, [ctx, _FP]),
         "b200nb_sync": (c_int, [ctx]),
         "b200nb_n_bodies": (c_uint64, [ctx]),
         "b200nb_n_local_gpus": (c_int, [ctx]),
@@ -298,6 +300,23 @@ class Context:
         out = (c_double * len(self.METRIC_NAMES))()
         self._check(self._L.b200nb_metrics(self._ctx, out), "b200nb_metrics")
         return dict(zip(self.METRIC_NAMES, list(out)))
+
+    def field(self, px, py, pz) -> tuple[np.ndarray, np.ndarray, np.ndarray, np.ndarray]:
+        """Acceleration and potential at arbitrary points, summed over every body (include/b200nb.h: b200nb_field).
+        px, py, pz: 1-D arrays of equal length.  Returns (ax, ay, az, phi), float32."""
+        p = [_f32(a) for a in (px, py, pz)]
+        if any(a.ndim != 1 for a in p) or len({a.shape for a in p}) != 1:
+            raise ValueError(f"expected three 1-D arrays of equal length, got {[a.shape for a in p]}")
+        m = p[0].shape[0]
+        out = [np.empty(m, dtype=np.float32) for _ in range(4)]
+        self._check(self._L.b200nb_field(self._ctx, m, *[_p(a) for a in p], *[_p(a) for a in out]), "b200nb_field")
+        return out[0], out[1], out[2], out[3]
+
+    def potential(self) -> np.ndarray:
+        """Per-body potential phi_i, self pair excluded (include/b200nb.h: b200nb_potential).  float32[n]."""
+        phi = np.empty(self.n, dtype=np.float32)
+        self._check(self._L.b200nb_potential(self._ctx, _p(phi)), "b200nb_potential")
+        return phi
 
     def sync(self):
         self._check(self._L.b200nb_sync(self._ctx), "b200nb_sync")

@@ -20,6 +20,7 @@
 #include <vector>
 
 #include "../../include/b200nb.h"
+#include "field_sm100.cuh"
 #include "integrate_sm100.cuh"
 #include "plan.hpp"
 // The default force-kernel variant once more, as a cubin whose hot loop has been re-ordered after ptxas by
@@ -155,6 +156,11 @@ struct Shard {
     float *stage_full = nullptr; // one rank per process only: 3 x stage_stride floats for a full-system position download (lazy)
     double *energy_blocks = nullptr, *energy_out = nullptr;
     void *l2_scratch = nullptr;
+    // field / potential scratch (grow-only): [S][4][cap] partial rows | [3][cap] points | [4][cap] results, and with one
+    // rank per process [n_ranks][4][cap] gathered results.  cap = targets per launch.
+    float *field_buf = nullptr;
+    uint32_t field_cap = 0;
+    uint64_t field_bytes = 0;
     ncclComm_t comm = nullptr;
     CUmodule resched_mod = nullptr;   // the re-ordered cubin of the default variant on this device (nullptr: not in use)
     CUfunction resched_fn = nullptr;
@@ -885,7 +891,7 @@ void b200nb_destroy(b200nb_ctx *c)
         for (auto e : s.prof) cudaEventDestroy(e);
         for (auto e : s.prof_free) cudaEventDestroy(e);
         cudaFree(s.bodies); cudaFree(s.bodies_next); cudaFree(s.vel); cudaFree(s.acc); cudaFree(s.mass); cudaFree(s.partial); cudaFree(s.stage); cudaFree(s.stage_full);
-        cudaFree(s.energy_blocks); cudaFree(s.energy_out); cudaFree(s.l2_scratch);
+        cudaFree(s.energy_blocks); cudaFree(s.energy_out); cudaFree(s.l2_scratch); cudaFree(s.field_buf);
         for (auto t : s.timer) if (t) cudaEventDestroy(t);
         if (s.ev_integrated) cudaEventDestroy(s.ev_integrated);
         if (s.ev_gathered) cudaEventDestroy(s.ev_gathered);
@@ -1215,6 +1221,118 @@ int b200nb_metrics(b200nb_ctx *c, double *out)
         out[B200NB_METRIC_DENSITY_X + k] = raw[MR_W] != 0.0 ? raw[MR_WX + k] / raw[MR_W] : out[B200NB_METRIC_COM_X + k];
     }
     return B200NB_OK;
+}
+
+// Grow-only scratch of the field / potential path, sized for `cap` targets per launch.
+static int field_scratch(b200nb_ctx *c, Shard &s, uint32_t cap)
+{
+    if (s.field_cap >= cap) return B200NB_OK;
+    const bool gather = c->shards.size() != (size_t)c->n_ranks;
+    const size_t floats = ((size_t)field_chunks(c->n) * 4 + 3 + 4 + (gather ? 4 * (size_t)c->n_ranks : 0)) * cap;
+    CU(c, cudaSetDevice(s.device));
+    if (s.field_buf) {
+        CU(c, cudaFree(s.field_buf));
+        s.field_buf = nullptr;
+        s.bytes -= s.field_bytes;
+        s.field_cap = 0;
+        s.field_bytes = 0;
+    }
+    CU(c, cudaMalloc((void **)&s.field_buf, floats * 4));
+    s.field_cap = cap;
+    s.field_bytes = floats * 4;
+    s.bytes += s.field_bytes;
+    return B200NB_OK;
+}
+
+// Field at points (self == false) or potential of every body (self == true).  The targets are cut into one contiguous
+// range of Q per rank (points: ceil(M / n_ranks); bodies: the rank's slice) and each range into launches of at most
+// `cap` targets.  In-process shards copy their results straight to the host.  With one rank per process every rank runs
+// the same number of rounds and each round's results are all-gathered, the way download_sliced gathers accelerations.
+// Reads only the body array and writes only the field scratch: the simulation state and cached step graphs are untouched.
+static int field_run(b200nb_ctx *c, bool self, uint64_t m, const float *const pts[3], float *const out[4])
+{
+    DeviceGuard guard;
+    const bool gather = c->shards.size() != (size_t)c->n_ranks;
+    const uint64_t Q = self ? c->L : (m + c->n_ranks - 1) / c->n_ranks;
+    const uint32_t cap = (uint32_t)std::min<uint64_t>(FIELD_BATCH, (Q + FIELD_TI - 1) / FIELD_TI * FIELD_TI);
+    const uint64_t rounds = (Q + cap - 1) / cap;
+    const uint32_t S = field_chunks(c->n);
+    const size_t P = cap;
+    for (auto &s : c->shards) {
+        if (int rc = field_scratch(c, s, cap)) return rc;
+        CU(c, cudaSetDevice(s.device));
+        // an asynchronous step may still be exchanging positions: the whole body array is read
+        if (c->n_ranks > 1)
+            if (int rc = wait_remote_positions(c, s)) return rc;
+        float *partial = s.field_buf, *dpts = partial + (size_t)S * 4 * P, *dout = dpts + 3 * P, *dgat = dout + 4 * P;
+        const uint64_t lo = (uint64_t)s.rank * Q;
+        const uint64_t hi = self ? lo + s.n_local : std::min<uint64_t>(lo + Q, m);
+        for (uint64_t r = 0; r < rounds; ++r) {
+            const uint64_t base = lo + r * cap;
+            const uint32_t cnt = base < hi ? (uint32_t)std::min<uint64_t>(cap, hi - base) : 0u;
+            if (cnt == 0 && !gather) break;
+            if (cnt > 0) {
+                FieldArgs a{};
+                a.src = s.bodies;
+                a.partial = partial;
+                a.stride = cap;
+                a.count = cnt;
+                a.src_nblk = (uint32_t)((c->n + BLK - 1) / BLK);
+                a.n_chunks = S;
+                a.soft2 = c->soft2;
+                const dim3 grid((cnt + FIELD_TI - 1) / FIELD_TI, S);
+                if (self) {
+                    a.self0 = base; // a multiple of BLK: slices and batches are
+                    field_kernel<true><<<grid, FIELD_THREADS, field_smem_bytes(), s.s_compute>>>(a);
+                } else {
+                    for (int k = 0; k < 3; ++k)
+                        CU(c, cudaMemcpyAsync(dpts + k * P, pts[k] + base, (size_t)cnt * 4, cudaMemcpyHostToDevice, s.s_compute));
+                    a.px = dpts; a.py = dpts + P; a.pz = dpts + 2 * P;
+                    field_kernel<false><<<grid, FIELD_THREADS, field_smem_bytes(), s.s_compute>>>(a);
+                }
+                field_reduce_kernel<<<(cnt + 255) / 256, 256, 0, s.s_compute>>>(partial, S, cap, cnt, dout);
+                c->launches += 2;
+                CU(c, cudaGetLastError());
+            }
+            if (!gather) {
+                for (int q = 0; q < 4; ++q)
+                    if (out[q]) CU(c, cudaMemcpyAsync(out[q] + base, dout + q * P, (size_t)cnt * 4, cudaMemcpyDeviceToHost, s.s_compute));
+                continue;
+            }
+            NC(c, g_nccl.AllGather(dout, dgat, 4 * P, ncclFloat, s.comm, s.s_compute));
+            for (int rk = 0; rk < c->n_ranks; ++rk) {
+                const uint64_t rb = (uint64_t)rk * Q + r * cap;
+                const uint64_t rhi = std::min<uint64_t>((uint64_t)rk * Q + Q, self ? c->n : m);
+                if (rb >= rhi) continue;
+                const size_t rcnt = (size_t)std::min<uint64_t>(cap, rhi - rb);
+                for (int q = 0; q < 4; ++q)
+                    if (out[q])
+                        CU(c, cudaMemcpyAsync(out[q] + rb, dgat + ((size_t)rk * 4 + q) * P, rcnt * 4, cudaMemcpyDeviceToHost, s.s_compute));
+            }
+        }
+    }
+    return sync_all(c);
+}
+
+int b200nb_field(b200nb_ctx *c, uint64_t n_points, const float *px, const float *py, const float *pz, float *ax, float *ay,
+                 float *az, float *phi)
+{
+    if (!c) return B200NB_EINVAL;
+    if (!c->uploaded) return fail(c, B200NB_ESTATE, "field before upload");
+    if (n_points == 0) return B200NB_OK;
+    if (!px || !py || !pz) return fail(c, B200NB_EINVAL, "field: NULL point array");
+    const float *pts[3] = {px, py, pz};
+    float *out[4] = {ax, ay, az, phi};
+    return field_run(c, false, n_points, pts, out);
+}
+
+int b200nb_potential(b200nb_ctx *c, float *phi)
+{
+    if (!c) return B200NB_EINVAL;
+    if (!c->uploaded) return fail(c, B200NB_ESTATE, "potential before upload");
+    if (!phi) return fail(c, B200NB_EINVAL, "potential: phi is NULL");
+    float *out[4] = {nullptr, nullptr, nullptr, phi};
+    return field_run(c, true, c->n, nullptr, out);
 }
 
 int b200nb_sync(b200nb_ctx *c)
