@@ -159,6 +159,34 @@ int b200nb_field(b200nb_ctx *ctx, uint64_t n_points, const float *px, const floa
 /* Per-body potential of the current positions, self pair excluded, all n_bodies values.  Collective when n_ranks > 1. */
 int b200nb_potential(b200nb_ctx *ctx, float *phi);
 
+/* ---- nearest neighbours ---------------------------------------------------------------------------------------
+ * The k nearest bodies of every body, or of arbitrary points (close encounters, bound pairs, Casertano-Hut densities
+ * from the 6th neighbour, nearest-distance time-step criteria).  The reference has no counterpart.  Definition, for a
+ * target p and a body j at q_j (fp32, round to nearest, no softening, no flush to zero):
+ *   dx = xj - px, dy = yj - py, dz = zj - pz;   d2 = dx*dx;  d2 = fmaf(dy, dy, d2);  d2 = fmaf(dz, dz, d2);
+ * Candidates are ordered by the key (d2, j) lexicographically, a strict total order, so the k smallest keys are unique
+ * and the result is a pure function of the fp32 positions: it does not depend on batching, shard or rank count, and
+ * the answer for k is the first k columns of the answer for any larger k.  Reported distance: sqrtf(d2), correctly
+ * rounded.  Bodies mode excludes the self pair by INDEX (a coincident body is a neighbour at distance 0); points mode
+ * takes every body (a point on a body has it at distance 0).  Mass plays no part: zero-mass bodies are neighbours too.
+ * Padding bodies (index >= n_bodies) are never candidates.  Slots that cannot be filled (k > n_bodies - 1 for bodies,
+ * k > n_bodies for points) hold idx = 0xFFFFFFFF, dist = +inf.  d2 overflows to +inf for separations above ~1.8e19 m
+ * (the force pass forms the same fp32 d2, so the library already assumes smaller systems); such pairs still come in
+ * (d2, j) order, after every finite one.  Bodies at non-finite positions are never neighbours.
+ * k ranges over [1, 32].  Same calling contract as the field section: ordered after a preceding asynchronous
+ * b200nb_step, joins the devices, collective when n_ranks > 1 (every rank receives every row), no change to the
+ * simulation state.  Device scratch is grow-only, owned by the context, counted in b200nb_allocated_bytes and bounded
+ * independently of n_bodies and n_points: each launch's batch is sized from k so that its candidate rows stay within
+ * 2^23 entries (64 MiB); with the staged points and result rows it stays within 84 MiB per GPU, plus 16 MiB per rank
+ * for the gathered rows when each rank is its own process.  Errors: B200NB_ESTATE before an upload, B200NB_EINVAL for k outside
+ * [1, 32] or NULL point arrays. */
+
+/* k nearest other bodies of every body; idx/dist are [n_bodies][k] row-major; either may be NULL. */
+int b200nb_neighbors(b200nb_ctx *ctx, uint32_t k, uint32_t *idx, float *dist);
+/* k nearest bodies of n_points arbitrary points (host SoA); outputs [n_points][k].  n_points == 0 is a no-op. */
+int b200nb_neighbors_at(b200nb_ctx *ctx, uint64_t n_points, const float *px, const float *py, const float *pz,
+                        uint32_t k, uint32_t *idx, float *dist);
+
 /* Joins every device and communication stream.  main.cpp:353-371 only synchronises the current device, so the glue
  * calls this when more than one device is in use. */
 int b200nb_sync(b200nb_ctx *ctx);

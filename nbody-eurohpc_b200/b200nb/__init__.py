@@ -28,6 +28,7 @@ G_F32 = np.float32(6.67384e-11)  # SimulationNBodyInterface.hpp:18 (a float lite
 INTEGRATOR_MURB, INTEGRATOR_LEAPFROG = 0, 1
 OK, EINVAL, ECUDA, ENCCL, ESTATE = 0, 1, 2, 3, 4
 _FP = POINTER(c_float)
+_UP = POINTER(c_uint)
 
 
 class B200Error(RuntimeError):
@@ -79,6 +80,8 @@ def lib() -> ctypes.CDLL:
         "b200nb_metrics": (c_int, [ctx, POINTER(c_double)]),
         "b200nb_field": (c_int, [ctx, c_uint64] + [_FP] * 7),
         "b200nb_potential": (c_int, [ctx, _FP]),
+        "b200nb_neighbors": (c_int, [ctx, c_uint, _UP, _FP]),
+        "b200nb_neighbors_at": (c_int, [ctx, c_uint64, _FP, _FP, _FP, c_uint, _UP, _FP]),
         "b200nb_sync": (c_int, [ctx]),
         "b200nb_n_bodies": (c_uint64, [ctx]),
         "b200nb_n_local_gpus": (c_int, [ctx]),
@@ -317,6 +320,36 @@ class Context:
         phi = np.empty(self.n, dtype=np.float32)
         self._check(self._L.b200nb_potential(self._ctx, _p(phi)), "b200nb_potential")
         return phi
+
+    NEIGHBORS_K_MAX = 32
+
+    def _k(self, k) -> int:
+        if isinstance(k, bool) or not isinstance(k, (int, np.integer)) or not 1 <= int(k) <= self.NEIGHBORS_K_MAX:
+            raise ValueError(f"k must be an integer in [1, {self.NEIGHBORS_K_MAX}], got {k!r}")
+        return int(k)
+
+    def neighbors(self, k) -> tuple[np.ndarray, np.ndarray]:
+        """k nearest other bodies of every body (include/b200nb.h: b200nb_neighbors).  Returns (idx uint32[n, k],
+        dist float32[n, k]), each row sorted by (distance, index); empty slots are (0xFFFFFFFF, inf)."""
+        k = self._k(k)
+        idx = np.empty((self.n, k), dtype=np.uint32)
+        dist = np.empty((self.n, k), dtype=np.float32)
+        self._check(self._L.b200nb_neighbors(self._ctx, k, idx.ctypes.data_as(_UP), _p(dist)), "b200nb_neighbors")
+        return idx, dist
+
+    def neighbors_at(self, px, py, pz, k) -> tuple[np.ndarray, np.ndarray]:
+        """k nearest bodies of arbitrary points (include/b200nb.h: b200nb_neighbors_at).  px, py, pz: 1-D arrays of equal
+        length m.  Returns (idx uint32[m, k], dist float32[m, k])."""
+        k = self._k(k)
+        p = [_f32(a) for a in (px, py, pz)]
+        if any(a.ndim != 1 for a in p) or len({a.shape for a in p}) != 1:
+            raise ValueError(f"expected three 1-D arrays of equal length, got {[a.shape for a in p]}")
+        m = p[0].shape[0]
+        idx = np.empty((m, k), dtype=np.uint32)
+        dist = np.empty((m, k), dtype=np.float32)
+        self._check(self._L.b200nb_neighbors_at(self._ctx, m, *[_p(a) for a in p], k, idx.ctypes.data_as(_UP), _p(dist)),
+                    "b200nb_neighbors_at")
+        return idx, dist
 
     def sync(self):
         self._check(self._L.b200nb_sync(self._ctx), "b200nb_sync")

@@ -21,6 +21,7 @@
 
 #include "../../include/b200nb.h"
 #include "field_sm100.cuh"
+#include "neighbors_sm100.cuh"
 #include "integrate_sm100.cuh"
 #include "plan.hpp"
 // The default force-kernel variant once more, as a cubin whose hot loop has been re-ordered after ptxas by
@@ -156,11 +157,9 @@ struct Shard {
     float *stage_full = nullptr; // one rank per process only: 3 x stage_stride floats for a full-system position download (lazy)
     double *energy_blocks = nullptr, *energy_out = nullptr;
     void *l2_scratch = nullptr;
-    // field / potential scratch (grow-only): [S][4][cap] partial rows | [3][cap] points | [4][cap] results, and with one
-    // rank per process [n_ranks][4][cap] gathered results.  cap = targets per launch.
-    float *field_buf = nullptr;
-    uint32_t field_cap = 0;
-    uint64_t field_bytes = 0;
+    // scratch of the field / potential / neighbours calls (grow-only, laid out by run_targets)
+    unsigned char *query_buf = nullptr;
+    uint64_t query_bytes = 0;
     ncclComm_t comm = nullptr;
     CUmodule resched_mod = nullptr;   // the re-ordered cubin of the default variant on this device (nullptr: not in use)
     CUfunction resched_fn = nullptr;
@@ -812,6 +811,112 @@ int download_sliced(b200nb_ctx *c, float *Shard::*field, float *hx, float *hy, f
     return B200NB_OK;
 }
 
+// Grow-only scratch of the field / potential / neighbours calls.
+int query_scratch(b200nb_ctx *c, Shard &s, size_t bytes)
+{
+    if (s.query_bytes >= bytes) return B200NB_OK;
+    CU(c, cudaSetDevice(s.device));
+    if (s.query_buf) {
+        CU(c, cudaFree(s.query_buf));
+        s.query_buf = nullptr;
+        s.bytes -= s.query_bytes;
+        s.query_bytes = 0;
+    }
+    CU(c, cudaMalloc((void **)&s.query_buf, bytes));
+    s.query_bytes = bytes;
+    s.bytes += bytes;
+    return B200NB_OK;
+}
+
+// One result of run_targets: `bytes` per target, written to host rows (host == nullptr: not copied back).
+struct TargetOut {
+    void *host;
+    size_t bytes;
+};
+
+// Targets are the points (self == false, m of them) or every body (self == true).  They are cut into one contiguous
+// range of Q per rank (points: ceil(m / n_ranks); bodies: the rank's slice) and each range into launches of at most
+// `cap` targets, cap = min(batch, Q rounded up to whole tiles).  In-process shards copy their results straight to the
+// host.  With one rank per process every rank runs the same number of rounds and each round's results are all-gathered,
+// the way download_sliced gathers accelerations.
+// Scratch per shard: work_bytes(cap) | [3][cap] points | the outputs' [cap] rows one after another | with one rank per
+// process, n_ranks copies of those rows.  launch(s, base, cnt, cap, work, dpts, dout) enqueues on s.s_compute what
+// leaves the results of targets base + [0, cnt) in dout.
+// Reads only the body array and writes only this scratch: the simulation state and cached step graphs are untouched.
+template <class Work, class Launch>
+int run_targets(b200nb_ctx *c, bool self, uint64_t m, const float *const pts[3], uint32_t tile, uint32_t batch,
+                       const std::vector<TargetOut> &out, Work work_bytes, Launch launch)
+{
+    DeviceGuard guard;
+    const bool gather = c->shards.size() != (size_t)c->n_ranks;
+    const uint64_t Q = self ? c->L : (m + c->n_ranks - 1) / c->n_ranks;
+    const uint32_t cap = (uint32_t)std::min<uint64_t>(batch, (Q + tile - 1) / tile * tile);
+    const uint64_t rounds = (Q + cap - 1) / cap;
+    const size_t P = cap;
+    size_t row_bytes = 0; // all outputs of one target
+    for (auto &o : out) row_bytes += o.bytes;
+    const size_t work = work_bytes(cap);
+    for (auto &s : c->shards) {
+        if (int rc = query_scratch(c, s, work + 3 * 4 * P + (1 + (gather ? c->n_ranks : 0)) * row_bytes * P)) return rc;
+        CU(c, cudaSetDevice(s.device));
+        // an asynchronous step may still be exchanging positions: the whole body array is read
+        if (c->n_ranks > 1)
+            if (int rc = wait_remote_positions(c, s)) return rc;
+        float *dpts = reinterpret_cast<float *>(s.query_buf + work);
+        unsigned char *dout = reinterpret_cast<unsigned char *>(dpts + 3 * P), *dgat = dout + row_bytes * P;
+        const uint64_t lo = (uint64_t)s.rank * Q;
+        const uint64_t hi = self ? lo + s.n_local : std::min<uint64_t>(lo + Q, m);
+        for (uint64_t r = 0; r < rounds; ++r) {
+            const uint64_t base = lo + r * cap;
+            const uint32_t cnt = base < hi ? (uint32_t)std::min<uint64_t>(cap, hi - base) : 0u;
+            if (cnt == 0 && !gather) break;
+            if (cnt > 0) {
+                if (!self)
+                    for (int k = 0; k < 3; ++k)
+                        CU(c, cudaMemcpyAsync(dpts + k * P, pts[k] + base, (size_t)cnt * 4, cudaMemcpyHostToDevice, s.s_compute));
+                if (int rc = launch(s, base, cnt, cap, s.query_buf, dpts, dout)) return rc;
+                CU(c, cudaGetLastError());
+            }
+            if (!gather) {
+                size_t off = 0;
+                for (auto &o : out) {
+                    if (o.host)
+                        CU(c, cudaMemcpyAsync(static_cast<unsigned char *>(o.host) + base * o.bytes, dout + off * P, cnt * o.bytes,
+                                              cudaMemcpyDeviceToHost, s.s_compute));
+                    off += o.bytes;
+                }
+                continue;
+            }
+            NC(c, g_nccl.AllGather(dout, dgat, row_bytes / 4 * P, ncclFloat, s.comm, s.s_compute));
+            for (int rk = 0; rk < c->n_ranks; ++rk) {
+                const uint64_t rb = (uint64_t)rk * Q + r * cap;
+                const uint64_t rhi = std::min<uint64_t>((uint64_t)rk * Q + Q, self ? c->n : m);
+                if (rb >= rhi) continue;
+                const size_t rcnt = (size_t)std::min<uint64_t>(cap, rhi - rb);
+                size_t off = 0;
+                for (auto &o : out) {
+                    if (o.host)
+                        CU(c, cudaMemcpyAsync(static_cast<unsigned char *>(o.host) + rb * o.bytes, dgat + (rk * row_bytes + off) * P,
+                                              rcnt * o.bytes, cudaMemcpyDeviceToHost, s.s_compute));
+                    off += o.bytes;
+                }
+            }
+        }
+    }
+    return sync_all(c);
+}
+
+template <int KB>
+void nb_launch(bool self, const NbArgs &a, uint32_t k, uint32_t *idx, float *dist, cudaStream_t st)
+{
+    const dim3 grid((a.count + nb_tile(KB) - 1) / nb_tile(KB), a.n_chunks);
+    if (self)
+        neighbors_kernel<KB, true><<<grid, NB_THREADS, nb_smem_bytes(), st>>>(a);
+    else
+        neighbors_kernel<KB, false><<<grid, NB_THREADS, nb_smem_bytes(), st>>>(a);
+    nb_merge_kernel<KB><<<(a.count + 127) / 128, 128, 0, st>>>(a.cd2, a.cidx, a.n_chunks, a.stride, a.count, k, idx, dist);
+}
+
 } // namespace
 
 // =================================================================================================== C ABI
@@ -891,7 +996,7 @@ void b200nb_destroy(b200nb_ctx *c)
         for (auto e : s.prof) cudaEventDestroy(e);
         for (auto e : s.prof_free) cudaEventDestroy(e);
         cudaFree(s.bodies); cudaFree(s.bodies_next); cudaFree(s.vel); cudaFree(s.acc); cudaFree(s.mass); cudaFree(s.partial); cudaFree(s.stage); cudaFree(s.stage_full);
-        cudaFree(s.energy_blocks); cudaFree(s.energy_out); cudaFree(s.l2_scratch); cudaFree(s.field_buf);
+        cudaFree(s.energy_blocks); cudaFree(s.energy_out); cudaFree(s.l2_scratch); cudaFree(s.query_buf);
         for (auto t : s.timer) if (t) cudaEventDestroy(t);
         if (s.ev_integrated) cudaEventDestroy(s.ev_integrated);
         if (s.ev_gathered) cudaEventDestroy(s.ev_gathered);
@@ -1223,95 +1328,37 @@ int b200nb_metrics(b200nb_ctx *c, double *out)
     return B200NB_OK;
 }
 
-// Grow-only scratch of the field / potential path, sized for `cap` targets per launch.
-static int field_scratch(b200nb_ctx *c, Shard &s, uint32_t cap)
-{
-    if (s.field_cap >= cap) return B200NB_OK;
-    const bool gather = c->shards.size() != (size_t)c->n_ranks;
-    const size_t floats = ((size_t)field_chunks(c->n) * 4 + 3 + 4 + (gather ? 4 * (size_t)c->n_ranks : 0)) * cap;
-    CU(c, cudaSetDevice(s.device));
-    if (s.field_buf) {
-        CU(c, cudaFree(s.field_buf));
-        s.field_buf = nullptr;
-        s.bytes -= s.field_bytes;
-        s.field_cap = 0;
-        s.field_bytes = 0;
-    }
-    CU(c, cudaMalloc((void **)&s.field_buf, floats * 4));
-    s.field_cap = cap;
-    s.field_bytes = floats * 4;
-    s.bytes += s.field_bytes;
-    return B200NB_OK;
-}
-
-// Field at points (self == false) or potential of every body (self == true).  The targets are cut into one contiguous
-// range of Q per rank (points: ceil(M / n_ranks); bodies: the rank's slice) and each range into launches of at most
-// `cap` targets.  In-process shards copy their results straight to the host.  With one rank per process every rank runs
-// the same number of rounds and each round's results are all-gathered, the way download_sliced gathers accelerations.
-// Reads only the body array and writes only the field scratch: the simulation state and cached step graphs are untouched.
+// Field at points (self == false) or potential of every body (self == true): [S][4][cap] partial rows, summed into
+// four [cap] rows (ax, ay, az, phi).
 static int field_run(b200nb_ctx *c, bool self, uint64_t m, const float *const pts[3], float *const out[4])
 {
-    DeviceGuard guard;
-    const bool gather = c->shards.size() != (size_t)c->n_ranks;
-    const uint64_t Q = self ? c->L : (m + c->n_ranks - 1) / c->n_ranks;
-    const uint32_t cap = (uint32_t)std::min<uint64_t>(FIELD_BATCH, (Q + FIELD_TI - 1) / FIELD_TI * FIELD_TI);
-    const uint64_t rounds = (Q + cap - 1) / cap;
     const uint32_t S = field_chunks(c->n);
-    const size_t P = cap;
-    for (auto &s : c->shards) {
-        if (int rc = field_scratch(c, s, cap)) return rc;
-        CU(c, cudaSetDevice(s.device));
-        // an asynchronous step may still be exchanging positions: the whole body array is read
-        if (c->n_ranks > 1)
-            if (int rc = wait_remote_positions(c, s)) return rc;
-        float *partial = s.field_buf, *dpts = partial + (size_t)S * 4 * P, *dout = dpts + 3 * P, *dgat = dout + 4 * P;
-        const uint64_t lo = (uint64_t)s.rank * Q;
-        const uint64_t hi = self ? lo + s.n_local : std::min<uint64_t>(lo + Q, m);
-        for (uint64_t r = 0; r < rounds; ++r) {
-            const uint64_t base = lo + r * cap;
-            const uint32_t cnt = base < hi ? (uint32_t)std::min<uint64_t>(cap, hi - base) : 0u;
-            if (cnt == 0 && !gather) break;
-            if (cnt > 0) {
-                FieldArgs a{};
-                a.src = s.bodies;
-                a.partial = partial;
-                a.stride = cap;
-                a.count = cnt;
-                a.src_nblk = (uint32_t)((c->n + BLK - 1) / BLK);
-                a.n_chunks = S;
-                a.soft2 = c->soft2;
-                const dim3 grid((cnt + FIELD_TI - 1) / FIELD_TI, S);
-                if (self) {
-                    a.self0 = base; // a multiple of BLK: slices and batches are
-                    field_kernel<true><<<grid, FIELD_THREADS, field_smem_bytes(), s.s_compute>>>(a);
-                } else {
-                    for (int k = 0; k < 3; ++k)
-                        CU(c, cudaMemcpyAsync(dpts + k * P, pts[k] + base, (size_t)cnt * 4, cudaMemcpyHostToDevice, s.s_compute));
-                    a.px = dpts; a.py = dpts + P; a.pz = dpts + 2 * P;
-                    field_kernel<false><<<grid, FIELD_THREADS, field_smem_bytes(), s.s_compute>>>(a);
-                }
-                field_reduce_kernel<<<(cnt + 255) / 256, 256, 0, s.s_compute>>>(partial, S, cap, cnt, dout);
-                c->launches += 2;
-                CU(c, cudaGetLastError());
-            }
-            if (!gather) {
-                for (int q = 0; q < 4; ++q)
-                    if (out[q]) CU(c, cudaMemcpyAsync(out[q] + base, dout + q * P, (size_t)cnt * 4, cudaMemcpyDeviceToHost, s.s_compute));
-                continue;
-            }
-            NC(c, g_nccl.AllGather(dout, dgat, 4 * P, ncclFloat, s.comm, s.s_compute));
-            for (int rk = 0; rk < c->n_ranks; ++rk) {
-                const uint64_t rb = (uint64_t)rk * Q + r * cap;
-                const uint64_t rhi = std::min<uint64_t>((uint64_t)rk * Q + Q, self ? c->n : m);
-                if (rb >= rhi) continue;
-                const size_t rcnt = (size_t)std::min<uint64_t>(cap, rhi - rb);
-                for (int q = 0; q < 4; ++q)
-                    if (out[q])
-                        CU(c, cudaMemcpyAsync(out[q] + rb, dgat + ((size_t)rk * 4 + q) * P, rcnt * 4, cudaMemcpyDeviceToHost, s.s_compute));
-            }
+    std::vector<TargetOut> outs;
+    for (int q = 0; q < 4; ++q) outs.push_back({out[q], 4});
+    auto work = [&](uint32_t cap) { return (size_t)S * 4 * cap * 4; };
+    auto launch = [&](Shard &s, uint64_t base, uint32_t cnt, uint32_t cap, unsigned char *wk, const float *dpts,
+                      unsigned char *dout) -> int {
+        FieldArgs a{};
+        a.src = s.bodies;
+        a.partial = reinterpret_cast<float *>(wk);
+        a.stride = cap;
+        a.count = cnt;
+        a.src_nblk = (uint32_t)((c->n + BLK - 1) / BLK);
+        a.n_chunks = S;
+        a.soft2 = c->soft2;
+        const dim3 grid((cnt + FIELD_TI - 1) / FIELD_TI, S);
+        if (self) {
+            a.self0 = base; // a multiple of BLK: slices and batches are
+            field_kernel<true><<<grid, FIELD_THREADS, field_smem_bytes(), s.s_compute>>>(a);
+        } else {
+            a.px = dpts; a.py = dpts + cap; a.pz = dpts + 2 * (size_t)cap;
+            field_kernel<false><<<grid, FIELD_THREADS, field_smem_bytes(), s.s_compute>>>(a);
         }
-    }
-    return sync_all(c);
+        field_reduce_kernel<<<(cnt + 255) / 256, 256, 0, s.s_compute>>>(a.partial, S, cap, cnt, reinterpret_cast<float *>(dout));
+        c->launches += 2;
+        return B200NB_OK;
+    };
+    return run_targets(c, self, m, pts, FIELD_TI, FIELD_BATCH, outs, work, launch);
 }
 
 int b200nb_field(b200nb_ctx *c, uint64_t n_points, const float *px, const float *py, const float *pz, float *ax, float *ay,
@@ -1333,6 +1380,61 @@ int b200nb_potential(b200nb_ctx *c, float *phi)
     if (!phi) return fail(c, B200NB_EINVAL, "potential: phi is NULL");
     float *out[4] = {nullptr, nullptr, nullptr, phi};
     return field_run(c, true, c->n, nullptr, out);
+}
+
+// k nearest bodies of the points (self == false) or of every body (self == true): [S][KB][cap] candidate d2 bits and
+// indices, merged into [cap][k] index and distance rows.
+static int neighbors_run(b200nb_ctx *c, bool self, uint64_t m, const float *const pts[3], uint32_t k, uint32_t *idx, float *dist)
+{
+    const int kb = nb_bucket((int)k);
+    const uint32_t src_nblk = (uint32_t)((c->n + BLK - 1) / BLK);
+    std::vector<TargetOut> outs = {{idx, 4 * (size_t)k}, {dist, 4 * (size_t)k}};
+    auto work = [&](uint32_t cap) { return (size_t)nb_max_chunks(kb, cap) * kb * cap * 8; };
+    auto launch = [&](Shard &s, uint64_t base, uint32_t cnt, uint32_t cap, unsigned char *wk, const float *dpts,
+                      unsigned char *dout) -> int {
+        NbArgs a{};
+        a.src = s.bodies;
+        a.self0 = self ? base : 0; // a multiple of BLK: slices and batches are
+        a.px = dpts; a.py = dpts + cap; a.pz = dpts + 2 * (size_t)cap;
+        a.n_chunks = nb_chunks(kb, cnt, cap, src_nblk, (uint32_t)s.n_sms * NB_MINB);
+        a.cd2 = reinterpret_cast<uint32_t *>(wk);
+        a.cidx = a.cd2 + (size_t)a.n_chunks * kb * cap;
+        a.stride = cap;
+        a.count = cnt;
+        a.n = (uint32_t)c->n;
+        a.src_nblk = src_nblk;
+        uint32_t *didx = reinterpret_cast<uint32_t *>(dout);
+        float *ddist = reinterpret_cast<float *>(dout + 4 * (size_t)k * cap);
+        switch (kb) {
+        case 1: nb_launch<1>(self, a, k, didx, ddist, s.s_compute); break;
+        case 8: nb_launch<8>(self, a, k, didx, ddist, s.s_compute); break;
+        case 16: nb_launch<16>(self, a, k, didx, ddist, s.s_compute); break;
+        default: nb_launch<32>(self, a, k, didx, ddist, s.s_compute); break;
+        }
+        c->launches += 2;
+        return B200NB_OK;
+    };
+    return run_targets(c, self, m, pts, nb_tile(kb), nb_batch(kb), outs, work, launch);
+}
+
+int b200nb_neighbors(b200nb_ctx *c, uint32_t k, uint32_t *idx, float *dist)
+{
+    if (!c) return B200NB_EINVAL;
+    if (!c->uploaded) return fail(c, B200NB_ESTATE, "neighbors before upload");
+    if (k < 1 || k > (uint32_t)NB_K_MAX) return fail(c, B200NB_EINVAL, "neighbors: k = %u is outside [1, %d]", k, NB_K_MAX);
+    return neighbors_run(c, true, c->n, nullptr, k, idx, dist);
+}
+
+int b200nb_neighbors_at(b200nb_ctx *c, uint64_t n_points, const float *px, const float *py, const float *pz, uint32_t k,
+                        uint32_t *idx, float *dist)
+{
+    if (!c) return B200NB_EINVAL;
+    if (!c->uploaded) return fail(c, B200NB_ESTATE, "neighbors_at before upload");
+    if (k < 1 || k > (uint32_t)NB_K_MAX) return fail(c, B200NB_EINVAL, "neighbors_at: k = %u is outside [1, %d]", k, NB_K_MAX);
+    if (n_points == 0) return B200NB_OK;
+    if (!px || !py || !pz) return fail(c, B200NB_EINVAL, "neighbors_at: NULL point array");
+    const float *pts[3] = {px, py, pz};
+    return neighbors_run(c, false, n_points, pts, k, idx, dist);
 }
 
 int b200nb_sync(b200nb_ctx *c)
