@@ -187,6 +187,29 @@ int b200nb_neighbors(b200nb_ctx *ctx, uint32_t k, uint32_t *idx, float *dist);
 int b200nb_neighbors_at(b200nb_ctx *ctx, uint64_t n_points, const float *px, const float *py, const float *pz,
                         uint32_t k, uint32_t *idx, float *dist);
 
+/* ---- friends-of-friends groups --------------------------------------------------------------------------------
+ * Which bodies form a structure together (the galaxies of a merger, tidal tails, satellites, clumps): the standard
+ * friends-of-friends group finder of N-body work.  The reference has no counterpart.  Definition, for bodies i != j
+ * (fp32, round to nearest, no flush to zero, the operation sequence of the nearest-neighbour section):
+ *   dx = xj - xi, dy = yj - yi, dz = zj - zi;   d2 = dx*dx;  d2 = fmaf(dy, dy, d2);  d2 = fmaf(dz, dz, d2);
+ * i and j are linked iff d2 <= b2, where b2 = b*b rounded to fp32.  fp32 subtraction is exactly antisymmetric, so d2(i, j)
+ * and d2(j, i) are bitwise equal: the relation is symmetric and the library visits each unordered pair from one side
+ * only.  Groups are the connected components of the link graph; group[i] is the SMALLEST body index in i's group, so a
+ * body without friends has group[i] = i.  The result is a pure function of the fp32 positions and b: it does not depend
+ * on shard or rank count, chunking, reruns or the order in which the device's atomics land.  Mass plays no part
+ * (zero-mass bodies link like any other); padding bodies (index >= n_bodies) are never linked; a body at a non-finite
+ * position has d2 NaN or +inf with everyone and is always alone.  b must be >= 0 with b*b finite in fp32 (b <= ~1.84e19);
+ * b = 0 links exactly the coincident bodies.  Same calling contract as the field section: ordered after a preceding
+ * asynchronous b200nb_step, joins the devices, collective when n_ranks > 1 (every rank receives all n_bodies labels), no
+ * change to the simulation state.  Device scratch is grow-only, owned by the context and counted in
+ * b200nb_allocated_bytes: with N_pad = n_ranks * b200nb_slice_length(n_bodies, n_ranks) and P = n_ranks, one forest of
+ * 4 * N_pad bytes per shard; the shard that merges (the first, when the shards are in one process), or every rank when
+ * each rank is its own process, holds P forests, 4 * N_pad * P bytes, instead.  O(N), independent of the number of
+ * links.  Errors: B200NB_ESTATE before an upload, B200NB_EINVAL for a NULL group or a b outside the range above. */
+
+/* friends-of-friends groups of linking length b; group[n_bodies] = smallest body index of each body's group */
+int b200nb_fof(b200nb_ctx *ctx, float b, uint32_t *group);
+
 /* Joins every device and communication stream.  main.cpp:353-371 only synchronises the current device, so the glue
  * calls this when more than one device is in use. */
 int b200nb_sync(b200nb_ctx *ctx);

@@ -20,6 +20,7 @@ import numpy as np
 __all__ = [
     "B200Error", "Context", "SimulationNBodyB200", "B200Bodies", "init_bodies", "lib", "lib_path", "header_functions",
     "G_F32", "INTEGRATOR_MURB", "INTEGRATOR_LEAPFROG", "slice_length", "load_tab",
+    "fof_groups",
 ]
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -82,6 +83,7 @@ def lib() -> ctypes.CDLL:
         "b200nb_potential": (c_int, [ctx, _FP]),
         "b200nb_neighbors": (c_int, [ctx, c_uint, _UP, _FP]),
         "b200nb_neighbors_at": (c_int, [ctx, c_uint64, _FP, _FP, _FP, c_uint, _UP, _FP]),
+        "b200nb_fof": (c_int, [ctx, c_float, _UP]),
         "b200nb_sync": (c_int, [ctx]),
         "b200nb_n_bodies": (c_uint64, [ctx]),
         "b200nb_n_local_gpus": (c_int, [ctx]),
@@ -351,6 +353,26 @@ class Context:
                     "b200nb_neighbors_at")
         return idx, dist
 
+    @staticmethod
+    def _fof_b(b) -> float:
+        """b as the fp32 value the library uses; ValueError unless b >= 0 with b * b finite in fp32."""
+        ok = not isinstance(b, bool) and isinstance(b, (int, float, np.integer, np.floating))
+        if ok:
+            with np.errstate(over="ignore", invalid="ignore"):
+                b32 = np.float32(b)
+                ok = bool(b32 >= 0) and bool(np.isfinite(b32 * b32))
+        if not ok:
+            raise ValueError(f"b must be a real number >= 0 with b * b finite in fp32, got {b!r}")
+        return float(b32)
+
+    def fof(self, b) -> np.ndarray:
+        """Friends-of-friends groups of linking length b (include/b200nb.h: b200nb_fof).  Returns uint32[n]: the
+        smallest body index of each body's group."""
+        b = self._fof_b(b)
+        group = np.empty(self.n, dtype=np.uint32)
+        self._check(self._L.b200nb_fof(self._ctx, b, group.ctypes.data_as(_UP)), "b200nb_fof")
+        return group
+
     def sync(self):
         self._check(self._L.b200nb_sync(self._ctx), "b200nb_sync")
 
@@ -394,6 +416,37 @@ class Context:
         ms, n = c_double(), c_uint64()
         self._check(self._L.b200nb_profile_get(self._ctx, byref(ms), byref(n)), "b200nb_profile_get")
         return ms.value, n.value
+
+
+def fof_groups(group, m, state, min_size: int = 20) -> dict[str, np.ndarray]:
+    """Catalogue of the friends-of-friends groups of at least `min_size` members (host, O(N)).
+
+    group: the labels of Context.fof; m: the masses; state: positions and velocities as Context.download_state returns
+    them.  Groups come sorted by size, largest first, then by root.  Returns arrays with one entry per group:
+      root uint32 (the smallest body index), size int64, mass float64, com float64[g, 3] (centre of mass),
+      vel float64[g, 3] (mass-weighted mean velocity; both NaN for a group of zero mass).
+    Sums are fp64 np.bincount sums, accumulated in body order, so the catalogue is reproducible."""
+    group = np.asarray(group)
+    if group.ndim != 1 or group.dtype.kind not in "ui" or (len(group) and (group.min() < 0 or group.max() >= len(group))):
+        raise ValueError("group must be a 1-D integer array of body indices")
+    n = len(group)
+    if isinstance(min_size, bool) or not isinstance(min_size, (int, np.integer)) or min_size < 1:
+        raise ValueError(f"min_size must be an integer >= 1, got {min_size!r}")
+    m = np.asarray(m, dtype=np.float64)
+    if m.shape != (n,):
+        raise ValueError(f"expected {n} masses, got {m.shape}")
+    size = np.bincount(group, minlength=n)
+    roots = np.flatnonzero(size >= min_size)
+    roots = roots[np.lexsort((roots, -size[roots]))]
+    mass = np.bincount(group, weights=m, minlength=n)[roots]
+
+    def mean(keys):
+        cols = [np.bincount(group, weights=m * np.asarray(state[k], dtype=np.float64), minlength=n)[roots] for k in keys]
+        with np.errstate(invalid="ignore", divide="ignore"):
+            return np.stack(cols, axis=1) / mass[:, None] if len(roots) else np.zeros((0, 3))
+
+    return {"root": roots.astype(np.uint32), "size": size[roots].astype(np.int64), "mass": mass,
+            "com": mean(("qx", "qy", "qz")), "vel": mean(("vx", "vy", "vz"))}
 
 
 class B200Bodies:

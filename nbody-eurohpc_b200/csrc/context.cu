@@ -12,6 +12,7 @@
 #include <dlfcn.h>
 #include <nccl.h>
 
+#include <cfloat>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -22,6 +23,7 @@
 #include "../../include/b200nb.h"
 #include "field_sm100.cuh"
 #include "neighbors_sm100.cuh"
+#include "fof_sm100.cuh"
 #include "integrate_sm100.cuh"
 #include "plan.hpp"
 // The default force-kernel variant once more, as a cubin whose hot loop has been re-ordered after ptxas by
@@ -157,7 +159,7 @@ struct Shard {
     float *stage_full = nullptr; // one rank per process only: 3 x stage_stride floats for a full-system position download (lazy)
     double *energy_blocks = nullptr, *energy_out = nullptr;
     void *l2_scratch = nullptr;
-    // scratch of the field / potential / neighbours calls (grow-only, laid out by run_targets)
+    // scratch of the field / potential / neighbours / friends-of-friends calls (grow-only)
     unsigned char *query_buf = nullptr;
     uint64_t query_bytes = 0;
     ncclComm_t comm = nullptr;
@@ -811,7 +813,7 @@ int download_sliced(b200nb_ctx *c, float *Shard::*field, float *hx, float *hy, f
     return B200NB_OK;
 }
 
-// Grow-only scratch of the field / potential / neighbours calls.
+// Grow-only scratch of the field / potential / neighbours / friends-of-friends calls.
 int query_scratch(b200nb_ctx *c, Shard &s, size_t bytes)
 {
     if (s.query_bytes >= bytes) return B200NB_OK;
@@ -1435,6 +1437,82 @@ int b200nb_neighbors_at(b200nb_ctx *c, uint64_t n_points, const float *px, const
     if (!px || !py || !pz) return fail(c, B200NB_EINVAL, "neighbors_at: NULL point array");
     const float *pts[3] = {px, py, pz};
     return neighbors_run(c, false, n_points, pts, k, idx, dist);
+}
+
+// Friends-of-friends labels of every body (b200nb_fof); b2u: the bits of b * b in fp32.  Every shard links its own bodies
+// against all bodies into a forest of F = total_pad entries (fof_sm100.cuh).  In-process shards copy their forests to
+// shard 0, one rank per process all-gathers them; then shard 0, or every rank, folds forests 1..P-1 into forest 0,
+// finalizes it to labels and downloads them.  Scratch: P forests on the shard that merges (every rank when each rank is
+// its own process), one on every other shard.  Reads only the body array: state and cached step graphs are untouched.
+static int fof_run(b200nb_ctx *c, uint32_t b2u, uint32_t *group)
+{
+    DeviceGuard guard;
+    const bool gather = c->shards.size() != (size_t)c->n_ranks;
+    const size_t F = c->total_pad;
+    const uint32_t P = (uint32_t)c->n_ranks, n = (uint32_t)c->n;
+    const uint32_t nb = (n + BLK - 1) / BLK, stream = std::min<uint32_t>(nb / 2 + FOF_R, nb);
+    for (size_t i = 0; i < c->shards.size(); ++i)
+        if (int rc = query_scratch(c, c->shards[i], 4 * F * (gather || i == 0 ? P : 1))) return rc;
+    for (auto &s : c->shards) {
+        CU(c, cudaSetDevice(s.device));
+        // an asynchronous step may still be exchanging positions: the whole body array is read
+        if (c->n_ranks > 1)
+            if (int rc = wait_remote_positions(c, s)) return rc;
+        uint32_t *forest = reinterpret_cast<uint32_t *>(s.query_buf) + (gather ? s.rank * F : 0);
+        fof_init_kernel<<<(unsigned)((F + 255) / 256), 256, 0, s.s_compute>>>(forest, (uint32_t)F);
+        c->launches++;
+        if (s.n_local > 0) {
+            FofArgs a{};
+            a.src = s.bodies;
+            a.parent = forest;
+            a.first = (uint32_t)((uint64_t)s.rank * c->L);
+            a.count = s.n_local;
+            a.n = n;
+            a.nb = nb;
+            a.stream = stream;
+            a.thr = b2u + 1;
+            const uint32_t tiles = (s.n_local + FOF_TI - 1) / FOF_TI;
+            a.n_chunks = fof_chunks(tiles, stream, (uint32_t)s.n_sms * FOF_MINB);
+            fof_link_kernel<<<dim3(tiles, a.n_chunks), FOF_THREADS, fof_smem_bytes(), s.s_compute>>>(a);
+            c->launches++;
+        }
+        CU(c, cudaGetLastError());
+    }
+    Shard &m = c->shards[0];
+    uint32_t *forests = reinterpret_cast<uint32_t *>(m.query_buf);
+    if (gather) {
+        CU(c, cudaSetDevice(m.device));
+        NC(c, g_nccl.AllGather(forests + m.rank * F, forests, F, ncclUint32, m.comm, m.s_compute));
+    } else {
+        for (size_t i = 1; i < c->shards.size(); ++i) {
+            Shard &s = c->shards[i];
+            CU(c, cudaSetDevice(s.device));
+            CU(c, cudaMemcpyPeerAsync(forests + (size_t)s.rank * F, m.device, s.query_buf, s.device, 4 * F, s.s_compute));
+            CU(c, cudaStreamSynchronize(s.s_compute)); // the merge on shard 0 reads the copy
+        }
+    }
+    CU(c, cudaSetDevice(m.device));
+    if (P > 1) {
+        fof_merge_kernel<<<(n + 255) / 256, 256, 0, m.s_compute>>>(forests, P, F, n);
+        c->launches++;
+    }
+    fof_finalize_kernel<<<(n + 255) / 256, 256, 0, m.s_compute>>>(forests, n);
+    c->launches++;
+    CU(c, cudaGetLastError());
+    CU(c, cudaMemcpyAsync(group, forests, (size_t)n * 4, cudaMemcpyDeviceToHost, m.s_compute));
+    return sync_all(c);
+}
+
+int b200nb_fof(b200nb_ctx *c, float b, uint32_t *group)
+{
+    if (!c) return B200NB_EINVAL;
+    if (!c->uploaded) return fail(c, B200NB_ESTATE, "fof before upload");
+    if (!group) return fail(c, B200NB_EINVAL, "fof: group is NULL");
+    const float b2 = b * b;
+    if (!(b >= 0.f) || !(b2 <= FLT_MAX)) return fail(c, B200NB_EINVAL, "fof: b = %g must be >= 0 with b * b finite in fp32", (double)b);
+    uint32_t b2u;
+    memcpy(&b2u, &b2, 4);
+    return fof_run(c, b2u, group);
 }
 
 int b200nb_sync(b200nb_ctx *c)
