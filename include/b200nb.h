@@ -210,6 +210,45 @@ int b200nb_neighbors_at(b200nb_ctx *ctx, uint64_t n_points, const float *px, con
 /* friends-of-friends groups of linking length b; group[n_bodies] = smallest body index of each body's group */
 int b200nb_fof(b200nb_ctx *ctx, float b, uint32_t *group);
 
+/* ---- group potential and unbinding ----------------------------------------------------------------------------
+ * Which bodies of a group are held together by gravity: the unbinding step of every halo or structure finder, whose
+ * result (the bound mass of each structure) is the diagnostic of a merger or of tidal stripping.  The reference has no
+ * counterpart.  Labels group[n_bodies] are arbitrary uint32 values (friends-of-friends roots of b200nb_fof, galaxy or
+ * component ids, halo ids from elsewhere); a body labelled B200NB_NO_GROUP takes no part in anything.
+ * Group potential, for a body i whose label g != B200NB_NO_GROUP:
+ *   phi^g_i = -sum_{j != i, group[j] = g} G m_j / (|r_ij|^2 + soft^2)^(1/2),
+ * self pair excluded by index, with the G, softening, G*m fold, fp32 pair terms and fp64 second-level sums of
+ * b200nb_potential; with a single label it agrees with b200nb_potential to about 1e-6 relative, not bitwise.  phi = +0
+ * for NO_GROUP bodies and for bodies alone in their label.  Padding bodies never contribute; zero-mass bodies feel the
+ * potential but add nothing to it; a body at a non-finite position makes its group's values NaN (b200nb_fof puts such
+ * bodies alone).  The result is a pure function of the positions, the masses and the whole label array: bit-identical
+ * on reruns, for any shard or rank count and straight after an asynchronous step.  It is not promised to be bitwise
+ * invariant under a relabelling, which may move rounding in the last bits.
+ * Unbinding: S_0 = {i : group[i] != NO_GROUP}.  Pass t = 1, 2, ..., max_iter takes phi_i, the group potential over
+ * S_(t-1), and for each label g the frame velocity V_g = sum m_j v_j / sum m_j over g's members in S_(t-1) (fp64 sums of
+ * the fp32 masses and velocities in a fixed order; V_g = 0 when their mass is 0), evaluates
+ * E_i = |v_i - V_g|^2 / 2 + phi_i in fp64 and keeps body i iff E_i < 0 (NaN leaves; a lone body, phi = 0, leaves).
+ * S_t is the bodies kept.  The loop stops after the first pass that removes nobody (converged) or after max_iter passes.
+ * Outputs: bound[i] = group[i] for i in the final set, NO_GROUP otherwise; phi (may be NULL) = phi of the last pass for
+ * the bodies of the set it was computed over, +0 for the others (on convergence: the group potential of the final
+ * set); n_iter = passes run (0 when S_0 is empty); converged.  n_iter and converged may be NULL.  It follows that
+ * unbind(unbind(g, 1).bound, 1) returns bound and phi bit-identical to unbind(g, 2).
+ * Same calling contract as the field section: ordered after a preceding asynchronous b200nb_step, joins the devices,
+ * collective when n_ranks > 1 (every rank passes the same labels and receives every result), no change to the
+ * simulation state or cached step graphs.  Device scratch is grow-only, owned by the context, counted in
+ * b200nb_allocated_bytes and O(N) whatever the group sizes: on every shard, with N = n_bodies and N_pad = n_ranks *
+ * b200nb_slice_length(n_bodies, n_ranks), at most 102 N + 16 N_pad bytes (rounded up to 256 B per array) plus 64 MiB of
+ * partial sums (less when N < 262144) plus CUB's temporary storage for sorting N (key, value) pairs.
+ * Errors: B200NB_ESTATE before an upload; B200NB_EINVAL for a NULL group, a NULL phi (group potential), a NULL bound or
+ * max_iter == 0 (unbinding). */
+#define B200NB_NO_GROUP 0xFFFFFFFFu
+
+/* phi[n_bodies] = the group potential of the labels group[n_bodies] */
+int b200nb_group_potential(b200nb_ctx *ctx, const uint32_t *group, float *phi);
+/* unbinding of the labels group[n_bodies], at most max_iter passes; bound[n_bodies], phi[n_bodies] (may be NULL) */
+int b200nb_unbind(b200nb_ctx *ctx, const uint32_t *group, uint32_t max_iter, uint32_t *bound, float *phi,
+                  uint32_t *n_iter, int *converged);
+
 /* Joins every device and communication stream.  main.cpp:353-371 only synchronises the current device, so the glue
  * calls this when more than one device is in use. */
 int b200nb_sync(b200nb_ctx *ctx);

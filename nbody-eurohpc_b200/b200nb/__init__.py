@@ -20,7 +20,7 @@ import numpy as np
 __all__ = [
     "B200Error", "Context", "SimulationNBodyB200", "B200Bodies", "init_bodies", "lib", "lib_path", "header_functions",
     "G_F32", "INTEGRATOR_MURB", "INTEGRATOR_LEAPFROG", "slice_length", "load_tab",
-    "fof_groups",
+    "fof_groups", "NO_GROUP", "bound_groups",
 ]
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -28,6 +28,7 @@ _REPO = os.path.dirname(os.path.dirname(_HERE))
 G_F32 = np.float32(6.67384e-11)  # SimulationNBodyInterface.hpp:18 (a float literal)
 INTEGRATOR_MURB, INTEGRATOR_LEAPFROG = 0, 1
 OK, EINVAL, ECUDA, ENCCL, ESTATE = 0, 1, 2, 3, 4
+NO_GROUP = 0xFFFFFFFF  # B200NB_NO_GROUP: a body with this label takes no part in the group calls
 _FP = POINTER(c_float)
 _UP = POINTER(c_uint)
 
@@ -84,6 +85,8 @@ def lib() -> ctypes.CDLL:
         "b200nb_neighbors": (c_int, [ctx, c_uint, _UP, _FP]),
         "b200nb_neighbors_at": (c_int, [ctx, c_uint64, _FP, _FP, _FP, c_uint, _UP, _FP]),
         "b200nb_fof": (c_int, [ctx, c_float, _UP]),
+        "b200nb_group_potential": (c_int, [ctx, _UP, _FP]),
+        "b200nb_unbind": (c_int, [ctx, _UP, c_uint, _UP, _FP, _UP, POINTER(c_int)]),
         "b200nb_sync": (c_int, [ctx]),
         "b200nb_n_bodies": (c_uint64, [ctx]),
         "b200nb_n_local_gpus": (c_int, [ctx]),
@@ -373,6 +376,37 @@ class Context:
         self._check(self._L.b200nb_fof(self._ctx, b, group.ctypes.data_as(_UP)), "b200nb_fof")
         return group
 
+    def _labels(self, group) -> np.ndarray:
+        """group as the uint32[n] labels the library reads; ValueError unless 1-D, n long, integer, in [0, 2^32 - 1]."""
+        g = np.asarray(group)
+        if g.ndim != 1 or g.shape[0] != self.n or g.dtype.kind not in "ui":
+            raise ValueError(f"group must be a 1-D integer array of {self.n} labels, got {g.dtype} {g.shape}")
+        if len(g) and (int(g.min()) < 0 or int(g.max()) > NO_GROUP):
+            raise ValueError("labels must lie in [0, 2^32 - 1]")
+        return np.ascontiguousarray(g, np.uint32)
+
+    def group_potential(self, group) -> np.ndarray:
+        """Potential of every body from the members of its own label only (include/b200nb.h: b200nb_group_potential).
+        group: uint32 labels, NO_GROUP for none.  Returns float32[n]; +0 for NO_GROUP bodies and lone members."""
+        g = self._labels(group)
+        phi = np.empty(self.n, dtype=np.float32)
+        self._check(self._L.b200nb_group_potential(self._ctx, g.ctypes.data_as(_UP), _p(phi)), "b200nb_group_potential")
+        return phi
+
+    def unbind(self, group, max_iter=100) -> tuple[np.ndarray, np.ndarray, int, bool]:
+        """Iterative removal of the members whose energy in their group's frame is not negative (include/b200nb.h:
+        b200nb_unbind).  Returns (bound uint32[n]: the label of every body still bound, NO_GROUP for the others;
+        phi float32[n]: the group potential of the last pass; passes run; converged)."""
+        g = self._labels(group)
+        if isinstance(max_iter, bool) or not isinstance(max_iter, (int, np.integer)) or not 1 <= int(max_iter) <= NO_GROUP:
+            raise ValueError(f"max_iter must be an integer in [1, 2^32 - 1], got {max_iter!r}")
+        bound = np.empty(self.n, dtype=np.uint32)
+        phi = np.empty(self.n, dtype=np.float32)
+        n_iter, conv = c_uint(), c_int()
+        self._check(self._L.b200nb_unbind(self._ctx, g.ctypes.data_as(_UP), int(max_iter), bound.ctypes.data_as(_UP), _p(phi),
+                                          byref(n_iter), byref(conv)), "b200nb_unbind")
+        return bound, phi, int(n_iter.value), bool(conv.value)
+
     def sync(self):
         self._check(self._L.b200nb_sync(self._ctx), "b200nb_sync")
 
@@ -447,6 +481,50 @@ def fof_groups(group, m, state, min_size: int = 20) -> dict[str, np.ndarray]:
 
     return {"root": roots.astype(np.uint32), "size": size[roots].astype(np.int64), "mass": mass,
             "com": mean(("qx", "qy", "qz")), "vel": mean(("vx", "vy", "vz"))}
+
+
+def bound_groups(bound, m, state, phi, min_size: int = 20) -> dict[str, np.ndarray]:
+    """Catalogue of the bound groups of Context.unbind (host, O(N)).
+
+    bound: the labels Context.unbind returns (NO_GROUP: not bound); m: the masses; state: positions and velocities as
+    Context.download_state returns them; phi: the group potential Context.unbind returns.  Labels with at least
+    `min_size` bound members come sorted by size, largest first, then by label.  Returns arrays with one entry per group:
+      label uint32, size int64, mass float64, com float64[g, 3] (centre of mass), vel float64[g, 3] (mass-weighted mean
+      velocity V; both NaN for a group of zero mass), kinetic float64 (sum m |v - V|^2 / 2), potential float64
+      (sum m phi / 2, each pair counted once).
+    Sums are fp64 np.bincount sums, accumulated in body order, so the catalogue is reproducible."""
+    bound = np.asarray(bound)
+    if bound.ndim != 1 or bound.dtype.kind not in "ui" or (len(bound) and (int(bound.min()) < 0 or int(bound.max()) > NO_GROUP)):
+        raise ValueError("bound must be a 1-D integer array of labels in [0, 2^32 - 1]")
+    n = len(bound)
+    if isinstance(min_size, bool) or not isinstance(min_size, (int, np.integer)) or min_size < 1:
+        raise ValueError(f"min_size must be an integer >= 1, got {min_size!r}")
+    m = np.asarray(m, dtype=np.float64)
+    phi = np.asarray(phi, dtype=np.float64)
+    if m.shape != (n,) or phi.shape != (n,):
+        raise ValueError(f"expected {n} masses and potentials, got {m.shape} and {phi.shape}")
+    members = np.flatnonzero(bound.astype(np.uint64) != NO_GROUP)
+    labels, gid = np.unique(bound[members].astype(np.uint64), return_inverse=True)
+    ng = len(labels)
+    size = np.bincount(gid, minlength=ng)
+    keep = np.flatnonzero(size >= min_size)
+    keep = keep[np.lexsort((labels[keep], -size[keep]))]
+    mm = m[members]
+    mass = np.bincount(gid, weights=mm, minlength=ng)
+
+    def mean(keys):
+        cols = [np.bincount(gid, weights=mm * np.asarray(state[k], dtype=np.float64)[members], minlength=ng) for k in keys]
+        with np.errstate(invalid="ignore", divide="ignore"):
+            return np.stack(cols, axis=1) / mass[:, None] if ng else np.zeros((0, 3))
+
+    com, vel = mean(("qx", "qy", "qz")), mean(("vx", "vy", "vz"))
+    kin = np.zeros(ng)
+    for k, key in enumerate(("vx", "vy", "vz")):
+        dv = np.asarray(state[key], dtype=np.float64)[members] - vel[gid, k]
+        kin += np.bincount(gid, weights=0.5 * mm * dv * dv, minlength=ng)
+    pot = np.bincount(gid, weights=0.5 * mm * phi[members], minlength=ng)
+    return {"label": labels[keep].astype(np.uint32), "size": size[keep].astype(np.int64), "mass": mass[keep],
+            "com": com[keep].reshape(-1, 3), "vel": vel[keep].reshape(-1, 3), "kinetic": kin[keep], "potential": pot[keep]}
 
 
 class B200Bodies:

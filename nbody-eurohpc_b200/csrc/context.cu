@@ -24,6 +24,7 @@
 #include "field_sm100.cuh"
 #include "neighbors_sm100.cuh"
 #include "fof_sm100.cuh"
+#include "groups_sm100.cuh"
 #include "integrate_sm100.cuh"
 #include "plan.hpp"
 // The default force-kernel variant once more, as a cubin whose hot loop has been re-ordered after ptxas by
@@ -159,7 +160,7 @@ struct Shard {
     float *stage_full = nullptr; // one rank per process only: 3 x stage_stride floats for a full-system position download (lazy)
     double *energy_blocks = nullptr, *energy_out = nullptr;
     void *l2_scratch = nullptr;
-    // scratch of the field / potential / neighbours / friends-of-friends calls (grow-only)
+    // scratch of the field / potential / neighbours / friends-of-friends / group calls (grow-only)
     unsigned char *query_buf = nullptr;
     uint64_t query_bytes = 0;
     ncclComm_t comm = nullptr;
@@ -1513,6 +1514,245 @@ int b200nb_fof(b200nb_ctx *c, float b, uint32_t *group)
     uint32_t b2u;
     memcpy(&b2u, &b2, 4);
     return fof_run(c, b2u, group);
+}
+
+} // extern "C"
+
+namespace {
+
+// Carving of the group calls' scratch (groups_sm100.cuh), the same on every shard.  The sort buffers alias `piece`,
+// which is first written after the sort.
+struct GpBufs {
+    uint32_t *key[2], *val[2];
+    uint64_t *mem[2];
+    unsigned char *flags;
+    float *src, *phi, *vm, *phi_out, *partial;
+    uint32_t *lo, *hi, *bound, *info;
+    GpSum *piece;
+    void *temp;
+    size_t temp_bytes, total;
+};
+
+GpBufs gp_carve(unsigned char *base, uint64_t n, uint64_t n_pad, uint32_t P, uint32_t cap, size_t temp_bytes)
+{
+    GpBufs b{};
+    size_t off = 0;
+    auto take = [&](size_t bytes) { unsigned char *p = base ? base + off : nullptr; off += (bytes + 255) / 256 * 256; return p; };
+    b.piece = reinterpret_cast<GpSum *>(take(sizeof(GpSum) * n));
+    for (int i = 0; i < 2; ++i) {
+        b.key[i] = reinterpret_cast<uint32_t *>(base ? reinterpret_cast<unsigned char *>(b.piece) + 8 * n * i : nullptr);
+        b.val[i] = reinterpret_cast<uint32_t *>(base ? reinterpret_cast<unsigned char *>(b.piece) + 8 * n * i + 4 * n : nullptr);
+    }
+    for (int i = 0; i < 2; ++i) b.mem[i] = reinterpret_cast<uint64_t *>(take(8 * n));
+    b.flags = take(n);
+    b.src = reinterpret_cast<float *>(take(16 * ((n + BLK - 1) / BLK * BLK)));
+    b.lo = reinterpret_cast<uint32_t *>(take(4 * n));
+    b.hi = reinterpret_cast<uint32_t *>(take(4 * n));
+    b.phi = reinterpret_cast<float *>(take(4 * n));
+    b.vm = reinterpret_cast<float *>(take(16 * n_pad));
+    b.bound = reinterpret_cast<uint32_t *>(take(4 * n));
+    b.phi_out = reinterpret_cast<float *>(take(4 * n));
+    b.partial = reinterpret_cast<float *>(take((size_t)4 * GP_MAX_CHUNKS * cap));
+    b.info = reinterpret_cast<uint32_t *>(take(4 * ((size_t)P + 2)));
+    b.temp = take(temp_bytes);
+    b.temp_bytes = temp_bytes;
+    b.total = off;
+    return b;
+}
+
+// Group potential (max_iter == 0) or unbinding (max_iter passes at most) of the labels `group`; see include/b200nb.h.
+// Every shard sorts and packs the same members and runs the same O(N) unbinding step; the potential pass is split over
+// the shards by tile cost.  The host reads the member count and the split once per pass.
+int groups_run(b200nb_ctx *c, const uint32_t *group, uint32_t max_iter, uint32_t *bound, float *phi, uint32_t *n_iter,
+               int *converged)
+{
+    DeviceGuard guard;
+    // ordered after a preceding asynchronous step: positions exchanged, velocities final
+    if (int rc = sync_all(c)) return rc;
+    const bool gather = c->shards.size() != (size_t)c->n_ranks;
+    const bool unbind = max_iter > 0;
+    const uint32_t n = (uint32_t)c->n, P = (uint32_t)c->n_ranks, L = (uint32_t)c->L;
+    const uint32_t cap = (uint32_t)std::min<uint64_t>(GP_BATCH, (c->n + GP_TI - 1) / GP_TI * GP_TI);
+    std::vector<GpBufs> bufs;
+    for (auto &s : c->shards) {
+        CU(c, cudaSetDevice(s.device));
+        size_t sort_bytes = 0, sel_bytes = 0;
+        CU(c, cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, (const uint32_t *)nullptr, (uint32_t *)nullptr,
+                                              (const uint32_t *)nullptr, (uint32_t *)nullptr, (int)n));
+        CU(c, cub::DeviceSelect::Flagged(nullptr, sel_bytes, (const uint64_t *)nullptr, (const unsigned char *)nullptr,
+                                         (uint64_t *)nullptr, (uint32_t *)nullptr, (int)n));
+        const size_t temp = std::max(sort_bytes, sel_bytes);
+        if (int rc = query_scratch(c, s, gp_carve(nullptr, n, c->total_pad, P, cap, temp).total)) return rc;
+        bufs.push_back(gp_carve(s.query_buf, n, c->total_pad, P, cap, temp));
+    }
+    const unsigned g256 = (n + 255) / 256;
+    // members of the current set, packed sources, label ranges and (P > 1) the cost split, from info[0] = M <= bound
+    auto prepare = [&](Shard &s, GpBufs &b, int cur, uint32_t bound_m) -> int {
+        const uint32_t span = (bound_m + BLK - 1) / BLK * BLK;
+        gp_pack_kernel<<<(span + 255) / 256, 256, 0, s.s_compute>>>(s.bodies, b.mem[cur], b.info, span, b.src, b.lo, b.hi);
+        c->launches++;
+        if (P > 1) {
+            gp_split_kernel<<<1, GP_SPLIT_THREADS, 0, s.s_compute>>>(b.lo, b.hi, b.info, P);
+            c->launches++;
+        }
+        CU(c, cudaGetLastError());
+        return B200NB_OK;
+    };
+    for (size_t k = 0; k < c->shards.size(); ++k) {
+        Shard &s = c->shards[k];
+        GpBufs &b = bufs[k];
+        CU(c, cudaSetDevice(s.device));
+        CU(c, cudaMemcpyAsync(b.key[0], group, (size_t)n * 4, cudaMemcpyHostToDevice, s.s_compute));
+        gp_iota_kernel<<<g256, 256, 0, s.s_compute>>>(b.val[0], n);
+        CU(c, cudaMemsetAsync(b.info, 0, 4 * ((size_t)P + 2), s.s_compute));
+        CU(c, cub::DeviceRadixSort::SortPairs(b.temp, b.temp_bytes, b.key[0], b.key[1], b.val[0], b.val[1], (int)n, 0, 32,
+                                              s.s_compute));
+        gp_members_kernel<<<g256, 256, 0, s.s_compute>>>(b.key[1], b.val[1], n, b.mem[0], b.info);
+        c->launches += 3; // iota, the sort (counted once), members
+        CU(c, cudaMemsetAsync(b.phi_out, 0, (size_t)n * 4, s.s_compute));
+        CU(c, cudaMemsetAsync(b.bound, 0xFF, (size_t)n * 4, s.s_compute));
+        if (unbind && !gather) // velocities and masses of every shard, [P][4][L]: vx, vy, vz, m
+            for (auto &o : c->shards) {
+                CU(c, cudaMemcpyPeerAsync(b.vm + (size_t)o.rank * 4 * L, s.device, o.vel, o.device, (size_t)12 * L, s.s_compute));
+                CU(c, cudaMemcpyPeerAsync(b.vm + ((size_t)o.rank * 4 + 3) * L, s.device, o.mass, o.device, (size_t)4 * L, s.s_compute));
+            }
+        if (unbind && gather) {
+            float *mine = b.vm + (size_t)s.rank * 4 * L;
+            CU(c, cudaMemcpyAsync(mine, s.vel, (size_t)12 * L, cudaMemcpyDeviceToDevice, s.s_compute));
+            CU(c, cudaMemcpyAsync(mine + (size_t)3 * L, s.mass, (size_t)4 * L, cudaMemcpyDeviceToDevice, s.s_compute));
+            NC(c, g_nccl.AllGather(mine, b.vm, (size_t)4 * L, ncclFloat, s.comm, s.s_compute));
+        }
+        if (int rc = prepare(s, b, 0, n)) return rc;
+    }
+    std::vector<uint32_t> info(P + 2);
+    auto read_info = [&]() -> int {
+        Shard &s = c->shards[0];
+        CU(c, cudaSetDevice(s.device));
+        CU(c, cudaMemcpyAsync(info.data(), bufs[0].info, 4 * info.size(), cudaMemcpyDeviceToHost, s.s_compute));
+        return sync_all(c);
+    };
+    if (int rc = read_info()) return rc;
+    uint32_t M = info[0], t = 0;
+    int cur = 0;
+    bool conv = false;
+    const float soft2 = c->soft2;
+    for (;;) {
+        if (M == 0) { // S_0 empty: no pass.  Later: a pass over the empty set removes nobody.
+            if (t > 0) {
+                ++t;
+                for (size_t k = 0; k < c->shards.size(); ++k) {
+                    CU(c, cudaSetDevice(c->shards[k].device));
+                    CU(c, cudaMemsetAsync(bufs[k].phi_out, 0, (size_t)n * 4, c->shards[k].s_compute));
+                }
+            }
+            conv = true;
+            break;
+        }
+        // ---- the potential pass: this shard's tiles [split[rank], split[rank + 1]) in batches of `cap` targets
+        const uint32_t T = (M + GP_TI - 1) / GP_TI, cb = gp_chunk_blks(M);
+        const uint32_t n_chunks = ((M + BLK - 1) / BLK + cb - 1) / cb;
+        auto range = [&](int rank, uint32_t &a, uint32_t &e) {
+            const uint32_t ta = P > 1 ? info[1 + rank] : 0, tb = P > 1 ? info[2 + rank] : T;
+            a = std::min(ta * GP_TI, M);
+            e = std::min(tb * GP_TI, M);
+        };
+        for (size_t k = 0; k < c->shards.size(); ++k) {
+            Shard &s = c->shards[k];
+            GpBufs &b = bufs[k];
+            CU(c, cudaSetDevice(s.device));
+            if (gather) CU(c, cudaMemsetAsync(b.phi, 0, (size_t)M * 4, s.s_compute)); // summed over the ranks below
+            uint32_t a, e;
+            range(s.rank, a, e);
+            for (uint32_t t0 = a; t0 < e; t0 += cap) {
+                GpArgs g{};
+                g.src = b.src; g.lo = b.lo; g.hi = b.hi; g.partial = b.partial;
+                g.stride = cap; g.t0 = t0; g.count = std::min(cap, e - t0); g.cb = cb; g.soft2 = soft2;
+                group_potential_kernel<<<dim3((g.count + GP_TI - 1) / GP_TI, n_chunks), GP_THREADS, gp_smem_bytes(), s.s_compute>>>(g);
+                group_reduce_kernel<<<(g.count + 255) / 256, 256, 0, s.s_compute>>>(b.partial, cap, t0, g.count, cb, b.lo, b.hi, b.phi);
+                c->launches += 2;
+                CU(c, cudaGetLastError());
+            }
+        }
+        if (P > 1 && gather) {
+            Shard &s = c->shards[0];
+            CU(c, cudaSetDevice(s.device));
+            // every other rank's entries are +0 here, and x + 0 == x for every value phi takes (never -0)
+            NC(c, g_nccl.AllReduce(bufs[0].phi, bufs[0].phi, M, ncclFloat, ncclSum, s.comm, s.s_compute));
+        } else if (P > 1) {
+            for (size_t k = 0; k < c->shards.size(); ++k) {
+                Shard &s = c->shards[k];
+                uint32_t a, e;
+                range(s.rank, a, e);
+                if (a >= e) continue;
+                CU(c, cudaSetDevice(s.device));
+                for (size_t o = 0; o < c->shards.size(); ++o)
+                    if (o != k)
+                        CU(c, cudaMemcpyPeerAsync(bufs[o].phi + a, c->shards[o].device, bufs[k].phi + a, s.device, (size_t)(e - a) * 4,
+                                                  s.s_compute));
+            }
+            if (int rc = sync_all(c)) return rc; // every shard's phi is complete
+        }
+        ++t;
+        // ---- the unbinding step, the same on every shard: frame velocities, energies, flags, compaction, next set
+        for (size_t k = 0; k < c->shards.size(); ++k) {
+            Shard &s = c->shards[k];
+            GpBufs &b = bufs[k];
+            CU(c, cudaSetDevice(s.device));
+            const unsigned gm = (M + 255) / 256;
+            if (unbind) {
+                CU(c, cudaMemsetAsync(b.phi_out, 0, (size_t)n * 4, s.s_compute));
+                const uint32_t pieces = (M + GP_PIECE - 1) / GP_PIECE;
+                gp_piece_kernel<<<(pieces + 255) / 256, 256, 0, s.s_compute>>>(b.mem[cur], b.info, b.vm, L, b.piece);
+                gp_frame_kernel<<<gm, 256, 0, s.s_compute>>>(b.lo, b.hi, b.info, b.piece);
+                c->launches += 2;
+            }
+            gp_finish_kernel<<<gm, 256, 0, s.s_compute>>>(b.mem[cur], b.info, b.lo, unbind ? b.vm : nullptr, L, b.piece, b.phi,
+                                                          b.flags, b.bound, b.phi_out);
+            c->launches++;
+            CU(c, cudaGetLastError());
+            if (!unbind) continue;
+            CU(c, cub::DeviceSelect::Flagged(b.temp, b.temp_bytes, b.mem[cur], b.flags, b.mem[cur ^ 1], b.info, (int)M, s.s_compute));
+            c->launches++; // the compaction (counted once)
+            if (t < max_iter)
+                if (int rc = prepare(s, b, cur ^ 1, M)) return rc;
+        }
+        if (!unbind) break;
+        cur ^= 1;
+        if (int rc = read_info()) return rc;
+        if (info[0] == M) { conv = true; break; }
+        M = info[0];
+        if (t == max_iter) break;
+    }
+    Shard &s = c->shards[0];
+    CU(c, cudaSetDevice(s.device));
+    if (phi) CU(c, cudaMemcpyAsync(phi, bufs[0].phi_out, (size_t)n * 4, cudaMemcpyDeviceToHost, s.s_compute));
+    if (bound) CU(c, cudaMemcpyAsync(bound, bufs[0].bound, (size_t)n * 4, cudaMemcpyDeviceToHost, s.s_compute));
+    if (int rc = sync_all(c)) return rc;
+    if (n_iter) *n_iter = t;
+    if (converged) *converged = conv ? 1 : 0;
+    return B200NB_OK;
+}
+
+} // namespace
+
+extern "C" {
+
+int b200nb_group_potential(b200nb_ctx *c, const uint32_t *group, float *phi)
+{
+    if (!c) return B200NB_EINVAL;
+    if (!c->uploaded) return fail(c, B200NB_ESTATE, "group_potential before upload");
+    if (!group || !phi) return fail(c, B200NB_EINVAL, "group_potential: group or phi is NULL");
+    return groups_run(c, group, 0, nullptr, phi, nullptr, nullptr);
+}
+
+int b200nb_unbind(b200nb_ctx *c, const uint32_t *group, uint32_t max_iter, uint32_t *bound, float *phi, uint32_t *n_iter,
+                  int *converged)
+{
+    if (!c) return B200NB_EINVAL;
+    if (!c->uploaded) return fail(c, B200NB_ESTATE, "unbind before upload");
+    if (!group || !bound) return fail(c, B200NB_EINVAL, "unbind: group or bound is NULL");
+    if (max_iter == 0) return fail(c, B200NB_EINVAL, "unbind: max_iter must be >= 1");
+    return groups_run(c, group, max_iter, bound, phi, n_iter, converged);
 }
 
 int b200nb_sync(b200nb_ctx *c)
