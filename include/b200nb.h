@@ -249,6 +249,48 @@ int b200nb_group_potential(b200nb_ctx *ctx, const uint32_t *group, float *phi);
 int b200nb_unbind(b200nb_ctx *ctx, const uint32_t *group, uint32_t max_iter, uint32_t *bound, float *phi,
                   uint32_t *n_iter, int *converged);
 
+/* ---- test particles -------------------------------------------------------------------------------------------
+ * Massless test particles ("tracers") moving in the field of the bodies: the restricted N-body method (Toomre & Toomre)
+ * that resolves tidal tails, bridges and stripped material at N*M instead of (N+M)^2 interactions per step.  The
+ * reference has no counterpart.  A context holds M >= 0 tracers, each an fp32 position p and velocity w.  Tracers have
+ * no mass: they never act on the bodies or on each other, and the bodies move exactly as without them.
+ * Every b200nb_step iteration advances them with the bodies' integrator and dt.  A tracer's acceleration a(p) is the
+ * b200nb_field acceleration at p over all bodies, bit for bit (same kernel, same chunking, same fixed-order fp64
+ * reduction, rounded once to fp32), taken at the body positions of the same instant:
+ *  - MUrB:      a = a(p_n; q_n), the positions before the update; then p and w are updated with the operation sequence of
+ *               the bodies' MUrB update:  adt = a*dt (fp32);  p' = fp32(p + (w + adt*0.5)*dt) evaluated in fp64;
+ *               w' = w + adt (fp32);
+ *  - leapfrog:  w+ = fmaf(a(p_n; q_n), dt*0.5f, w);  p' = fp32(fma((double)w+, dt, (double)p));
+ *               w' = fmaf(a(p'; q_{n+1}), dt*0.5f, w+),  the bodies' kick-drift-kick; a(p_n; q_n) is kept between steps
+ *               as the bodies keep a(x_n).
+ * It follows that a tracer's trajectory depends only on its own initial state and on the body trajectory: not on the
+ * other tracers, on M, on the shard or rank count, on whether a step went through a captured graph, or on reruns.
+ * Non-finite tracer states, and a tracer exactly on a body when soft = 0, give what b200nb_field gives there.
+ * Body uploads: tracers persist across b200nb_upload; an upload invalidates their stored acceleration, as it does the
+ * bodies' a(x_0), so the next leapfrog step evaluates a(p; q) anew.  b200nb_integrate_host_accel moves the bodies but not
+ * the tracers, and invalidates their stored acceleration likewise.  b200nb_accel, the field / neighbour / group calls,
+ * b200nb_energy and b200nb_metrics neither read nor change tracers.  With M = 0 a context behaves exactly as one that
+ * never had tracers: the same launches, the same step graphs, the same state and the same b200nb_allocated_bytes.
+ * Placement: tracers are split contiguously over the ranks, T = ceil(M / n_ranks) rounded up to a multiple of 512 per
+ * shard (rank r owns tracers [r*T, min((r+1)*T, M)); later shards may own none); a shard keeps its slice as device SoA
+ * and never exchanges it.  Device bytes, counted in b200nb_allocated_bytes and freed with the tracer set (replacement,
+ * removal or b200nb_destroy), on every local shard when M > 0:
+ *     36 * T + 16 * S * min(T, 65536),     S = min(64, max(1, ceil(ceil(n_bodies / 128) / 32)))
+ * (positions, velocities and the stored acceleration, plus the partial sums of the field pass, at most 64 MiB).
+ * Both calls are collective when n_ranks > 1: every rank passes the full arrays and keeps only its own slice, or
+ * receives every tracer.  Host pointers are borrowed for the duration of the call.  b200nb_set_tracers is allowed before
+ * the first b200nb_upload (a step still needs one); it joins the devices and drops the cached step graphs.
+ * Errors: B200NB_EINVAL for NULL arrays with n_tracers > 0 or a per-shard slice T >= 2^31; B200NB_ECUDA when the device
+ * memory cannot be allocated (a set larger than a device's free memory fails before anything is allocated).  Any error
+ * leaves the context with no tracers at all, never half set. */
+
+/* replaces the context's tracers; n_tracers == 0 removes them (pointers ignored); SoA host arrays of n_tracers floats */
+int b200nb_set_tracers(b200nb_ctx *ctx, uint64_t n_tracers, const float *qx, const float *qy, const float *qz,
+                       const float *vx, const float *vy, const float *vz);
+/* joins the devices, copies back all tracers (any pointer may be NULL) */
+int b200nb_download_tracers(b200nb_ctx *ctx, float *qx, float *qy, float *qz, float *vx, float *vy, float *vz);
+uint64_t b200nb_n_tracers(const b200nb_ctx *ctx);
+
 /* Joins every device and communication stream.  main.cpp:353-371 only synchronises the current device, so the glue
  * calls this when more than one device is in use. */
 int b200nb_sync(b200nb_ctx *ctx);

@@ -87,6 +87,9 @@ def lib() -> ctypes.CDLL:
         "b200nb_fof": (c_int, [ctx, c_float, _UP]),
         "b200nb_group_potential": (c_int, [ctx, _UP, _FP]),
         "b200nb_unbind": (c_int, [ctx, _UP, c_uint, _UP, _FP, _UP, POINTER(c_int)]),
+        "b200nb_set_tracers": (c_int, [ctx, c_uint64] + [_FP] * 6),
+        "b200nb_download_tracers": (c_int, [ctx] + [_FP] * 6),
+        "b200nb_n_tracers": (c_uint64, [ctx]),
         "b200nb_sync": (c_int, [ctx]),
         "b200nb_n_bodies": (c_uint64, [ctx]),
         "b200nb_n_local_gpus": (c_int, [ctx]),
@@ -406,6 +409,26 @@ class Context:
         self._check(self._L.b200nb_unbind(self._ctx, g.ctypes.data_as(_UP), int(max_iter), bound.ctypes.data_as(_UP), _p(phi),
                                           byref(n_iter), byref(conv)), "b200nb_unbind")
         return bound, phi, int(n_iter.value), bool(conv.value)
+
+    def set_tracers(self, qx, qy, qz, vx, vy, vz):
+        """Replaces the massless test particles (include/b200nb.h: b200nb_set_tracers): six 1-D arrays of equal length
+        M, positions and velocities.  Empty arrays remove them."""
+        t = [_f32(a) for a in (qx, qy, qz, vx, vy, vz)]
+        if any(a.ndim != 1 for a in t) or len({a.shape for a in t}) != 1:
+            raise ValueError(f"expected six 1-D arrays of equal length, got {[a.shape for a in t]}")
+        m = t[0].shape[0]
+        ptrs = [_p(a) for a in t] if m else [None] * 6
+        self._check(self._L.b200nb_set_tracers(self._ctx, m, *ptrs), "b200nb_set_tracers")
+
+    def download_tracers(self) -> dict[str, np.ndarray]:
+        """Positions and velocities of every tracer after the steps enqueued so far: keys qx .. vz, float32[M]."""
+        out = {k: np.empty(self.n_tracers, dtype=np.float32) for k in self._STATE}
+        self._check(self._L.b200nb_download_tracers(self._ctx, *[_p(out[k]) for k in self._STATE]), "b200nb_download_tracers")
+        return out
+
+    @property
+    def n_tracers(self) -> int:
+        return int(self._L.b200nb_n_tracers(self._ctx))
 
     def sync(self):
         self._check(self._L.b200nb_sync(self._ctx), "b200nb_sync")

@@ -25,6 +25,7 @@
 #include "neighbors_sm100.cuh"
 #include "fof_sm100.cuh"
 #include "groups_sm100.cuh"
+#include "tracers_sm100.cuh"
 #include "integrate_sm100.cuh"
 #include "plan.hpp"
 // The default force-kernel variant once more, as a cubin whose hot loop has been re-ordered after ptxas by
@@ -163,6 +164,12 @@ struct Shard {
     // scratch of the field / potential / neighbours / friends-of-friends / group calls (grow-only)
     unsigned char *query_buf = nullptr;
     uint64_t query_bytes = 0;
+    // test particles (b200nb_set_tracers): tr = [9][tr_T] rows qx qy qz vx vy vz ax ay az of the shard's tracers, the
+    // first tr_local columns real; tr_part = the [S][4][tr_cap] partial rows of their field pass.  Both are owned by the
+    // tracer set, never by query_buf: a captured step graph bakes their addresses in.
+    float *tr = nullptr, *tr_part = nullptr;
+    uint32_t tr_local = 0;
+    uint64_t tr_bytes = 0;
     ncclComm_t comm = nullptr;
     CUmodule resched_mod = nullptr;   // the re-ordered cubin of the default variant on this device (nullptr: not in use)
     CUfunction resched_fn = nullptr;
@@ -208,6 +215,11 @@ struct b200nb_ctx {
     uint32_t sk_rows_own = 0, sk_rows_rem = 0;
     std::vector<Shard> shards;
     bool uploaded = false, acc_valid = false, profiling = false;
+    // test particles: M in all, T per shard (ceil(M / P) in whole FIELD_TI tiles), batch of one field launch; the stored
+    // tracer a(p) is valid for the current positions (the leapfrog's counterpart of acc_valid, kept apart from it)
+    uint64_t m_tracers = 0, tr_T = 0;
+    uint32_t tr_cap = 0;
+    bool tr_acc_valid = false;
     uint64_t launches = 0;
     std::string err;
 };
@@ -920,6 +932,76 @@ void nb_launch(bool self, const NbArgs &a, uint32_t k, uint32_t *idx, float *dis
     nb_merge_kernel<KB><<<(a.count + 127) / 128, 128, 0, st>>>(a.cd2, a.cidx, a.n_chunks, a.stride, a.count, k, idx, dist);
 }
 
+// ------------------------------------------------------------------------------------------------ test particles
+// Device bytes of one shard's tracer set (include/b200nb.h states the same formula)
+uint64_t tracer_bytes(uint64_t T, uint32_t cap, uint32_t S) { return 36 * T + 16 * (uint64_t)S * cap; }
+
+// the context holds no tracers afterwards (callers have joined the streams)
+void free_tracers(b200nb_ctx *c)
+{
+    for (auto &s : c->shards) {
+        if (s.tr || s.tr_part) {
+            cudaSetDevice(s.device);
+            cudaFree(s.tr);
+            cudaFree(s.tr_part);
+        }
+        s.tr = s.tr_part = nullptr;
+        s.bytes -= s.tr_bytes;
+        s.tr_bytes = 0;
+        s.tr_local = 0;
+    }
+    c->m_tracers = c->tr_T = 0;
+    c->tr_cap = 0;
+    c->tr_acc_valid = false;
+}
+
+// The field of the current body array at every tracer of every shard, in batches of at most FIELD_BATCH targets, each
+// batch summed and applied by tracer_update_kernel (TracerMode `mode`).  The pass reads the whole body array, so with
+// several ranks it waits for the position exchange itself.
+int enqueue_tracer_pass(b200nb_ctx *c, int mode, float dt)
+{
+    const uint32_t S = field_chunks(c->n);
+    for (auto &s : c->shards) {
+        if (s.tr_local == 0) continue;
+        CU(c, cudaSetDevice(s.device));
+        if (c->n_ranks > 1)
+            if (int rc = wait_remote_positions(c, s)) return rc;
+        for (uint32_t base = 0; base < s.tr_local; base += c->tr_cap) {
+            const uint32_t cnt = std::min(c->tr_cap, s.tr_local - base);
+            FieldArgs a{};
+            a.src = s.bodies;
+            a.px = s.tr + base; a.py = s.tr + c->tr_T + base; a.pz = s.tr + 2 * c->tr_T + base;
+            a.partial = s.tr_part;
+            a.stride = c->tr_cap;
+            a.count = cnt;
+            a.src_nblk = (uint32_t)((c->n + BLK - 1) / BLK);
+            a.n_chunks = S;
+            a.soft2 = c->soft2;
+            field_kernel<false><<<dim3((cnt + FIELD_TI - 1) / FIELD_TI, S), FIELD_THREADS, field_smem_bytes(), s.s_compute>>>(a);
+            TracerArgs u{};
+            u.partial = s.tr_part; u.n_chunks = S; u.stride = c->tr_cap; u.count = cnt;
+            u.tr = s.tr + base; u.T = c->tr_T; u.dt = dt; u.mode = mode;
+            tracer_update_kernel<<<(cnt + 255) / 256, 256, 0, s.s_compute>>>(u);
+            c->launches += 2;
+            CU(c, cudaGetLastError());
+        }
+    }
+    return B200NB_OK;
+}
+
+// the leapfrog's kick-drift of every tracer with its stored a(p); element-wise, no body is read
+int enqueue_tracer_kick_drift(b200nb_ctx *c, float dt)
+{
+    for (auto &s : c->shards) {
+        if (s.tr_local == 0) continue;
+        CU(c, cudaSetDevice(s.device));
+        tracer_kick_drift_kernel<<<(s.tr_local + 255) / 256, 256, 0, s.s_compute>>>(s.tr, c->tr_T, s.tr_local, dt);
+        c->launches++;
+        CU(c, cudaGetLastError());
+    }
+    return B200NB_OK;
+}
+
 } // namespace
 
 // =================================================================================================== C ABI
@@ -1000,6 +1082,7 @@ void b200nb_destroy(b200nb_ctx *c)
         for (auto e : s.prof_free) cudaEventDestroy(e);
         cudaFree(s.bodies); cudaFree(s.bodies_next); cudaFree(s.vel); cudaFree(s.acc); cudaFree(s.mass); cudaFree(s.partial); cudaFree(s.stage); cudaFree(s.stage_full);
         cudaFree(s.energy_blocks); cudaFree(s.energy_out); cudaFree(s.l2_scratch); cudaFree(s.query_buf);
+        cudaFree(s.tr); cudaFree(s.tr_part);
         for (auto t : s.timer) if (t) cudaEventDestroy(t);
         if (s.ev_integrated) cudaEventDestroy(s.ev_integrated);
         if (s.ev_gathered) cudaEventDestroy(s.ev_gathered);
@@ -1067,6 +1150,7 @@ int b200nb_upload(b200nb_ctx *c, const float *qx, const float *qy, const float *
     }
     c->uploaded = true;
     c->acc_valid = false;
+    c->tr_acc_valid = false; // the tracers stay, their stored a(p) was taken in the old field
     return B200NB_OK;
 }
 
@@ -1151,24 +1235,37 @@ int b200nb_download_accel(b200nb_ctx *c, float *ax, float *ay, float *az)
     return download_sliced(c, &Shard::acc, ax, ay, az);
 }
 
-// one iteration, enqueued on the compute stream(s)
+// one iteration, enqueued on the compute stream(s).  Tracers (if any) read the body positions of the same instant as the
+// bodies' own accelerations: q_n for MUrB, so their pass precedes the integrator, which overwrites the own slice in
+// place (or, p2p, swaps `bodies`); q_{n+1} for the leapfrog's closing kick, read from the current `bodies` after the swap.
 static int enqueue_one_step(b200nb_ctx *c, float dt, int integrator)
 {
+    const bool tracers = c->m_tracers > 0;
     if (integrator == B200NB_INTEGRATOR_MURB) {
         if (int rc = enqueue_force(c)) return rc;
+        if (tracers)
+            if (int rc = enqueue_tracer_pass(c, TM_MURB, dt)) return rc;
         if (int rc = enqueue_integrate(c, IM_MURB, dt)) return rc;
         if (int rc = enqueue_gather(c)) return rc;
         c->acc_valid = false; // acc belongs to the positions before the update
+        c->tr_acc_valid = false;
     } else {
         if (!c->acc_valid) { // a(x_0): once after an upload
             if (int rc = enqueue_force(c)) return rc;
             if (int rc = enqueue_integrate(c, IM_REDUCE_ONLY, dt)) return rc;
         }
+        if (tracers && !c->tr_acc_valid) // a(p_0; q_0): once after the tracers, the bodies or the scheme changed
+            if (int rc = enqueue_tracer_pass(c, TM_LF_ACC, dt)) return rc;
         if (int rc = enqueue_integrate(c, IM_LF_KICK_DRIFT, dt)) return rc;
         if (int rc = enqueue_gather(c)) return rc;
+        if (tracers) // beside the exchange
+            if (int rc = enqueue_tracer_kick_drift(c, dt)) return rc;
         if (int rc = enqueue_force(c)) return rc;
+        if (tracers)
+            if (int rc = enqueue_tracer_pass(c, TM_LF_KICK, dt)) return rc;
         if (int rc = enqueue_integrate(c, IM_LF_KICK, dt)) return rc;
         c->acc_valid = true; // acc == a(x_{n+1})
+        c->tr_acc_valid = tracers;
     }
     return B200NB_OK;
 }
@@ -1182,7 +1279,7 @@ static int get_step_graph(b200nb_ctx *c, float dt, int integrator, StepGraph **o
     Shard &s = c->shards[0];
     CU(c, cudaSetDevice(s.device));
     const uint64_t before = c->launches;
-    const bool acc_valid = c->acc_valid;
+    const bool acc_valid = c->acc_valid, tr_acc_valid = c->tr_acc_valid;
     CU(c, cudaStreamBeginCapture(s.s_compute, cudaStreamCaptureModeThreadLocal));
     int rc = B200NB_OK;
     for (int i = 0; i < GRAPH_STEPS && rc == B200NB_OK; ++i) rc = enqueue_one_step(c, dt, integrator);
@@ -1192,6 +1289,7 @@ static int get_step_graph(b200nb_ctx *c, float dt, int integrator, StepGraph **o
     g.integrator = integrator; g.dt = dt; g.steps = GRAPH_STEPS; g.launches = c->launches - before;
     c->launches = before;      // nothing ran yet
     c->acc_valid = acc_valid;
+    c->tr_acc_valid = tr_acc_valid;
     if (rc != B200NB_OK) { if (graph) cudaGraphDestroy(graph); return rc; }
     if (e != cudaSuccess) return fail(c, B200NB_ECUDA, "cudaStreamEndCapture: %s", cudaGetErrorString(e));
     const cudaError_t ei = cudaGraphInstantiate(&g.exec, graph, 0);
@@ -1220,7 +1318,8 @@ int b200nb_step(b200nb_ctx *c, float dt, int integrator, int n_steps)
     int it = 0;
     static const bool no_graph = getenv("B200NB_NO_GRAPH") != nullptr;
     if (c->n_ranks == 1 && !c->profiling && !no_graph && n_steps >= GRAPH_MIN_STEPS) {
-        if (integrator == B200NB_INTEGRATOR_LEAPFROG && !c->acc_valid) { // the one-off a(x_0) pass stays outside the graph
+        // the one-off a(x_0) and tracer a(p_0) passes stay outside the graph
+        if (integrator == B200NB_INTEGRATOR_LEAPFROG && (!c->acc_valid || (c->m_tracers > 0 && !c->tr_acc_valid))) {
             if (int rc = enqueue_one_step(c, dt, integrator)) return rc;
             ++it;
         }
@@ -1233,6 +1332,7 @@ int b200nb_step(b200nb_ctx *c, float dt, int integrator, int n_steps)
             c->launches += g->launches;
         }
         c->acc_valid = integrator == B200NB_INTEGRATOR_LEAPFROG;
+        c->tr_acc_valid = c->acc_valid && c->m_tracers > 0;
     }
     for (; it < n_steps; ++it)
         if (int rc = enqueue_one_step(c, dt, integrator)) return rc;
@@ -1272,6 +1372,7 @@ int b200nb_integrate_host_accel(b200nb_ctx *c, const float *ax, const float *ay,
     if (int rc = enqueue_integrate(c, IM_MURB_STORED, dt)) return rc;
     if (int rc = enqueue_gather(c)) return rc;
     c->acc_valid = false;
+    c->tr_acc_valid = false; // the bodies moved, the tracers did not
     return sync_all(c); // borrowed host pointers (see upload)
 }
 
@@ -1515,6 +1616,115 @@ int b200nb_fof(b200nb_ctx *c, float b, uint32_t *group)
     memcpy(&b2u, &b2, 4);
     return fof_run(c, b2u, group);
 }
+
+int b200nb_set_tracers(b200nb_ctx *c, uint64_t n_tracers, const float *qx, const float *qy, const float *qz, const float *vx,
+                       const float *vy, const float *vz)
+{
+    if (!c) return B200NB_EINVAL;
+    if (n_tracers > 0 && (!qx || !qy || !qz || !vx || !vy || !vz)) return fail(c, B200NB_EINVAL, "set_tracers: NULL array");
+    const uint64_t per = (n_tracers + c->n_ranks - 1) / c->n_ranks;
+    const uint64_t T = (per + FIELD_TI - 1) / FIELD_TI * FIELD_TI;
+    if (T >= (1ull << 31))
+        return fail(c, B200NB_EINVAL, "set_tracers: %llu tracers per shard; the field kernel counts targets in 32 bits",
+                    (unsigned long long)T);
+    DeviceGuard guard;
+    // steps in flight read the old tracers, and captured step graphs hold their buffers and count
+    if (int rc = sync_all(c)) return rc;
+    for (auto &g : c->graphs)
+        if (g.exec) cudaGraphExecDestroy(g.exec);
+    c->graphs.clear();
+    free_tracers(c);
+    if (n_tracers == 0) return B200NB_OK;
+    const uint32_t S = field_chunks(c->n), cap = (uint32_t)std::min<uint64_t>(FIELD_BATCH, T);
+    const uint64_t bytes = tracer_bytes(T, cap, S);
+    // a set that cannot fit fails before it takes any memory (shards may share a device)
+    for (auto &s : c->shards) {
+        uint64_t need = 0;
+        for (auto &o : c->shards) need += o.device == s.device ? bytes : 0;
+        size_t free_b = 0, total_b = 0;
+        CU(c, cudaSetDevice(s.device));
+        CU(c, cudaMemGetInfo(&free_b, &total_b));
+        if (need > free_b)
+            return fail(c, B200NB_ECUDA, "set_tracers: %llu tracers need %llu bytes on device %d, %llu are free",
+                        (unsigned long long)n_tracers, (unsigned long long)need, s.device, (unsigned long long)free_b);
+    }
+    for (auto &s : c->shards) {
+        cudaError_t e = cudaSetDevice(s.device);
+        if (e == cudaSuccess) e = cudaMalloc((void **)&s.tr, 9 * T * 4);
+        if (e == cudaSuccess) e = cudaMalloc((void **)&s.tr_part, (size_t)S * 4 * cap * 4);
+        if (e != cudaSuccess) { // never half set: no tracers at all
+            (void)cudaGetLastError();
+            free_tracers(c);
+            return fail(c, B200NB_ECUDA, "set_tracers: %s", cudaGetErrorString(e));
+        }
+        s.tr_bytes = bytes;
+        s.bytes += bytes;
+    }
+    const float *src[6] = {qx, qy, qz, vx, vy, vz};
+    for (auto &s : c->shards) {
+        const uint64_t first = (uint64_t)s.rank * T;
+        s.tr_local = first >= n_tracers ? 0u : (uint32_t)std::min<uint64_t>(T, n_tracers - first);
+        cudaError_t e = cudaSetDevice(s.device);
+        for (int k = 0; k < 6 && s.tr_local > 0 && e == cudaSuccess; ++k)
+            e = cudaMemcpyAsync(s.tr + k * T, src[k] + first, (size_t)s.tr_local * 4, cudaMemcpyHostToDevice, s.s_compute);
+        if (e != cudaSuccess) {
+            (void)cudaGetLastError();
+            sync_all(c);
+            free_tracers(c);
+            return fail(c, B200NB_ECUDA, "set_tracers: %s", cudaGetErrorString(e));
+        }
+    }
+    // host pointers are only borrowed for the call (see upload)
+    if (int rc = sync_all(c)) { free_tracers(c); return rc; }
+    c->m_tracers = n_tracers;
+    c->tr_T = T;
+    c->tr_cap = cap;
+    return B200NB_OK;
+}
+
+int b200nb_download_tracers(b200nb_ctx *c, float *qx, float *qy, float *qz, float *vx, float *vy, float *vz)
+{
+    if (!c) return B200NB_EINVAL;
+    DeviceGuard guard;
+    if (int rc = sync_all(c)) return rc;
+    const uint64_t M = c->m_tracers, T = c->tr_T;
+    float *dst[6] = {qx, qy, qz, vx, vy, vz};
+    if (M == 0) return B200NB_OK;
+    if (c->shards.size() == (size_t)c->n_ranks) { // every shard is local: each one returns its own slice
+        for (auto &s : c->shards) {
+            if (s.tr_local == 0) continue;
+            CU(c, cudaSetDevice(s.device));
+            for (int k = 0; k < 6; ++k)
+                if (dst[k])
+                    CU(c, cudaMemcpyAsync(dst[k] + (size_t)s.rank * T, s.tr + k * T, (size_t)s.tr_local * 4, cudaMemcpyDeviceToHost,
+                                          s.s_compute));
+        }
+        return sync_all(c);
+    }
+    // one rank per process: all-gather the [6][T] slices through a temporary [P][6][T] device buffer (download_sliced)
+    Shard &s = c->shards[0];
+    CU(c, cudaSetDevice(s.device));
+    struct Scratch { // freed on every exit path
+        float *p = nullptr;
+        ~Scratch() { if (p) cudaFree(p); }
+    } tmp;
+    const size_t count = 6 * (size_t)T;
+    CU(c, cudaMalloc((void **)&tmp.p, count * c->n_ranks * 4));
+    NC(c, g_nccl.AllGather(s.tr, tmp.p, count, ncclFloat, s.comm, s.s_compute));
+    for (int rk = 0; rk < c->n_ranks; ++rk) {
+        const uint64_t first = (uint64_t)rk * T;
+        if (first >= M) break;
+        const size_t cnt = (size_t)std::min<uint64_t>(T, M - first);
+        for (int k = 0; k < 6; ++k)
+            if (dst[k])
+                CU(c, cudaMemcpyAsync(dst[k] + first, tmp.p + (size_t)rk * count + (size_t)k * T, cnt * 4, cudaMemcpyDeviceToHost,
+                                      s.s_compute));
+    }
+    CU(c, cudaStreamSynchronize(s.s_compute));
+    return B200NB_OK;
+}
+
+uint64_t b200nb_n_tracers(const b200nb_ctx *c) { return c ? c->m_tracers : 0; }
 
 } // extern "C"
 

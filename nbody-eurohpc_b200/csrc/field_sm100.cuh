@@ -230,16 +230,28 @@ __global__ void __launch_bounds__(FIELD_THREADS, FIELD_MINB) field_kernel(const 
     }
 }
 
+// s[q] = the fixed-order fp64 sum of the S chunk rows of component q < NQ (0..2: x, y, z; 3: G*m*inv) of target i.
+// The one summation behind every field value: b200nb_field and the test-particle step (tracers_sm100.cuh) both use it,
+// which is what makes a tracer's acceleration bit-identical to b200nb_field at its position.
+template <int NQ>
+__device__ __forceinline__ void field_sum_rows(const float *__restrict__ partial, uint32_t n_chunks, uint32_t stride,
+                                               uint32_t i, double (&s)[NQ])
+{
+#pragma unroll
+    for (int q = 0; q < NQ; ++q) s[q] = 0.0;
+    for (uint32_t r = 0; r < n_chunks; ++r)
+#pragma unroll
+        for (int q = 0; q < NQ; ++q) s[q] += (double)partial[((size_t)r * 4 + q) * stride + i];
+}
+
 // out[q * stride + i], q = 0..3: ax, ay, az, phi.  Fixed-order fp64 sum of the S chunk rows, rounded once.
 __global__ void __launch_bounds__(256) field_reduce_kernel(const float *__restrict__ partial, uint32_t n_chunks,
                                                           uint32_t stride, uint32_t count, float *__restrict__ out)
 {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= count) return;
-    double s[4] = {0.0, 0.0, 0.0, 0.0};
-    for (uint32_t r = 0; r < n_chunks; ++r)
-#pragma unroll
-        for (int q = 0; q < 4; ++q) s[q] += (double)partial[((size_t)r * 4 + q) * stride + i];
+    double s[4];
+    field_sum_rows<4>(partial, n_chunks, stride, i, s);
 #pragma unroll
     for (int q = 0; q < 3; ++q) out[(size_t)q * stride + i] = (float)s[q];
     out[(size_t)3 * stride + i] = (float)-s[3];
