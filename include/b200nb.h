@@ -159,6 +159,35 @@ int b200nb_field(b200nb_ctx *ctx, uint64_t n_points, const float *px, const floa
 /* Per-body potential of the current positions, self pair excluded, all n_bodies values.  Collective when n_ranks > 1. */
 int b200nb_potential(b200nb_ctx *ctx, float *phi);
 
+/* ---- the tidal tensor -----------------------------------------------------------------------------------------
+ * The derivative of the field above, T_ab = d a_a / d p_b = -d^2 phi / dp_a dp_b: the input of tidal and Jacobi radii,
+ * tidal-field histories along orbits, tidal-environment classification by eigenvalue signs and |lambda|^(-1/2)
+ * time-step criteria.  The reference has no counterpart.  Same G, softening and G*m fold as b200nb_field; with
+ * d = q_j - p and s^2 = |d|^2 + soft^2:
+ *   at a point p, over ALL bodies:         T_ab(p) = sum_j G m_j [ 3 d_a d_b / s^5 - delta_ab / s^3 ],
+ *   per body, self pair excluded by INDEX: T_ab,i  = sum_{j != i} (the same term with p = q_i),
+ * exactly d a_a / d p_b of the softened a(p) of b200nb_field.  One body at distance r with soft = 0 gives
+ * G m / r^3 * diag(2, -1, -1) in a frame whose x axis points at it; the trace is -3 soft^2 sum_j G m_j / s^5 (0 for
+ * soft = 0 away from bodies).  Output: six fp32 components per target, rows t[i][6] in the order xx, yy, zz, xy, xz, yz.
+ * Accuracy: fp32 pair terms whose every intermediate stays in fp32's normal range, sums finished in fp64; every entry is
+ * within 5e-6 * A_ab of fp64, A_ab = sum_j G m_j (3 |d_a d_b| / s^5 + delta_ab / s^3) (the cancellation-free scale).
+ * Same calling contract as the field section: a result depends only on its point (or body) and the current bodies,
+ * bit-identical whatever the other points of the call, the batching, the shard or rank count, and on reruns; ordered after
+ * a preceding asynchronous b200nb_step; joins the devices; collective when n_ranks > 1 (every rank passes the same points
+ * and receives every row); no change to the simulation state, the stored accelerations, the tracers or cached step
+ * graphs.  Padding bodies add nothing.  Non-finite results occur exactly where b200nb_field gives them (a point on a body,
+ * or coincident bodies, when soft = 0).  Device scratch is grow-only, owned by the context and counted in
+ * b200nb_allocated_bytes; targets go through in batches of B = min(32768, Q rounded up to a multiple of 256), Q = the
+ * points or bodies of one rank, and a call needs 28 * S * B + 36 * B bytes per GPU (at most 56 MiB + 1.125 MiB), plus
+ * 24 * B * n_ranks for the gathered rows when each rank is its own process, S = min(64, max(1, ceil(ceil(n_bodies / 128)
+ * / 32))).  The buffer is shared with the field, neighbour and friends-of-friends calls: it grows to the largest need.
+ * Errors: B200NB_ESTATE before an upload; B200NB_EINVAL for NULL point arrays or a NULL t.  n_points == 0 is a no-op. */
+
+/* Tidal tensor at n_points arbitrary points (host SoA); t[n_points][6]. */
+int b200nb_tidal(b200nb_ctx *ctx, uint64_t n_points, const float *px, const float *py, const float *pz, float *t);
+/* Tidal tensor of every body, self pair excluded; t[n_bodies][6]. */
+int b200nb_tidal_bodies(b200nb_ctx *ctx, float *t);
+
 /* ---- nearest neighbours ---------------------------------------------------------------------------------------
  * The k nearest bodies of every body, or of arbitrary points (close encounters, bound pairs, Casertano-Hut densities
  * from the 6th neighbour, nearest-distance time-step criteria).  The reference has no counterpart.  Definition, for a

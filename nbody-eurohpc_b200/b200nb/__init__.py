@@ -82,6 +82,8 @@ def lib() -> ctypes.CDLL:
         "b200nb_metrics": (c_int, [ctx, POINTER(c_double)]),
         "b200nb_field": (c_int, [ctx, c_uint64] + [_FP] * 7),
         "b200nb_potential": (c_int, [ctx, _FP]),
+        "b200nb_tidal": (c_int, [ctx, c_uint64, _FP, _FP, _FP, _FP]),
+        "b200nb_tidal_bodies": (c_int, [ctx, _FP]),
         "b200nb_neighbors": (c_int, [ctx, c_uint, _UP, _FP]),
         "b200nb_neighbors_at": (c_int, [ctx, c_uint64, _FP, _FP, _FP, c_uint, _UP, _FP]),
         "b200nb_fof": (c_int, [ctx, c_float, _UP]),
@@ -328,6 +330,34 @@ class Context:
         phi = np.empty(self.n, dtype=np.float32)
         self._check(self._L.b200nb_potential(self._ctx, _p(phi)), "b200nb_potential")
         return phi
+
+    # the six columns xx, yy, zz, xy, xz, yz of b200nb_tidal's rows, as (row, column) of the symmetric 3x3 matrix
+    _TIDAL_IDX = ([0, 1, 2, 0, 0, 1], [0, 1, 2, 1, 2, 2])
+
+    @classmethod
+    def _tidal_matrix(cls, t6: np.ndarray) -> np.ndarray:
+        t = np.empty((t6.shape[0], 3, 3), dtype=np.float32)
+        r, c = cls._TIDAL_IDX
+        t[:, r, c] = t6
+        t[:, c, r] = t6
+        return t
+
+    def tidal(self, px, py, pz) -> np.ndarray:
+        """Tidal tensor T_ab = d a_a / d p_b at arbitrary points, summed over every body (include/b200nb.h: b200nb_tidal).
+        px, py, pz: 1-D arrays of equal length.  Returns float32[m, 3, 3], symmetric."""
+        p = [_f32(a) for a in (px, py, pz)]
+        if any(a.ndim != 1 for a in p) or len({a.shape for a in p}) != 1:
+            raise ValueError(f"expected three 1-D arrays of equal length, got {[a.shape for a in p]}")
+        m = p[0].shape[0]
+        t6 = np.empty((m, 6), dtype=np.float32)
+        self._check(self._L.b200nb_tidal(self._ctx, m, *[_p(a) for a in p], _p(t6)), "b200nb_tidal")
+        return self._tidal_matrix(t6)
+
+    def tidal_bodies(self) -> np.ndarray:
+        """Tidal tensor of every body, self pair excluded (include/b200nb.h: b200nb_tidal_bodies).  float32[n, 3, 3]."""
+        t6 = np.empty((self.n, 6), dtype=np.float32)
+        self._check(self._L.b200nb_tidal_bodies(self._ctx, _p(t6)), "b200nb_tidal_bodies")
+        return self._tidal_matrix(t6)
 
     NEIGHBORS_K_MAX = 32
 

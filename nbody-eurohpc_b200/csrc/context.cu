@@ -26,6 +26,7 @@
 #include "fof_sm100.cuh"
 #include "groups_sm100.cuh"
 #include "tracers_sm100.cuh"
+#include "tidal_sm100.cuh"
 #include "integrate_sm100.cuh"
 #include "plan.hpp"
 // The default force-kernel variant once more, as a cubin whose hot loop has been re-ordered after ptxas by
@@ -1484,6 +1485,57 @@ int b200nb_potential(b200nb_ctx *c, float *phi)
     if (!phi) return fail(c, B200NB_EINVAL, "potential: phi is NULL");
     float *out[4] = {nullptr, nullptr, nullptr, phi};
     return field_run(c, true, c->n, nullptr, out);
+}
+
+// Tidal tensor at points (self == false) or of every body (self == true): [S][7][cap] partial rows, summed into one
+// [cap][6] row block (xx, yy, zz, xy, xz, yz).
+static int tidal_run(b200nb_ctx *c, bool self, uint64_t m, const float *const pts[3], float *t)
+{
+    const uint32_t S = field_chunks(c->n);
+    const std::vector<TargetOut> outs = {{t, 6 * 4}};
+    auto work = [&](uint32_t cap) { return (size_t)S * TIDAL_NQ * cap * 4; };
+    auto launch = [&](Shard &s, uint64_t base, uint32_t cnt, uint32_t cap, unsigned char *wk, const float *dpts,
+                      unsigned char *dout) -> int {
+        FieldArgs a{};
+        a.src = s.bodies;
+        a.partial = reinterpret_cast<float *>(wk);
+        a.stride = cap;
+        a.count = cnt;
+        a.src_nblk = (uint32_t)((c->n + BLK - 1) / BLK);
+        a.n_chunks = S;
+        a.soft2 = c->soft2;
+        const dim3 grid((cnt + TIDAL_TI - 1) / TIDAL_TI, S);
+        if (self) {
+            a.self0 = base; // a multiple of BLK: slices and batches are
+            tidal_kernel<true><<<grid, TIDAL_THREADS, tidal_smem_bytes(), s.s_compute>>>(a);
+        } else {
+            a.px = dpts; a.py = dpts + cap; a.pz = dpts + 2 * (size_t)cap;
+            tidal_kernel<false><<<grid, TIDAL_THREADS, tidal_smem_bytes(), s.s_compute>>>(a);
+        }
+        tidal_reduce_kernel<<<(cnt + 255) / 256, 256, 0, s.s_compute>>>(a.partial, S, cap, cnt, reinterpret_cast<float *>(dout));
+        c->launches += 2;
+        return B200NB_OK;
+    };
+    return run_targets(c, self, m, pts, TIDAL_TI, TIDAL_BATCH, outs, work, launch);
+}
+
+int b200nb_tidal(b200nb_ctx *c, uint64_t n_points, const float *px, const float *py, const float *pz, float *t)
+{
+    if (!c) return B200NB_EINVAL;
+    if (!c->uploaded) return fail(c, B200NB_ESTATE, "tidal before upload");
+    if (n_points == 0) return B200NB_OK;
+    if (!px || !py || !pz) return fail(c, B200NB_EINVAL, "tidal: NULL point array");
+    if (!t) return fail(c, B200NB_EINVAL, "tidal: t is NULL");
+    const float *pts[3] = {px, py, pz};
+    return tidal_run(c, false, n_points, pts, t);
+}
+
+int b200nb_tidal_bodies(b200nb_ctx *c, float *t)
+{
+    if (!c) return B200NB_EINVAL;
+    if (!c->uploaded) return fail(c, B200NB_ESTATE, "tidal_bodies before upload");
+    if (!t) return fail(c, B200NB_EINVAL, "tidal_bodies: t is NULL");
+    return tidal_run(c, true, c->n, nullptr, t);
 }
 
 // k nearest bodies of the points (self == false) or of every body (self == true): [S][KB][cap] candidate d2 bits and
