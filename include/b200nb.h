@@ -188,6 +188,50 @@ int b200nb_tidal(b200nb_ctx *ctx, uint64_t n_points, const float *px, const floa
 /* Tidal tensor of every body, self pair excluded; t[n_bodies][6]. */
 int b200nb_tidal_bodies(b200nb_ctx *ctx, float *t);
 
+/* ---- field by component ---------------------------------------------------------------------------------------
+ * Who pulls on whom in a run with several structures (the galaxies of a merger, a disk, bulge and halo, a satellite):
+ * the field of b200nb_field split by source component, the input of rotation-curve decompositions, the self and
+ * interaction energies of a merger, and the force and torque between components (dynamical friction, angular-momentum
+ * exchange).  The reference has no counterpart.  Labels comp[n_bodies] (uint32) and n_comp in [1, 64]: a body with
+ * comp[j] = h < n_comp is a source of component h; a body labelled B200NB_NO_GROUP is a source of nothing but is still a
+ * target in bodies mode.  Same law, G, softening and G*m fold as b200nb_field; with d = q_j - p:
+ *   at a point p:  a^h(p)   = sum_{j: comp[j] = h} G m_j d / (|d|^2 + soft^2)^(3/2),
+ *                  phi^h(p) = -sum_{j: comp[j] = h} G m_j / (|d|^2 + soft^2)^(1/2);
+ *   per body i:    the same sums at p = q_i, self pair excluded by INDEX (it matters only for h = comp[i]).
+ * A component without members gives a = 0 and phi = -0.  Rows: acc[m][n_comp][3], phi[m][n_comp].
+ * Promises:
+ *  1. bit-identity with the field: with one component holding every body (n_comp = 1, every label 0),
+ *     b200nb_component_field returns b200nb_field's ax, ay, az and phi, and b200nb_component_field_bodies returns
+ *     b200nb_potential's phi, bit for bit;
+ *  2. locality: the value for (target, h) depends only on the target (its point, or its index in bodies mode) and on the
+ *     positions and masses of h's members in index order.  It is bit-identical when other bodies are relabelled, merged,
+ *     split or set to NO_GROUP, when n_comp changes and when h is renumbered, and across reruns, batching, the other
+ *     points of the call, and the shard and rank count;
+ *  3. accuracy: per component, the field's bound: |a - a64| <= 1e-6 * sum_{j in h} |a_ij| and |phi - phi64| <= 1e-6 *
+ *     |phi64| (galaxy and random schemes, soft 2e8 and 1e4).
+ * Calling contract of the field section: ordered after a preceding asynchronous b200nb_step; joins the devices;
+ * collective when n_ranks > 1 (every rank passes the same labels and points and receives every row); no change to the
+ * simulation state, the stored accelerations, the leapfrog's a(x_n), the tracers or cached step graphs.  acc or phi may be
+ * NULL.  n_points == 0 is a no-op.  Errors: B200NB_ESTATE before an upload; B200NB_EINVAL for a NULL comp, n_comp outside
+ * [1, 64], a label that is neither < n_comp nor B200NB_NO_GROUP, or NULL point arrays.
+ * Cost: one field pass whatever n_comp, plus at most 127 padding sources per component.  Device scratch is grow-only,
+ * owned by the context, counted in b200nb_allocated_bytes and shared with the field, tidal, neighbour and friends-of-
+ * friends calls.  With M_h the members of h, T = sum_h 128 * ceil(M_h / 128) packed sources, S_h = 0 for M_h = 0 and
+ * min(64, max(1, ceil(ceil(M_h / 128) / 32))) otherwise, S = sum_h S_h (<= ceil(n_bodies / 4096) + n_comp), and targets in
+ * batches of B = min(Q rounded up to a multiple of 512, 65536, max(1, floor(2^22 / (512 * max(S, 1)))) * 512), Q = the
+ * points or bodies of one rank, a call needs per GPU
+ *     r(16 * S * B) + r(16 * T) + r(4 * T) + r(4 * n_bodies) [bodies mode only] + r(8 * S) + r(4 * (n_comp + 1))
+ *     + 12 * B + 16 * n_comp * B,     r(x) = x rounded up to a multiple of 256,
+ * plus 16 * n_comp * B * n_ranks for the gathered rows when each rank is its own process: at most 64 MiB of partial rows
+ * and 64 MiB of result rows, plus 20 B per packed source.  Kernel launches per call: one packing kernel per GPU when some
+ * component has members, and per batch the field kernel (when some component has members) and one reduction. */
+
+/* a^h and phi^h at n_points arbitrary points (host SoA): acc[n_points][n_comp][3], phi[n_points][n_comp] */
+int b200nb_component_field(b200nb_ctx *ctx, const uint32_t *comp, uint32_t n_comp, uint64_t n_points, const float *px,
+                           const float *py, const float *pz, float *acc, float *phi);
+/* a^h and phi^h of every body, self pair excluded: acc[n_bodies][n_comp][3], phi[n_bodies][n_comp] */
+int b200nb_component_field_bodies(b200nb_ctx *ctx, const uint32_t *comp, uint32_t n_comp, float *acc, float *phi);
+
 /* ---- nearest neighbours ---------------------------------------------------------------------------------------
  * The k nearest bodies of every body, or of arbitrary points (close encounters, bound pairs, Casertano-Hut densities
  * from the 6th neighbour, nearest-distance time-step criteria).  The reference has no counterpart.  Definition, for a

@@ -20,7 +20,7 @@ import numpy as np
 __all__ = [
     "B200Error", "Context", "SimulationNBodyB200", "B200Bodies", "init_bodies", "lib", "lib_path", "header_functions",
     "G_F32", "INTEGRATOR_MURB", "INTEGRATOR_LEAPFROG", "slice_length", "load_tab",
-    "fof_groups", "NO_GROUP", "bound_groups",
+    "fof_groups", "NO_GROUP", "bound_groups", "component_budget", "COMPONENTS_MAX",
 ]
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -29,6 +29,7 @@ G_F32 = np.float32(6.67384e-11)  # SimulationNBodyInterface.hpp:18 (a float lite
 INTEGRATOR_MURB, INTEGRATOR_LEAPFROG = 0, 1
 OK, EINVAL, ECUDA, ENCCL, ESTATE = 0, 1, 2, 3, 4
 NO_GROUP = 0xFFFFFFFF  # B200NB_NO_GROUP: a body with this label takes no part in the group calls
+COMPONENTS_MAX = 64    # n_comp of the component-field calls lies in [1, COMPONENTS_MAX]
 _FP = POINTER(c_float)
 _UP = POINTER(c_uint)
 
@@ -84,6 +85,8 @@ def lib() -> ctypes.CDLL:
         "b200nb_potential": (c_int, [ctx, _FP]),
         "b200nb_tidal": (c_int, [ctx, c_uint64, _FP, _FP, _FP, _FP]),
         "b200nb_tidal_bodies": (c_int, [ctx, _FP]),
+        "b200nb_component_field": (c_int, [ctx, _UP, c_uint, c_uint64] + [_FP] * 5),
+        "b200nb_component_field_bodies": (c_int, [ctx, _UP, c_uint, _FP, _FP]),
         "b200nb_neighbors": (c_int, [ctx, c_uint, _UP, _FP]),
         "b200nb_neighbors_at": (c_int, [ctx, c_uint64, _FP, _FP, _FP, c_uint, _UP, _FP]),
         "b200nb_fof": (c_int, [ctx, c_float, _UP]),
@@ -440,6 +443,41 @@ class Context:
                                           byref(n_iter), byref(conv)), "b200nb_unbind")
         return bound, phi, int(n_iter.value), bool(conv.value)
 
+    def _components(self, comp, n_comp) -> tuple[np.ndarray, int]:
+        """(labels, n_comp) as the library reads them; ValueError unless n_comp is an integer in [1, COMPONENTS_MAX] and
+        every label is < n_comp or NO_GROUP."""
+        if isinstance(n_comp, bool) or not isinstance(n_comp, (int, np.integer)) or not 1 <= int(n_comp) <= COMPONENTS_MAX:
+            raise ValueError(f"n_comp must be an integer in [1, {COMPONENTS_MAX}], got {n_comp!r}")
+        g = self._labels(comp)
+        if np.any((g >= n_comp) & (g != NO_GROUP)):
+            raise ValueError(f"every label must be < n_comp = {int(n_comp)} or NO_GROUP")
+        return g, int(n_comp)
+
+    def component_field(self, comp, n_comp, px, py, pz) -> tuple[np.ndarray, np.ndarray]:
+        """Acceleration and potential at arbitrary points from each source component (include/b200nb.h:
+        b200nb_component_field).  comp: uint32 labels in [0, n_comp) or NO_GROUP; px, py, pz: 1-D arrays of equal length m.
+        Returns (acc float32[m, n_comp, 3], phi float32[m, n_comp])."""
+        g, C = self._components(comp, n_comp)
+        p = [_f32(a) for a in (px, py, pz)]
+        if any(a.ndim != 1 for a in p) or len({a.shape for a in p}) != 1:
+            raise ValueError(f"expected three 1-D arrays of equal length, got {[a.shape for a in p]}")
+        m = p[0].shape[0]
+        acc = np.empty((m, C, 3), dtype=np.float32)
+        phi = np.empty((m, C), dtype=np.float32)
+        self._check(self._L.b200nb_component_field(self._ctx, g.ctypes.data_as(_UP), C, m, *[_p(a) for a in p], _p(acc), _p(phi)),
+                    "b200nb_component_field")
+        return acc, phi
+
+    def component_field_bodies(self, comp, n_comp) -> tuple[np.ndarray, np.ndarray]:
+        """Acceleration and potential of every body from each source component, self pair excluded (include/b200nb.h:
+        b200nb_component_field_bodies).  Returns (acc float32[n, n_comp, 3], phi float32[n, n_comp])."""
+        g, C = self._components(comp, n_comp)
+        acc = np.empty((self.n, C, 3), dtype=np.float32)
+        phi = np.empty((self.n, C), dtype=np.float32)
+        self._check(self._L.b200nb_component_field_bodies(self._ctx, g.ctypes.data_as(_UP), C, _p(acc), _p(phi)),
+                    "b200nb_component_field_bodies")
+        return acc, phi
+
     def set_tracers(self, qx, qy, qz, vx, vy, vz):
         """Replaces the massless test particles (include/b200nb.h: b200nb_set_tracers): six 1-D arrays of equal length
         M, positions and velocities.  Empty arrays remove them."""
@@ -578,6 +616,63 @@ def bound_groups(bound, m, state, phi, min_size: int = 20) -> dict[str, np.ndarr
     pot = np.bincount(gid, weights=0.5 * mm * phi[members], minlength=ng)
     return {"label": labels[keep].astype(np.uint32), "size": size[keep].astype(np.int64), "mass": mass[keep],
             "com": com[keep].reshape(-1, 3), "vel": vel[keep].reshape(-1, 3), "kinetic": kin[keep], "potential": pot[keep]}
+
+
+def component_budget(comp, n_comp, m, state, acc, phi, centre=(0.0, 0.0, 0.0)) -> dict[str, np.ndarray]:
+    """Mass, momentum, energy and torque budget of the source components (host, O(N * n_comp)).
+
+    comp, n_comp: the labels of Context.component_field_bodies (NO_GROUP bodies belong to no component and are left out);
+    m: the masses; state: positions and velocities as Context.download_state returns them; acc, phi: the rows
+    Context.component_field_bodies returns (float[n, n_comp, 3] and float[n, n_comp]); centre: the point about which spins
+    and torques are taken.  With r_i, v_i the body's position and velocity and c the centre, returns for each component g:
+      mass float64[C], com float64[C, 3] (centre of mass), vel float64[C, 3] (mass-weighted mean velocity; both NaN for a
+      component of zero mass), kinetic float64[C] (sum m |v|^2 / 2), spin float64[C, 3] (sum m (r - c) x v),
+    and for each pair (g, h), the action of the sources h on the bodies of g:
+      force float64[C, C, 3] = sum_{i in g} m_i a_i^h, torque float64[C, C, 3] = sum_{i in g} m_i (r_i - c) x a_i^h,
+      W float64[C, C] = sum_{i in g} m_i phi_i^h (the interaction energy for g != h is W[g, h] = W[h, g]).
+    The total potential energy of the components is (1/2) sum_gh W[g, h], so sum_g kinetic[g] + (1/2) sum_gh W[g, h] is
+    their total energy; Newton's third law makes force and torque antisymmetric in (g, h), with force[g, g] = 0 and
+    torque[g, g] = 0 up to rounding.  Sums are fp64 np.bincount sums, accumulated in body order, so the budget is
+    reproducible."""
+    if isinstance(n_comp, bool) or not isinstance(n_comp, (int, np.integer)) or not 1 <= int(n_comp) <= COMPONENTS_MAX:
+        raise ValueError(f"n_comp must be an integer in [1, {COMPONENTS_MAX}], got {n_comp!r}")
+    C = int(n_comp)
+    comp = np.asarray(comp)
+    if comp.ndim != 1 or comp.dtype.kind not in "ui":
+        raise ValueError("comp must be a 1-D integer array of labels")
+    n = len(comp)
+    lab = comp.astype(np.int64)
+    if n and np.any(((lab < 0) | (lab >= C)) & (lab != NO_GROUP)):
+        raise ValueError(f"every label must lie in [0, {C}) or be NO_GROUP")
+    m = np.asarray(m, dtype=np.float64)
+    acc = np.asarray(acc, dtype=np.float64)
+    phi = np.asarray(phi, dtype=np.float64)
+    if m.shape != (n,) or acc.shape != (n, C, 3) or phi.shape != (n, C):
+        raise ValueError(f"expected m[{n}], acc[{n}, {C}, 3] and phi[{n}, {C}], got {m.shape}, {acc.shape} and {phi.shape}")
+    c = np.asarray(centre, dtype=np.float64)
+    if c.shape != (3,):
+        raise ValueError(f"centre must be 3 numbers, got shape {c.shape}")
+    members = np.flatnonzero(lab != NO_GROUP)
+    gid = lab[members]
+    mm = m[members]
+    r = np.stack([np.asarray(state[k], dtype=np.float64)[members] for k in ("qx", "qy", "qz")], axis=1) - c
+    v = np.stack([np.asarray(state[k], dtype=np.float64)[members] for k in ("vx", "vy", "vz")], axis=1)
+
+    def gsum(w):  # per-component sums of the columns of w[members, ...]
+        w = w.reshape(len(members), int(np.prod(w.shape[1:])))
+        return np.stack([np.bincount(gid, weights=w[:, k], minlength=C) for k in range(w.shape[1])], axis=1)
+
+    mass = np.bincount(gid, weights=mm, minlength=C)
+    with np.errstate(invalid="ignore", divide="ignore"):
+        com = gsum(mm[:, None] * (r + c)) / mass[:, None]
+        vel = gsum(mm[:, None] * v) / mass[:, None]
+    ma = mm[:, None, None] * acc[members]  # [members, C, 3]
+    return {"mass": mass, "com": com, "vel": vel,
+            "kinetic": np.bincount(gid, weights=0.5 * mm * np.einsum("ik,ik->i", v, v), minlength=C),
+            "spin": gsum(mm[:, None] * np.cross(r, v)),
+            "force": gsum(ma).reshape(C, C, 3),
+            "torque": gsum(np.cross(r[:, None, :], ma)).reshape(C, C, 3),
+            "W": gsum(mm[:, None] * phi[members])}
 
 
 class B200Bodies:

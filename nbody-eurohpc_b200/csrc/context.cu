@@ -27,6 +27,7 @@
 #include "groups_sm100.cuh"
 #include "tracers_sm100.cuh"
 #include "tidal_sm100.cuh"
+#include "components_sm100.cuh"
 #include "integrate_sm100.cuh"
 #include "plan.hpp"
 // The default force-kernel variant once more, as a cubin whose hot loop has been re-ordered after ptxas by
@@ -1536,6 +1537,153 @@ int b200nb_tidal_bodies(b200nb_ctx *c, float *t)
     if (!c->uploaded) return fail(c, B200NB_ESTATE, "tidal_bodies before upload");
     if (!t) return fail(c, B200NB_EINVAL, "tidal_bodies: t is NULL");
     return tidal_run(c, true, c->n, nullptr, t);
+}
+
+// Scratch of the component calls (components_sm100.cuh) ahead of run_targets' points and rows, the same on every shard;
+// each array is rounded up to 256 B.
+struct CompBufs {
+    float *partial, *src;
+    uint32_t *map, *pos, *chunk0;
+    uint2 *chunk;
+    size_t total;
+};
+
+static CompBufs comp_carve(unsigned char *base, uint32_t n_chunks, uint32_t cap, uint32_t T, uint32_t n_pos, uint32_t C)
+{
+    CompBufs b{};
+    size_t off = 0;
+    auto take = [&](size_t bytes) { unsigned char *p = base ? base + off : nullptr; off += (bytes + 255) / 256 * 256; return p; };
+    b.partial = reinterpret_cast<float *>(take((size_t)16 * n_chunks * cap));
+    b.src = reinterpret_cast<float *>(take((size_t)16 * T));
+    b.map = reinterpret_cast<uint32_t *>(take((size_t)4 * T));
+    b.pos = reinterpret_cast<uint32_t *>(take((size_t)4 * n_pos));
+    b.chunk = reinterpret_cast<uint2 *>(take((size_t)8 * n_chunks));
+    b.chunk0 = reinterpret_cast<uint32_t *>(take((size_t)4 * (C + 1)));
+    b.total = off;
+    return b;
+}
+
+// Field by source component at points (self == false) or of every body (self == true); labels already checked.
+// The host sorts the members, packs their order and cuts the chunks; every shard packs the same source array once per
+// call, then runs its targets in batches: [sum S][4][cap] partial rows, summed per component into [cap][C][3] and
+// [cap][C] rows.
+static int component_run(b200nb_ctx *c, const uint32_t *comp, uint32_t C, bool self, uint64_t m, const float *const pts[3],
+                         float *acc, float *phi)
+{
+    const uint32_t n = (uint32_t)c->n;
+    std::vector<uint32_t> cnt(C, 0);
+    for (uint32_t i = 0; i < n; ++i)
+        if (comp[i] != B200NB_NO_GROUP) cnt[comp[i]]++;
+    // component h: packed blocks [blk0[h], blk0[h] + nblk_h), chunks [chunk0[h], chunk0[h + 1]) cut as field_kernel cuts
+    std::vector<uint32_t> blk0(C), chunk0(C + 1);
+    std::vector<uint2> chunk;
+    uint32_t nb = 0, max_chunk = 0;
+    for (uint32_t h = 0; h < C; ++h) {
+        const uint32_t nblk = (cnt[h] + BLK - 1) / BLK, S = cnt[h] ? field_chunks(cnt[h]) : 0;
+        blk0[h] = nb;
+        chunk0[h] = (uint32_t)chunk.size();
+        for (uint32_t k = 0; k < S; ++k) {
+            const uint2 r = make_uint2(nb + (uint32_t)((uint64_t)nblk * k / S), nb + (uint32_t)((uint64_t)nblk * (k + 1) / S));
+            max_chunk = std::max(max_chunk, r.y - r.x);
+            chunk.push_back(r);
+        }
+        nb += nblk;
+    }
+    const uint32_t n_chunks = (uint32_t)chunk.size();
+    chunk0[C] = n_chunks;
+    const uint32_t T = nb * BLK;
+    // the stable (component, index) order: map[packed position] = body (padding: COMP_PAD | h's last member), pos = its inverse
+    std::vector<uint32_t> map(T), pos(self ? n : 0), next(C);
+    for (uint32_t h = 0; h < C; ++h) next[h] = blk0[h] * BLK;
+    for (uint32_t i = 0; i < n; ++i) {
+        const uint32_t h = comp[i];
+        if (h == B200NB_NO_GROUP) {
+            if (self) pos[i] = COMP_NONE;
+            continue;
+        }
+        map[next[h]] = i;
+        if (self) pos[i] = next[h];
+        next[h]++;
+    }
+    for (uint32_t h = 0; h < C; ++h)
+        for (uint32_t p = next[h]; p < (blk0[h] + (cnt[h] + BLK - 1) / BLK) * BLK; ++p) map[p] = map[next[h] - 1] | COMP_PAD;
+
+    const uint32_t batch = std::min<uint32_t>(FIELD_BATCH, std::max<uint32_t>(1, COMP_PARTIAL_FLOATS / 4 / std::max(n_chunks, 1u) / FIELD_TI) * FIELD_TI);
+    const std::vector<TargetOut> outs = {{acc, 12 * (size_t)C}, {phi, 4 * (size_t)C}};
+    auto work = [&](uint32_t cap) { return comp_carve(nullptr, n_chunks, cap, T, (uint32_t)pos.size(), C).total; };
+    std::vector<char> packed(c->shards.size(), 0);
+    auto launch = [&](Shard &s, uint64_t base, uint32_t cnt_, uint32_t cap, unsigned char *wk, const float *dpts,
+                      unsigned char *dout) -> int {
+        const CompBufs b = comp_carve(wk, n_chunks, cap, T, (uint32_t)pos.size(), C);
+        char &done = packed[&s - c->shards.data()];
+        if (!done) { // once per shard and call: the tables and the packed sources
+            if (T) CU(c, cudaMemcpyAsync(b.map, map.data(), (size_t)4 * T, cudaMemcpyHostToDevice, s.s_compute));
+            if (self) CU(c, cudaMemcpyAsync(b.pos, pos.data(), (size_t)4 * n, cudaMemcpyHostToDevice, s.s_compute));
+            if (n_chunks) CU(c, cudaMemcpyAsync(b.chunk, chunk.data(), (size_t)8 * n_chunks, cudaMemcpyHostToDevice, s.s_compute));
+            CU(c, cudaMemcpyAsync(b.chunk0, chunk0.data(), (size_t)4 * (C + 1), cudaMemcpyHostToDevice, s.s_compute));
+            if (T) {
+                component_pack_kernel<<<(T + 255) / 256, 256, 0, s.s_compute>>>(s.bodies, b.map, T, b.src);
+                c->launches++;
+            }
+            done = 1;
+        }
+        float *dacc = reinterpret_cast<float *>(dout), *dphi = dacc + (size_t)3 * C * cap;
+        if (n_chunks) {
+            CompArgs a{};
+            a.src = b.src;
+            a.chunk = b.chunk;
+            a.partial = b.partial;
+            a.stride = cap;
+            a.count = cnt_;
+            a.soft2 = c->soft2;
+            const dim3 grid((cnt_ + FIELD_TI - 1) / FIELD_TI, n_chunks);
+            if (self) {
+                a.bodies = s.bodies;
+                a.pos = b.pos;
+                a.self0 = base;
+                component_field_kernel<true><<<grid, FIELD_THREADS, comp_smem_bytes(max_chunk), s.s_compute>>>(a);
+            } else {
+                a.px = dpts; a.py = dpts + cap; a.pz = dpts + 2 * (size_t)cap;
+                component_field_kernel<false><<<grid, FIELD_THREADS, field_smem_bytes(), s.s_compute>>>(a);
+            }
+            c->launches++;
+        }
+        component_reduce_kernel<<<dim3((cnt_ + 255) / 256, C), 256, 0, s.s_compute>>>(b.partial, b.chunk0, cap, cnt_, C, dacc, dphi);
+        c->launches++;
+        return B200NB_OK;
+    };
+    return run_targets(c, self, m, pts, FIELD_TI, batch, outs, work, launch);
+}
+
+// B200NB_EINVAL unless comp is non-NULL, n_comp is in [1, COMP_MAX] and every label is < n_comp or B200NB_NO_GROUP
+static int component_labels(b200nb_ctx *c, const char *what, const uint32_t *comp, uint32_t n_comp)
+{
+    if (!comp) return fail(c, B200NB_EINVAL, "%s: comp is NULL", what);
+    if (n_comp < 1 || n_comp > COMP_MAX) return fail(c, B200NB_EINVAL, "%s: n_comp = %u outside [1, %u]", what, n_comp, COMP_MAX);
+    for (uint64_t i = 0; i < c->n; ++i)
+        if (comp[i] >= n_comp && comp[i] != B200NB_NO_GROUP)
+            return fail(c, B200NB_EINVAL, "%s: comp[%llu] = %u is neither < n_comp nor B200NB_NO_GROUP", what, (unsigned long long)i, comp[i]);
+    return B200NB_OK;
+}
+
+int b200nb_component_field(b200nb_ctx *c, const uint32_t *comp, uint32_t n_comp, uint64_t n_points, const float *px,
+                           const float *py, const float *pz, float *acc, float *phi)
+{
+    if (!c) return B200NB_EINVAL;
+    if (!c->uploaded) return fail(c, B200NB_ESTATE, "component_field before upload");
+    if (n_points == 0) return B200NB_OK;
+    if (int rc = component_labels(c, "component_field", comp, n_comp)) return rc;
+    if (!px || !py || !pz) return fail(c, B200NB_EINVAL, "component_field: NULL point array");
+    const float *pts[3] = {px, py, pz};
+    return component_run(c, comp, n_comp, false, n_points, pts, acc, phi);
+}
+
+int b200nb_component_field_bodies(b200nb_ctx *c, const uint32_t *comp, uint32_t n_comp, float *acc, float *phi)
+{
+    if (!c) return B200NB_EINVAL;
+    if (!c->uploaded) return fail(c, B200NB_ESTATE, "component_field_bodies before upload");
+    if (int rc = component_labels(c, "component_field_bodies", comp, n_comp)) return rc;
+    return component_run(c, comp, n_comp, true, c->n, nullptr, acc, phi);
 }
 
 // k nearest bodies of the points (self == false) or of every body (self == true): [S][KB][cap] candidate d2 bits and
