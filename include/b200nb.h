@@ -364,6 +364,63 @@ int b200nb_set_tracers(b200nb_ctx *ctx, uint64_t n_tracers, const float *qx, con
 int b200nb_download_tracers(b200nb_ctx *ctx, float *qx, float *qy, float *qz, float *vx, float *vy, float *vz);
 uint64_t b200nb_n_tracers(const b200nb_ctx *ctx);
 
+/* ---- external potential --------------------------------------------------------------------------------------
+ * A static analytic host potential acting on the bodies and the tracers: the galaxy, halo or cluster that strips a
+ * satellite, at O(N) per step instead of the millions of live bodies it would take.  The reference has no counterpart.
+ * A context holds 0 to B200NB_EXTERNAL_MAX terms; Phi_ext is their sum and a_ext = -grad Phi_ext.  SI units, fp64
+ * parameters.  With d = p - centre evaluated in fp64 from the fp32 position p, r = |d| and R^2 = dx^2 + dy^2:
+ *   Plummer         Phi = -gm / sqrt(r^2 + a^2)                      a >= 0 (a = 0: a point mass)
+ *   Hernquist       Phi = -gm / (r + a)                              a > 0; a_ext = 0 exactly at r = 0
+ *   NFW             Phi = -gm ln(1 + r/a) / r  (-gm/a at r = 0)      a = r_s > 0; gm = G M_s = 4 pi G rho_0 r_s^3;
+ *                   a_ext = -gm mu(r/a) d / r^3, mu(x) = ln(1+x) - x/(1+x); a_ext = 0 exactly at r = 0
+ *   Miyamoto-Nagai  Phi = -gm / sqrt(R^2 + (a + sqrt(z^2 + b^2))^2) a >= 0, b > 0
+ *   logarithmic     Phi = gm/2 ln(R^2 + z^2/q^2 + r_c^2)             gm = v_0^2, a = r_c > 0, b = q > 0
+ * Every parameter must be finite, gm >= 0, reserved = 0, and b = 0 for Plummer, Hernquist and NFW.  The terms are summed
+ * in the order given, starting from +0, in explicitly rounded fp64 arithmetic whose operation order
+ * csrc/external_sm100.cuh states: a host restatement of that order compiled without contraction matches bit for bit
+ * wherever no log is involved (every Phi and a_ext of Plummer, Hernquist and Miyamoto-Nagai, the logarithmic a_ext),
+ * and within 1e-14 relative otherwise.  NFW's mu(x) uses a positive series below x = 0.1, so Phi and |a_ext| are within
+ * 1e-12 relative of exact for every x >= 0.
+ * Where the terms act, with e = a_ext in fp64 at the current fp32 position:
+ *  - bodies: the step rounds S + e to fp32, S the fp64 sum of the self-gravity partials (MUrB at q_n; leapfrog at the
+ *    positions of the force pass, a(x_0) and the closing kick at x_{n+1}).  The stored accelerations include e:
+ *    b200nb_download_accel, b200nb_accel and the leapfrog's a(x_n).  b200nb_integrate_host_accel adds nothing;
+ *  - tracers: a(p) = fp32(a_field(p) sums + e(p)), at the same instants as without terms;
+ *  - b200nb_energy and METRIC_ENERGY add sum_i m_i Phi_ext(q_i) in fp64; the other metrics are unchanged;
+ *  - b200nb_field, potential, tidal, component_field*, neighbors*, fof, group_potential and unbind keep describing the
+ *    bodies' own field; add b200nb_external_field for the total.
+ * With no terms a context makes the same launches and graphs, holds the same b200nb_allocated_bytes and gives
+ * bit-identical results to one that never had terms; with terms the step makes no extra launches.  The terms are
+ * kernel arguments, no device memory is set aside for them.
+ * b200nb_set_external replaces the set (n_terms = 0 removes it).  It is allowed before the first upload, joins the
+ * devices, drops the cached step graphs and invalidates the leapfrog's stored a(x_n) and tracer a(p), so the next
+ * leapfrog step evaluates them under the new terms.  Every rank must pass the same terms.  Not collective.
+ * Errors (B200NB_EINVAL; the previous terms stay in place): n_terms > B200NB_EXTERNAL_MAX, NULL terms with n_terms > 0,
+ * an unknown kind, reserved != 0, a parameter outside the rules above. */
+#define B200NB_EXTERNAL_MAX 8
+enum {
+    B200NB_EXT_PLUMMER = 0, B200NB_EXT_HERNQUIST = 1, B200NB_EXT_NFW = 2,
+    B200NB_EXT_MIYAMOTO_NAGAI = 3, B200NB_EXT_LOGARITHMIC = 4
+};
+typedef struct b200nb_external_term { /* 56 bytes */
+    int32_t kind, reserved; /* reserved must be 0 */
+    double gm;              /* G*M [m^3 s^-2]; NFW: G*M_s = 4 pi G rho_0 r_s^3; logarithmic: v_0^2 [m^2 s^-2] */
+    double a;               /* Plummer a | Hernquist a | NFW r_s | MN a | logarithmic r_c   [m] */
+    double b;               /* MN b [m] | logarithmic q (flattening); must be 0 for the other kinds */
+    double centre[3];       /* [m] */
+} b200nb_external_term;
+
+int b200nb_set_external(b200nb_ctx *ctx, uint32_t n_terms, const b200nb_external_term *terms);
+/* the current terms into out[0 .. *n_terms) (out has room for B200NB_EXTERNAL_MAX) */
+int b200nb_get_external(const b200nb_ctx *ctx, b200nb_external_term *out, uint32_t *n_terms);
+/* a_ext and Phi_ext in fp64 at n_points fp32 points (host SoA): bit for bit the e and Phi_ext the step uses there (the
+ * same device evaluator).  Any output may be NULL; n_points == 0 is a no-op.  Allowed before an upload; not collective
+ * (each rank evaluates all its points).  Points go through the context's grow-only query scratch in batches of at most
+ * 2^20, 44 B each (at most 44 MiB per call, counted in b200nb_allocated_bytes and shared with the field calls).  Joins
+ * the device of the first local shard.  Errors: B200NB_EINVAL for NULL point arrays with n_points > 0. */
+int b200nb_external_field(b200nb_ctx *ctx, uint64_t n_points, const float *px, const float *py, const float *pz,
+                          double *ax, double *ay, double *az, double *phi);
+
 /* Joins every device and communication stream.  main.cpp:353-371 only synchronises the current device, so the glue
  * calls this when more than one device is in use. */
 int b200nb_sync(b200nb_ctx *ctx);

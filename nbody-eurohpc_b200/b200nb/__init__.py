@@ -21,6 +21,8 @@ __all__ = [
     "B200Error", "Context", "SimulationNBodyB200", "B200Bodies", "init_bodies", "lib", "lib_path", "header_functions",
     "G_F32", "INTEGRATOR_MURB", "INTEGRATOR_LEAPFROG", "slice_length", "load_tab",
     "fof_groups", "NO_GROUP", "bound_groups", "component_budget", "COMPONENTS_MAX",
+    "ExternalTerm", "EXTERNAL_MAX", "EXT_PLUMMER", "EXT_HERNQUIST", "EXT_NFW", "EXT_MIYAMOTO_NAGAI", "EXT_LOGARITHMIC",
+    "plummer", "hernquist", "nfw", "miyamoto_nagai", "logarithmic",
 ]
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -32,6 +34,65 @@ NO_GROUP = 0xFFFFFFFF  # B200NB_NO_GROUP: a body with this label takes no part i
 COMPONENTS_MAX = 64    # n_comp of the component-field calls lies in [1, COMPONENTS_MAX]
 _FP = POINTER(c_float)
 _UP = POINTER(c_uint)
+_DP = POINTER(c_double)
+
+# ---- external potential (include/b200nb.h, "external potential")
+EXTERNAL_MAX = 8
+EXT_PLUMMER, EXT_HERNQUIST, EXT_NFW, EXT_MIYAMOTO_NAGAI, EXT_LOGARITHMIC = 0, 1, 2, 3, 4
+
+
+class ExternalTerm(ctypes.Structure):
+    """Mirror of b200nb_external_term (56 bytes): kind, reserved (0), gm, a, b, centre[3]; SI units, fp64."""
+    _fields_ = [("kind", ctypes.c_int32), ("reserved", ctypes.c_int32), ("gm", c_double), ("a", c_double),
+                ("b", c_double), ("centre", c_double * 3)]
+
+    def __repr__(self):
+        return (f"ExternalTerm(kind={self.kind}, gm={self.gm!r}, a={self.a!r}, b={self.b!r}, "
+                f"centre={tuple(self.centre)!r})")
+
+
+assert ctypes.sizeof(ExternalTerm) == 56 and ExternalTerm.centre.offset == 32
+
+
+def _term(kind, gm, a, b, centre, rules):
+    """Builds a term after checking the rules the library enforces (B200NB_EINVAL otherwise)."""
+    vals = [float(gm), float(a), float(b)]
+    c = [float(x) for x in centre]
+    if len(c) != 3 or not all(np.isfinite(vals + c)):
+        raise ValueError(f"parameters must be finite and centre three numbers, got gm={gm}, a={a}, b={b}, centre={centre}")
+    if vals[0] < 0:
+        raise ValueError(f"gm must be >= 0, got {gm}")
+    for ok, what in rules:
+        if not ok:
+            raise ValueError(what)
+    return ExternalTerm(kind, 0, vals[0], vals[1], vals[2], (c_double * 3)(*c))
+
+
+def plummer(gm, a, centre=(0.0, 0.0, 0.0)) -> ExternalTerm:
+    """Phi = -gm / sqrt(r^2 + a^2); a >= 0 (a = 0: a point mass)."""
+    return _term(EXT_PLUMMER, gm, a, 0.0, centre, [(float(a) >= 0, f"Plummer needs a >= 0, got {a}")])
+
+
+def hernquist(gm, a, centre=(0.0, 0.0, 0.0)) -> ExternalTerm:
+    """Phi = -gm / (r + a); a > 0."""
+    return _term(EXT_HERNQUIST, gm, a, 0.0, centre, [(float(a) > 0, f"Hernquist needs a > 0, got {a}")])
+
+
+def nfw(gm, r_s, centre=(0.0, 0.0, 0.0)) -> ExternalTerm:
+    """Phi = -gm ln(1 + r/r_s) / r with gm = G M_s = 4 pi G rho_0 r_s^3; r_s > 0."""
+    return _term(EXT_NFW, gm, r_s, 0.0, centre, [(float(r_s) > 0, f"NFW needs r_s > 0, got {r_s}")])
+
+
+def miyamoto_nagai(gm, a, b, centre=(0.0, 0.0, 0.0)) -> ExternalTerm:
+    """Phi = -gm / sqrt(R^2 + (a + sqrt(z^2 + b^2))^2); a >= 0, b > 0."""
+    return _term(EXT_MIYAMOTO_NAGAI, gm, a, b, centre,
+                 [(float(a) >= 0, f"Miyamoto-Nagai needs a >= 0, got {a}"), (float(b) > 0, f"Miyamoto-Nagai needs b > 0, got {b}")])
+
+
+def logarithmic(v0_sq, r_c, q, centre=(0.0, 0.0, 0.0)) -> ExternalTerm:
+    """Phi = v0_sq / 2 * ln(R^2 + z^2/q^2 + r_c^2); r_c > 0, q > 0."""
+    return _term(EXT_LOGARITHMIC, v0_sq, r_c, q, centre,
+                 [(float(r_c) > 0, f"logarithmic needs r_c > 0, got {r_c}"), (float(q) > 0, f"logarithmic needs q > 0, got {q}")])
 
 
 class B200Error(RuntimeError):
@@ -95,6 +156,9 @@ def lib() -> ctypes.CDLL:
         "b200nb_set_tracers": (c_int, [ctx, c_uint64] + [_FP] * 6),
         "b200nb_download_tracers": (c_int, [ctx] + [_FP] * 6),
         "b200nb_n_tracers": (c_uint64, [ctx]),
+        "b200nb_set_external": (c_int, [ctx, c_uint, POINTER(ExternalTerm)]),
+        "b200nb_get_external": (c_int, [ctx, POINTER(ExternalTerm), POINTER(c_uint)]),
+        "b200nb_external_field": (c_int, [ctx, c_uint64] + [_FP] * 3 + [_DP] * 4),
         "b200nb_sync": (c_int, [ctx]),
         "b200nb_n_bodies": (c_uint64, [ctx]),
         "b200nb_n_local_gpus": (c_int, [ctx]),
@@ -497,6 +561,34 @@ class Context:
     @property
     def n_tracers(self) -> int:
         return int(self._L.b200nb_n_tracers(self._ctx))
+
+    def set_external(self, terms):
+        """Replaces the static external potential (include/b200nb.h: b200nb_set_external): a sequence of at most
+        EXTERNAL_MAX terms made by plummer, hernquist, nfw, miyamoto_nagai or logarithmic.  An empty sequence removes it."""
+        terms = list(terms)
+        if len(terms) > EXTERNAL_MAX:
+            raise ValueError(f"at most {EXTERNAL_MAX} external terms, got {len(terms)}")
+        arr = (ExternalTerm * max(1, len(terms)))(*terms)
+        self._check(self._L.b200nb_set_external(self._ctx, len(terms), arr if terms else None), "b200nb_set_external")
+
+    @property
+    def external(self) -> list[ExternalTerm]:
+        """The current external terms, in order."""
+        arr, n = (ExternalTerm * EXTERNAL_MAX)(), c_uint()
+        self._check(self._L.b200nb_get_external(self._ctx, arr, byref(n)), "b200nb_get_external")
+        return [arr[i] for i in range(n.value)]
+
+    def external_field(self, px, py, pz) -> tuple[np.ndarray, np.ndarray, np.ndarray, np.ndarray]:
+        """Acceleration and potential of the external terms at fp32 points, evaluated on the device: bit for bit what the
+        step adds there (include/b200nb.h: b200nb_external_field).  Returns (ax, ay, az, phi), float64."""
+        p = [_f32(a) for a in (px, py, pz)]
+        if any(a.ndim != 1 for a in p) or len({a.shape for a in p}) != 1:
+            raise ValueError(f"expected three 1-D arrays of equal length, got {[a.shape for a in p]}")
+        m = p[0].shape[0]
+        out = [np.empty(m, dtype=np.float64) for _ in range(4)]
+        self._check(self._L.b200nb_external_field(self._ctx, m, *[_p(a) for a in p], *[o.ctypes.data_as(_DP) for o in out]),
+                    "b200nb_external_field")
+        return out[0], out[1], out[2], out[3]
 
     def sync(self):
         self._check(self._L.b200nb_sync(self._ctx), "b200nb_sync")

@@ -13,6 +13,7 @@
 #include <nccl.h>
 
 #include <cfloat>
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -29,6 +30,7 @@
 #include "tidal_sm100.cuh"
 #include "components_sm100.cuh"
 #include "integrate_sm100.cuh"
+#include "external_sm100.cuh"
 #include "plan.hpp"
 // The default force-kernel variant once more, as a cubin whose hot loop has been re-ordered after ptxas by
 // tools/sass_resched.py (same instructions, same registers, same arithmetic: bit-identical results, ~5 % faster; the
@@ -222,6 +224,7 @@ struct b200nb_ctx {
     uint64_t m_tracers = 0, tr_T = 0;
     uint32_t tr_cap = 0;
     bool tr_acc_valid = false;
+    ExtTerms ext{}; // the external potential (b200nb_set_external); ext.n == 0: none
     uint64_t launches = 0;
     std::string err;
 };
@@ -737,7 +740,11 @@ int enqueue_integrate(b200nb_ctx *c, int mode, float dt)
             const uint32_t nbr = c->nblk_total - nbs;
             a.sk[1] = SkRows{(uint64_t)n_itiles * nbr, c->sk_grid, nbr, c->sk_rows_own};
         }
-        integrate_kernel<<<(s.n_local + 255) / 256, 256, 0, s.s_compute>>>(a);
+        // caller-supplied accelerations (IM_MURB_STORED) already are the whole acceleration: no terms added
+        if (c->ext.n > 0 && mode != IM_MURB_STORED)
+            integrate_kernel<true><<<(s.n_local + 255) / 256, 256, 0, s.s_compute>>>(a, c->ext);
+        else
+            integrate_kernel<false><<<(s.n_local + 255) / 256, 256, 0, s.s_compute>>>(a, c->ext);
         c->launches++;
         CU(c, cudaGetLastError());
     }
@@ -983,7 +990,10 @@ int enqueue_tracer_pass(b200nb_ctx *c, int mode, float dt)
             TracerArgs u{};
             u.partial = s.tr_part; u.n_chunks = S; u.stride = c->tr_cap; u.count = cnt;
             u.tr = s.tr + base; u.T = c->tr_T; u.dt = dt; u.mode = mode;
-            tracer_update_kernel<<<(cnt + 255) / 256, 256, 0, s.s_compute>>>(u);
+            if (c->ext.n > 0)
+                tracer_update_kernel<true><<<(cnt + 255) / 256, 256, 0, s.s_compute>>>(u, c->ext);
+            else
+                tracer_update_kernel<false><<<(cnt + 255) / 256, 256, 0, s.s_compute>>>(u, c->ext);
             c->launches += 2;
             CU(c, cudaGetLastError());
         }
@@ -1390,9 +1400,10 @@ static int metric_sums(b200nb_ctx *c, double *raw)
         const uint32_t nb = (s.n_local + ENERGY_THREADS - 1) / ENERGY_THREADS;
         double part[MR_COUNT];
         if (nb > 0) {
-            energy_kernel<<<nb, ENERGY_THREADS, 0, s.s_compute>>>(s.bodies, s.vel, s.mass, (uint32_t)c->L, s.n_local,
-                                                                 (uint64_t)s.rank * c->L, c->nblk_total, c->soft2,
-                                                                 s.energy_blocks);
+            auto energy = c->ext.n > 0 ? energy_kernel<true> : energy_kernel<false>;
+            energy<<<nb, ENERGY_THREADS, 0, s.s_compute>>>(s.bodies, s.vel, s.mass, (uint32_t)c->L, s.n_local,
+                                                          (uint64_t)s.rank * c->L, c->nblk_total, c->soft2,
+                                                          s.energy_blocks, c->ext);
             energy_final_kernel<<<MR_COUNT, 256, 0, s.s_compute>>>(s.energy_blocks, nb, s.energy_out);
             c->launches += 2;
             CU(c, cudaGetLastError());
@@ -1879,6 +1890,93 @@ int b200nb_set_tracers(b200nb_ctx *c, uint64_t n_tracers, const float *qx, const
     c->m_tracers = n_tracers;
     c->tr_T = T;
     c->tr_cap = cap;
+    return B200NB_OK;
+}
+
+// ------------------------------------------------------------------------------------------------ external potential
+// A term is valid when its parameters obey the rules of include/b200nb.h, "external potential".
+static bool external_term_ok(const b200nb_external_term &t, char *why, size_t n)
+{
+    const bool finite = std::isfinite(t.gm) && std::isfinite(t.a) && std::isfinite(t.b) && std::isfinite(t.centre[0]) &&
+                        std::isfinite(t.centre[1]) && std::isfinite(t.centre[2]);
+    const char *bad = nullptr;
+    if (t.kind < B200NB_EXT_PLUMMER || t.kind > B200NB_EXT_LOGARITHMIC) bad = "unknown kind";
+    else if (t.reserved != 0) bad = "reserved must be 0";
+    else if (!finite) bad = "non-finite parameter";
+    else if (!(t.gm >= 0.0)) bad = "gm must be >= 0";
+    else if (t.kind == B200NB_EXT_PLUMMER && !(t.a >= 0.0)) bad = "Plummer needs a >= 0";
+    else if ((t.kind == B200NB_EXT_HERNQUIST || t.kind == B200NB_EXT_NFW) && !(t.a > 0.0)) bad = "needs a > 0";
+    else if (t.kind <= B200NB_EXT_NFW && t.b != 0.0) bad = "b must be 0 for this kind";
+    else if (t.kind == B200NB_EXT_MIYAMOTO_NAGAI && !(t.a >= 0.0 && t.b > 0.0)) bad = "Miyamoto-Nagai needs a >= 0, b > 0";
+    else if (t.kind == B200NB_EXT_LOGARITHMIC && !(t.a > 0.0 && t.b > 0.0)) bad = "logarithmic needs r_c = a > 0, q = b > 0";
+    if (bad) snprintf(why, n, "%s", bad);
+    return bad == nullptr;
+}
+
+int b200nb_set_external(b200nb_ctx *c, uint32_t n_terms, const b200nb_external_term *terms)
+{
+    if (!c) return B200NB_EINVAL;
+    if (n_terms > B200NB_EXTERNAL_MAX)
+        return fail(c, B200NB_EINVAL, "set_external: %u terms, at most %d", n_terms, B200NB_EXTERNAL_MAX);
+    if (n_terms > 0 && !terms) return fail(c, B200NB_EINVAL, "set_external: NULL terms");
+    for (uint32_t k = 0; k < n_terms; ++k) {
+        char why[96];
+        if (!external_term_ok(terms[k], why, sizeof why))
+            return fail(c, B200NB_EINVAL, "set_external: term %u (kind %d): %s", k, terms[k].kind, why);
+    }
+    DeviceGuard guard;
+    // steps in flight read the old terms, and captured step graphs bake them in
+    if (int rc = sync_all(c)) return rc;
+    for (auto &g : c->graphs)
+        if (g.exec) cudaGraphExecDestroy(g.exec);
+    c->graphs.clear();
+    ExtTerms e{};
+    for (uint32_t k = 0; k < n_terms; ++k) e.t[k] = terms[k];
+    e.n = n_terms;
+    c->ext = e;
+    c->acc_valid = false; // the leapfrog's a(x_n) and a(p) were taken under the old terms
+    c->tr_acc_valid = false;
+    return B200NB_OK;
+}
+
+int b200nb_get_external(const b200nb_ctx *c, b200nb_external_term *out, uint32_t *n_terms)
+{
+    if (!c || !out || !n_terms) return B200NB_EINVAL;
+    for (uint32_t k = 0; k < c->ext.n; ++k) out[k] = c->ext.t[k];
+    *n_terms = c->ext.n;
+    return B200NB_OK;
+}
+
+constexpr uint32_t EXTERNAL_BATCH = 1u << 20; // points per launch of b200nb_external_field: 44 MiB of scratch
+
+int b200nb_external_field(b200nb_ctx *c, uint64_t n_points, const float *px, const float *py, const float *pz, double *ax,
+                          double *ay, double *az, double *phi)
+{
+    if (!c) return B200NB_EINVAL;
+    if (n_points == 0) return B200NB_OK;
+    if (!px || !py || !pz) return fail(c, B200NB_EINVAL, "external_field: NULL point array");
+    DeviceGuard guard;
+    Shard &s = c->shards[0];
+    const uint32_t cap = (uint32_t)std::min<uint64_t>(EXTERNAL_BATCH, (n_points + 255) / 256 * 256);
+    if (int rc = query_scratch(c, s, (size_t)cap * (3 * 4 + 4 * 8))) return rc;
+    CU(c, cudaSetDevice(s.device));
+    double *dout = reinterpret_cast<double *>(s.query_buf);
+    float *dpts = reinterpret_cast<float *>(dout + 4 * (size_t)cap);
+    const float *pts[3] = {px, py, pz};
+    double *out[4] = {ax, ay, az, phi};
+    for (uint64_t base = 0; base < n_points; base += cap) {
+        const uint32_t cnt = (uint32_t)std::min<uint64_t>(cap, n_points - base);
+        for (int k = 0; k < 3; ++k)
+            CU(c, cudaMemcpyAsync(dpts + (size_t)k * cap, pts[k] + base, (size_t)cnt * 4, cudaMemcpyHostToDevice, s.s_compute));
+        external_field_kernel<<<(cnt + 255) / 256, 256, 0, s.s_compute>>>(c->ext, dpts, dpts + cap, dpts + 2 * (size_t)cap,
+                                                                          cnt, cap, dout);
+        c->launches++;
+        CU(c, cudaGetLastError());
+        for (int k = 0; k < 4; ++k)
+            if (out[k])
+                CU(c, cudaMemcpyAsync(out[k] + base, dout + (size_t)k * cap, (size_t)cnt * 8, cudaMemcpyDeviceToHost, s.s_compute));
+    }
+    CU(c, cudaStreamSynchronize(s.s_compute));
     return B200NB_OK;
 }
 

@@ -10,6 +10,7 @@
 // are fused so one step is: force pass -> one integrator kernel.
 #pragma once
 #include "force_sm100.cuh"
+#include "external_sm100.cuh"
 
 namespace b200nb {
 
@@ -50,7 +51,10 @@ struct IntegrateArgs {
     SkRows sk[2];
 };
 
-__global__ void __launch_bounds__(256) integrate_kernel(const IntegrateArgs a)
+// EXT: the fp64 sum is rounded together with the external acceleration at the body's current position (include/b200nb.h,
+// "external potential"); <false> ignores `ext` and is the kernel without terms.
+template <bool EXT>
+__global__ void __launch_bounds__(256) integrate_kernel(const IntegrateArgs a, const __grid_constant__ ExtTerms ext)
 {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= a.n_local) return;
@@ -79,6 +83,12 @@ __global__ void __launch_bounds__(256) integrate_kernel(const IntegrateArgs a)
                     sx += (double)p[i]; sy += (double)p[P + i]; sz += (double)p[2 * P + i];
                 }
             }
+        }
+        if constexpr (EXT) {
+            const size_t g = a.first + i;
+            double e[3], phi;
+            ext_eval(ext, a.bodies[blk_index(g, 0)], a.bodies[blk_index(g, 1)], a.bodies[blk_index(g, 2)], e, &phi);
+            sx = __dadd_rn(sx, e[0]); sy = __dadd_rn(sy, e[1]); sz = __dadd_rn(sz, e[2]);
         }
         ax = (float)sx; ay = (float)sy; az = (float)sz;
         a.acc[i] = ax; a.acc[L + i] = ay; a.acc[2 * L + i] = az;
@@ -190,12 +200,14 @@ __device__ __forceinline__ float rsqrt_nr(float d)
     return y * fmaf(-0.5f * d, y * y, 1.5f);
 }
 
-// block_out[row * n_blocks + block]
+// block_out[row * n_blocks + block].  EXT: the energy row adds m_i Phi_ext(q_i); <false> ignores `ext`.
+template <bool EXT>
 __global__ void __launch_bounds__(ENERGY_THREADS) energy_kernel(const float *__restrict__ bodies,
                                                                 const float *__restrict__ vel,
                                                                 const float *__restrict__ mass, uint32_t L,
                                                                 uint32_t n_local, uint64_t first, uint32_t nblk_total,
-                                                                float soft2, double *__restrict__ block_out)
+                                                                float soft2, double *__restrict__ block_out,
+                                                                const __grid_constant__ ExtTerms ext)
 {
     __shared__ __align__(16) float tile[BLK_FLOATS];
     __shared__ double warp_sums[MR_COUNT][ENERGY_THREADS / 32];
@@ -231,6 +243,11 @@ __global__ void __launch_bounds__(ENERGY_THREADS) energy_kernel(const float *__r
         const double v2 = vx * vx + vy * vy + vz * vz;
         const double w = m * (pot - self);
         r[MR_ENERGY] = 0.5 * m * v2 - 0.5 * w;
+        if constexpr (EXT) {
+            double e[3], phi;
+            ext_eval(ext, xi, yi, zi, e, &phi);
+            r[MR_ENERGY] = __dadd_rn(r[MR_ENERGY], __dmul_rn(m, phi));
+        }
         r[MR_LX] = m * (y * vz - z * vy);
         r[MR_LY] = m * (z * vx - x * vz);
         r[MR_LZ] = m * (x * vy - y * vx);

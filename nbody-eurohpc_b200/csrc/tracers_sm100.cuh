@@ -12,6 +12,7 @@
 // shard holds the full body array after the position exchange.
 #pragma once
 #include "field_sm100.cuh"
+#include "external_sm100.cuh"
 
 namespace b200nb {
 
@@ -30,13 +31,20 @@ struct TracerArgs {
     int mode;
 };
 
-// after each field_kernel batch: fixed-order fp64 sum, rounded once, then the update
-__global__ void __launch_bounds__(256) tracer_update_kernel(const TracerArgs a)
+// after each field_kernel batch: fixed-order fp64 sum, rounded once, then the update.  EXT: the sum is rounded together
+// with the external acceleration at the tracer's current position, as integrate_kernel<true> does for the bodies.
+template <bool EXT>
+__global__ void __launch_bounds__(256) tracer_update_kernel(const TracerArgs a, const __grid_constant__ ExtTerms ext)
 {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= a.count) return;
     double s[3];
     field_sum_rows<3>(a.partial, a.n_chunks, a.stride, i, s);
+    if constexpr (EXT) {
+        double e[3], phi;
+        ext_eval(ext, a.tr[i], a.tr[a.T + i], a.tr[2 * a.T + i], e, &phi);
+        s[0] = __dadd_rn(s[0], e[0]); s[1] = __dadd_rn(s[1], e[1]); s[2] = __dadd_rn(s[2], e[2]);
+    }
     const float ax = (float)s[0], ay = (float)s[1], az = (float)s[2];
     float *q = a.tr + i;
     const size_t T = a.T;
