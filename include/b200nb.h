@@ -283,6 +283,38 @@ int b200nb_neighbors_at(b200nb_ctx *ctx, uint64_t n_points, const float *px, con
 /* friends-of-friends groups of linking length b; group[n_bodies] = smallest body index of each body's group */
 int b200nb_fof(b200nb_ctx *ctx, float b, uint32_t *group);
 
+/* ---- phase-space friends-of-friends ---------------------------------------------------------------------------
+ * Friends-of-friends in positions AND velocities (6D FoF, Diemand et al. 2006; the first stage of Rockstar).  When two
+ * systems overlap in space, in a collision or a fly-by, position-only groups merge them into one; their bodies are close
+ * in space but far apart in velocity, so in phase space they stay apart.  Definition (fp32, round to nearest, no flush to
+ * zero): the scales are s_x = 1.0f / b_x and s_v = 1.0f / b_v, each a correctly rounded fp32 division (b = +inf gives 0,
+ * which switches that part of the metric off).  The scaled coordinates of body i are
+ *   X = x*s_x, Y = y*s_x, Z = z*s_x, U = vx*s_v, V = vy*s_v, W = vz*s_v   (each product rounded to fp32)
+ * of the current state, as b200nb_download_state returns it.  For bodies i != j, with dX = Xj - Xi, ..., dW = Wj - Wi:
+ *   d2 = dX*dX;  d2 = fmaf(dY, dY, d2);  d2 = fmaf(dZ, dZ, d2);  d2 = fmaf(dU, dU, d2);  d2 = fmaf(dV, dV, d2);
+ *   d2 = fmaf(dW, dW, d2);
+ * i and j are linked iff d2 <= 1.0f.  fp32 subtraction is exactly antisymmetric, so d2(i, j) and d2(j, i) are bitwise
+ * equal and the library visits each unordered pair from one side only.  Groups are the connected components; group[i] is
+ * the SMALLEST body index in i's group: a pure function of the fp32 state and the two scales, independent of shard or
+ * rank count, chunking, reruns and the order of the device's atomics.  Mass plays no part; padding bodies are never
+ * linked; a non-finite scaled coordinate (a NaN or inf position or velocity, or an overflow for a tiny b) gives d2 NaN
+ * or +inf with everyone, so that body is alone.  If both b are +inf every body links to every other.
+ * If b_x is a power of two and b_v = +inf, the scaling is exact (away from subnormals and overflow, velocities finite)
+ * and the labels are b200nb_fof(b_x)'s: scaling by a power of two commutes with every rounding, so d2 is b200nb_fof's d2
+ * times s_x*s_x, and the velocity terms add exact zeros.
+ * b_x and b_v must be > 0 (+inf allowed); 0, negative values and NaN are B200NB_EINVAL.  The result feeds
+ * b200nb_unbind and b200nb.fof_groups like b200nb_fof's labels.  Same calling contract as b200nb_fof: ordered after a
+ * preceding asynchronous b200nb_step, joins the devices, collective when n_ranks > 1 (every rank receives all n_bodies
+ * labels), no change to the simulation state.  Device scratch is grow-only, owned by the context and counted in
+ * b200nb_allocated_bytes: with N_pad and P as in the friends-of-friends section, every shard holds the scaled array of
+ * all bodies, 24 * N_pad bytes, followed by b200nb_fof's forests (4 * N_pad bytes, or 4 * N_pad * P on the shard that
+ * merges and on every rank when each rank is its own process).  Errors: B200NB_ESTATE before an upload, B200NB_EINVAL
+ * for a NULL group or a b outside the range above. */
+
+/* phase-space friends-of-friends groups of linking lengths b_x (positions) and b_v (velocities); group[n_bodies] =
+ * smallest body index of each body's group */
+int b200nb_fof_phase(b200nb_ctx *ctx, float b_x, float b_v, uint32_t *group);
+
 /* ---- group potential and unbinding ----------------------------------------------------------------------------
  * Which bodies of a group are held together by gravity: the unbinding step of every halo or structure finder, whose
  * result (the bound mass of each structure) is the diagnostic of a merger or of tidal stripping.  The reference has no

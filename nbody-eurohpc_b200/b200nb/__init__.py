@@ -151,6 +151,7 @@ def lib() -> ctypes.CDLL:
         "b200nb_neighbors": (c_int, [ctx, c_uint, _UP, _FP]),
         "b200nb_neighbors_at": (c_int, [ctx, c_uint64, _FP, _FP, _FP, c_uint, _UP, _FP]),
         "b200nb_fof": (c_int, [ctx, c_float, _UP]),
+        "b200nb_fof_phase": (c_int, [ctx, c_float, c_float, _UP]),
         "b200nb_group_potential": (c_int, [ctx, _UP, _FP]),
         "b200nb_unbind": (c_int, [ctx, _UP, c_uint, _UP, _FP, _UP, POINTER(c_int)]),
         "b200nb_set_tracers": (c_int, [ctx, c_uint64] + [_FP] * 6),
@@ -476,6 +477,28 @@ class Context:
         self._check(self._L.b200nb_fof(self._ctx, b, group.ctypes.data_as(_UP)), "b200nb_fof")
         return group
 
+    @staticmethod
+    def _fof_phase_b(b, name) -> float:
+        """b as the fp32 value the library uses; ValueError unless b > 0 in fp32 (+inf allowed, a finite b that
+        overflows fp32 is not)."""
+        ok = not isinstance(b, bool) and isinstance(b, (int, float, np.integer, np.floating))
+        if ok:
+            with np.errstate(over="ignore"):
+                b32 = np.float32(b)
+            ok = bool(b32 > 0) and (bool(np.isfinite(b32)) or not np.isfinite(float(b)))
+        if not ok:
+            raise ValueError(f"{name} must be a real number > 0 in fp32 (+inf allowed), got {b!r}")
+        return float(b32)
+
+    def fof_phase(self, b_x, b_v) -> np.ndarray:
+        """Phase-space friends-of-friends groups of linking lengths b_x (positions, m) and b_v (velocities, m/s)
+        (include/b200nb.h: b200nb_fof_phase).  b = inf switches that part of the metric off.  Returns uint32[n]: the
+        smallest body index of each body's group, which fof_groups and bound_groups take as they take fof's."""
+        b_x, b_v = self._fof_phase_b(b_x, "b_x"), self._fof_phase_b(b_v, "b_v")
+        group = np.empty(self.n, dtype=np.uint32)
+        self._check(self._L.b200nb_fof_phase(self._ctx, b_x, b_v, group.ctypes.data_as(_UP)), "b200nb_fof_phase")
+        return group
+
     def _labels(self, group) -> np.ndarray:
         """group as the uint32[n] labels the library reads; ValueError unless 1-D, n long, integer, in [0, 2^32 - 1]."""
         g = np.asarray(group)
@@ -638,8 +661,8 @@ class Context:
 def fof_groups(group, m, state, min_size: int = 20) -> dict[str, np.ndarray]:
     """Catalogue of the friends-of-friends groups of at least `min_size` members (host, O(N)).
 
-    group: the labels of Context.fof; m: the masses; state: positions and velocities as Context.download_state returns
-    them.  Groups come sorted by size, largest first, then by root.  Returns arrays with one entry per group:
+    group: the labels of Context.fof or Context.fof_phase; m: the masses; state: positions and velocities as
+    Context.download_state returns them.  Groups come sorted by size, largest first, then by root.  Returns arrays with one entry per group:
       root uint32 (the smallest body index), size int64, mass float64, com float64[g, 3] (centre of mass),
       vel float64[g, 3] (mass-weighted mean velocity; both NaN for a group of zero mass).
     Sums are fp64 np.bincount sums, accumulated in body order, so the catalogue is reproducible."""

@@ -25,6 +25,7 @@
 #include "field_sm100.cuh"
 #include "neighbors_sm100.cuh"
 #include "fof_sm100.cuh"
+#include "phase_fof_sm100.cuh"
 #include "groups_sm100.cuh"
 #include "tracers_sm100.cuh"
 #include "tidal_sm100.cuh"
@@ -1752,47 +1753,49 @@ int b200nb_neighbors_at(b200nb_ctx *c, uint64_t n_points, const float *px, const
     return neighbors_run(c, false, n_points, pts, k, idx, dist);
 }
 
-// Friends-of-friends labels of every body (b200nb_fof); b2u: the bits of b * b in fp32.  Every shard links its own bodies
-// against all bodies into a forest of F = total_pad entries (fof_sm100.cuh).  In-process shards copy their forests to
+} // extern "C"
+
+namespace {
+
+// Scratch bytes of the friends-of-friends forests of shard i, from byte `off` of its query scratch: P forests of F =
+// total_pad entries on the shard that merges (every rank when each rank is its own process), one on every other shard.
+size_t fof_scratch_bytes(const b200nb_ctx *c, size_t i, size_t off)
+{
+    const bool gather = c->shards.size() != (size_t)c->n_ranks;
+    return off + 4 * c->total_pad * (gather || i == 0 ? (size_t)c->n_ranks : 1);
+}
+
+// The host side shared by the friends-of-friends calls (b200nb_fof, b200nb_fof_phase).  Every shard links its own bodies
+// against all bodies into a forest of F = total_pad entries at byte `off` of its query scratch (fof_sm100.cuh):
+// link(s, forest) enqueues that pass on s.s_compute when the shard has bodies.  In-process shards copy their forests to
 // shard 0, one rank per process all-gathers them; then shard 0, or every rank, folds forests 1..P-1 into forest 0,
-// finalizes it to labels and downloads them.  Scratch: P forests on the shard that merges (every rank when each rank is
-// its own process), one on every other shard.  Reads only the body array: state and cached step graphs are untouched.
-static int fof_run(b200nb_ctx *c, uint32_t b2u, uint32_t *group)
+// finalizes it to labels and downloads them.  Reads only the body array and the scratch: state and cached step graphs
+// are untouched.
+template <class Link>
+int fof_forests(b200nb_ctx *c, size_t off, uint32_t *group, Link link)
 {
     DeviceGuard guard;
     const bool gather = c->shards.size() != (size_t)c->n_ranks;
     const size_t F = c->total_pad;
     const uint32_t P = (uint32_t)c->n_ranks, n = (uint32_t)c->n;
-    const uint32_t nb = (n + BLK - 1) / BLK, stream = std::min<uint32_t>(nb / 2 + FOF_R, nb);
     for (size_t i = 0; i < c->shards.size(); ++i)
-        if (int rc = query_scratch(c, c->shards[i], 4 * F * (gather || i == 0 ? P : 1))) return rc;
+        if (int rc = query_scratch(c, c->shards[i], fof_scratch_bytes(c, i, off))) return rc;
     for (auto &s : c->shards) {
         CU(c, cudaSetDevice(s.device));
         // an asynchronous step may still be exchanging positions: the whole body array is read
         if (c->n_ranks > 1)
             if (int rc = wait_remote_positions(c, s)) return rc;
-        uint32_t *forest = reinterpret_cast<uint32_t *>(s.query_buf) + (gather ? s.rank * F : 0);
+        uint32_t *forest = reinterpret_cast<uint32_t *>(s.query_buf + off) + (gather ? s.rank * F : 0);
         fof_init_kernel<<<(unsigned)((F + 255) / 256), 256, 0, s.s_compute>>>(forest, (uint32_t)F);
         c->launches++;
         if (s.n_local > 0) {
-            FofArgs a{};
-            a.src = s.bodies;
-            a.parent = forest;
-            a.first = (uint32_t)((uint64_t)s.rank * c->L);
-            a.count = s.n_local;
-            a.n = n;
-            a.nb = nb;
-            a.stream = stream;
-            a.thr = b2u + 1;
-            const uint32_t tiles = (s.n_local + FOF_TI - 1) / FOF_TI;
-            a.n_chunks = fof_chunks(tiles, stream, (uint32_t)s.n_sms * FOF_MINB);
-            fof_link_kernel<<<dim3(tiles, a.n_chunks), FOF_THREADS, fof_smem_bytes(), s.s_compute>>>(a);
+            link(s, forest);
             c->launches++;
         }
         CU(c, cudaGetLastError());
     }
     Shard &m = c->shards[0];
-    uint32_t *forests = reinterpret_cast<uint32_t *>(m.query_buf);
+    uint32_t *forests = reinterpret_cast<uint32_t *>(m.query_buf + off);
     if (gather) {
         CU(c, cudaSetDevice(m.device));
         NC(c, g_nccl.AllGather(forests + m.rank * F, forests, F, ncclUint32, m.comm, m.s_compute));
@@ -1800,7 +1803,7 @@ static int fof_run(b200nb_ctx *c, uint32_t b2u, uint32_t *group)
         for (size_t i = 1; i < c->shards.size(); ++i) {
             Shard &s = c->shards[i];
             CU(c, cudaSetDevice(s.device));
-            CU(c, cudaMemcpyPeerAsync(forests + (size_t)s.rank * F, m.device, s.query_buf, s.device, 4 * F, s.s_compute));
+            CU(c, cudaMemcpyPeerAsync(forests + (size_t)s.rank * F, m.device, s.query_buf + off, s.device, 4 * F, s.s_compute));
             CU(c, cudaStreamSynchronize(s.s_compute)); // the merge on shard 0 reads the copy
         }
     }
@@ -1816,6 +1819,10 @@ static int fof_run(b200nb_ctx *c, uint32_t b2u, uint32_t *group)
     return sync_all(c);
 }
 
+} // namespace
+
+extern "C" {
+
 int b200nb_fof(b200nb_ctx *c, float b, uint32_t *group)
 {
     if (!c) return B200NB_EINVAL;
@@ -1825,7 +1832,100 @@ int b200nb_fof(b200nb_ctx *c, float b, uint32_t *group)
     if (!(b >= 0.f) || !(b2 <= FLT_MAX)) return fail(c, B200NB_EINVAL, "fof: b = %g must be >= 0 with b * b finite in fp32", (double)b);
     uint32_t b2u;
     memcpy(&b2u, &b2, 4);
-    return fof_run(c, b2u, group);
+    const uint32_t n = (uint32_t)c->n, nb = (n + BLK - 1) / BLK, stream = std::min<uint32_t>(nb / 2 + FOF_R, nb);
+    return fof_forests(c, 0, group, [&](Shard &s, uint32_t *forest) {
+        FofArgs a{};
+        a.src = s.bodies;
+        a.parent = forest;
+        a.first = (uint32_t)((uint64_t)s.rank * c->L);
+        a.count = s.n_local;
+        a.n = n;
+        a.nb = nb;
+        a.stream = stream;
+        a.thr = b2u + 1;
+        const uint32_t tiles = (s.n_local + FOF_TI - 1) / FOF_TI;
+        a.n_chunks = fof_chunks(tiles, stream, (uint32_t)s.n_sms * FOF_MINB);
+        fof_link_kernel<<<dim3(tiles, a.n_chunks), FOF_THREADS, fof_smem_bytes(), s.s_compute>>>(a);
+    });
+}
+
+} // extern "C"
+
+namespace {
+
+// Phase-space friends-of-friends labels (b200nb_fof_phase; phase_fof_sm100.cuh).  Scratch per shard: the 6-float array of
+// all N_pad = total_pad bodies (24 N_pad bytes), then fof_forests' forests.  Each shard packs its own slice from its
+// blocked positions and its own velocities; the slices are then replicated: in-process shards copy every slice to every
+// other shard (a plain copy when both share a device), one rank per process all-gathers them in place.  Each shard then
+// links its own bodies against all of them.
+int phase_fof_run(b200nb_ctx *c, float sx, float sv, uint32_t *group)
+{
+    DeviceGuard guard;
+    const bool gather = c->shards.size() != (size_t)c->n_ranks;
+    const size_t off = 24 * c->total_pad, slice = (size_t)6 * c->L; // floats of one shard's slice
+    const uint32_t L = (uint32_t)c->L, n = (uint32_t)c->n;
+    for (size_t i = 0; i < c->shards.size(); ++i)
+        if (int rc = query_scratch(c, c->shards[i], fof_scratch_bytes(c, i, off))) return rc;
+    for (auto &s : c->shards) {
+        CU(c, cudaSetDevice(s.device));
+        if (c->n_ranks > 1) // an asynchronous step may still be exchanging positions
+            if (int rc = wait_remote_positions(c, s)) return rc;
+        float *mine = reinterpret_cast<float *>(s.query_buf);
+        phase_fof_pack_kernel<<<(L + 255) / 256, 256, 0, s.s_compute>>>(s.bodies, s.vel, mine, (uint32_t)(s.rank * c->L), L,
+                                                                        s.n_local, sx, sv);
+        c->launches++;
+        CU(c, cudaGetLastError());
+    }
+    if (gather) {
+        Shard &s = c->shards[0];
+        float *arr = reinterpret_cast<float *>(s.query_buf);
+        CU(c, cudaSetDevice(s.device));
+        NC(c, g_nccl.AllGather(arr + (size_t)s.rank * slice, arr, slice, ncclFloat, s.comm, s.s_compute));
+    } else if (c->n_ranks > 1) {
+        if (int rc = sync_all(c)) return rc; // every slice is packed
+        for (auto &o : c->shards) { // into o, on o's stream: its link pass follows in stream order
+            CU(c, cudaSetDevice(o.device));
+            for (auto &s : c->shards) {
+                if (&s == &o) continue;
+                float *dst = reinterpret_cast<float *>(o.query_buf) + (size_t)s.rank * slice;
+                const float *src = reinterpret_cast<const float *>(s.query_buf) + (size_t)s.rank * slice;
+                if (s.device == o.device)
+                    CU(c, cudaMemcpyAsync(dst, src, slice * 4, cudaMemcpyDeviceToDevice, o.s_compute));
+                else
+                    CU(c, cudaMemcpyPeerAsync(dst, o.device, src, s.device, slice * 4, o.s_compute));
+            }
+        }
+    }
+    const uint32_t nb = (n + BLK - 1) / BLK, stream = std::min<uint32_t>(nb / 2 + PF_R, nb);
+    return fof_forests(c, off, group, [&](Shard &s, uint32_t *forest) {
+        PhaseFofArgs a{};
+        a.src = reinterpret_cast<const float *>(s.query_buf);
+        a.parent = forest;
+        a.first = (uint32_t)((uint64_t)s.rank * c->L);
+        a.count = s.n_local;
+        a.n = n;
+        a.nb = nb;
+        a.stream = stream;
+        const uint32_t tiles = (s.n_local + PF_TI - 1) / PF_TI;
+        a.n_chunks = fof_chunks(tiles, stream, (uint32_t)s.n_sms * PF_MINB);
+        phase_fof_link_kernel<<<dim3(tiles, a.n_chunks), PF_THREADS, phase_fof_smem_bytes(), s.s_compute>>>(a);
+    });
+}
+
+} // namespace
+
+extern "C" {
+
+int b200nb_fof_phase(b200nb_ctx *c, float b_x, float b_v, uint32_t *group)
+{
+    if (!c) return B200NB_EINVAL;
+    if (!c->uploaded) return fail(c, B200NB_ESTATE, "fof_phase before upload");
+    if (!group) return fail(c, B200NB_EINVAL, "fof_phase: group is NULL");
+    if (!(b_x > 0.f) || !(b_v > 0.f))
+        return fail(c, B200NB_EINVAL, "fof_phase: b_x = %g and b_v = %g must be > 0 (+inf allowed)", (double)b_x, (double)b_v);
+    // correctly rounded fp32 divisions (no fast-math here); 1 / +inf = 0 switches that part of the metric off
+    const float one = 1.0f, sx = one / b_x, sv = one / b_v;
+    return phase_fof_run(c, sx, sv, group);
 }
 
 int b200nb_set_tracers(b200nb_ctx *c, uint64_t n_tracers, const float *qx, const float *qy, const float *qz, const float *vx,
