@@ -10,7 +10,7 @@ PKG       := nbody-eurohpc_b200
 LIB       := $(PKG)/b200nb/libb200nb.so
 REF       ?= /root/reference
 
-all: lib oracle field_oracle neighbors_oracle fof_oracle groups_oracle tracers_oracle tidal_oracle components_oracle external_oracle phase_fof_oracle
+all: lib oracle field_oracle neighbors_oracle fof_oracle groups_oracle tracers_oracle tidal_oracle components_oracle external_oracle phase_fof_oracle scf_oracle
 
 # the default force-kernel variant with its hot loop re-ordered after ptxas (tools/sass_resched.py + the committed order)
 RESCHED_VARIANT := 32, 8, 2, 2, 1, false, 1, 8, 1
@@ -20,7 +20,7 @@ $(RESCHED_INC): tools/sass_resched.py $(RESCHED_ORDER) $(PKG)/csrc/force_sm100.c
 	mkdir -p $(dir $@) build/resched && python3 tools/sass_resched.py "$(RESCHED_VARIANT)" build/resched/default.cubin --order-in $(RESCHED_ORDER) --emit-header $@
 
 lib: $(LIB)
-$(LIB): $(PKG)/csrc/context.cu $(PKG)/csrc/host_ic.cpp $(PKG)/csrc/force_sm100.cuh $(PKG)/csrc/field_sm100.cuh $(PKG)/csrc/neighbors_sm100.cuh $(PKG)/csrc/fof_sm100.cuh $(PKG)/csrc/phase_fof_sm100.cuh $(PKG)/csrc/groups_sm100.cuh $(PKG)/csrc/tracers_sm100.cuh $(PKG)/csrc/tidal_sm100.cuh $(PKG)/csrc/components_sm100.cuh $(PKG)/csrc/external_sm100.cuh $(PKG)/csrc/integrate_sm100.cuh $(PKG)/csrc/plan.hpp include/b200nb.h $(RESCHED_INC)
+$(LIB): $(PKG)/csrc/context.cu $(PKG)/csrc/host_ic.cpp $(PKG)/csrc/force_sm100.cuh $(PKG)/csrc/field_sm100.cuh $(PKG)/csrc/neighbors_sm100.cuh $(PKG)/csrc/fof_sm100.cuh $(PKG)/csrc/phase_fof_sm100.cuh $(PKG)/csrc/groups_sm100.cuh $(PKG)/csrc/tracers_sm100.cuh $(PKG)/csrc/tidal_sm100.cuh $(PKG)/csrc/components_sm100.cuh $(PKG)/csrc/external_sm100.cuh $(PKG)/csrc/scf_sm100.cuh $(PKG)/csrc/integrate_sm100.cuh $(PKG)/csrc/plan.hpp include/b200nb.h $(RESCHED_INC)
 	$(NVCC) $(NVFLAGS) -shared -o $@ $(PKG)/csrc/context.cu $(PKG)/csrc/host_ic.cpp -ldl
 
 oracle: oracle/liboracle.so
@@ -80,6 +80,12 @@ external_oracle: build/libexternaloracle.so
 build/libexternaloracle.so: tests/external_oracle.c
 	mkdir -p build && $(ORACLE_CC) -O2 -ffp-contract=off -fPIC -shared -o $@ tests/external_oracle.c -lm
 
+# long-double restatement of the basis-function expansion (test infrastructure, beside the tests)
+scf_oracle: build/libscforacle.so
+build/libscforacle.so: tests/scf_oracle.c
+	mkdir -p build && ($(ORACLE_CC) -O2 -ffp-contract=off -fopenmp -fPIC -shared -o $@ tests/scf_oracle.c -lm || \
+	$(ORACLE_CC) -O2 -ffp-contract=off -fPIC -shared -o $@ tests/scf_oracle.c -lm)
+
 # reference-side artefacts (need $(REF); outputs only under oracle/_ref/)
 ref:
 	bash oracle/build_ref.sh $(REF)
@@ -89,6 +95,6 @@ build/kbench: tools/kbench.cu $(PKG)/csrc/force_sm100.cuh $(PKG)/csrc/plan.hpp
 	mkdir -p build && $(NVCC) $(ARCH) -O3 -std=c++17 -lineinfo -o $@ tools/kbench.cu -L/usr/local/cuda/lib64/stubs -lcuda
 
 clean:
-	rm -f $(LIB) oracle/liboracle.so build/kbench build/libfieldoracle.so build/libneighborsoracle.so build/libfoforacle.so build/libgroupsoracle.so build/libtracersoracle.so build/libtidaloracle.so build/libcomponentsoracle.so build/libexternaloracle.so build/libphasefoforacle.so; rm -rf oracle/_ref
+	rm -f $(LIB) oracle/liboracle.so build/kbench build/libfieldoracle.so build/libneighborsoracle.so build/libfoforacle.so build/libgroupsoracle.so build/libtracersoracle.so build/libtidaloracle.so build/libcomponentsoracle.so build/libexternaloracle.so build/libphasefoforacle.so build/libscforacle.so; rm -rf oracle/_ref
 
-.PHONY: all lib oracle field_oracle neighbors_oracle fof_oracle groups_oracle tracers_oracle tidal_oracle components_oracle external_oracle phase_fof_oracle ref kbench clean
+.PHONY: all lib oracle field_oracle neighbors_oracle fof_oracle groups_oracle tracers_oracle tidal_oracle components_oracle external_oracle phase_fof_oracle scf_oracle ref kbench clean

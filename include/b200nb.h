@@ -453,6 +453,69 @@ int b200nb_get_external(const b200nb_ctx *ctx, b200nb_external_term *out, uint32
 int b200nb_external_field(b200nb_ctx *ctx, uint64_t n_points, const float *px, const float *py, const float *pz,
                           double *ax, double *ay, double *az, double *phi);
 
+/* ---- basis-function expansion ---------------------------------------------------------------------------------
+ * The mean field of a structure in a few hundred numbers: the self-consistent-field (SCF) expansion of Hernquist &
+ * Ostriker (1992, ApJ 386, 375) in the normalisation of Lowing et al. (2011, MNRAS 416, 2697), the basis gala, AGAMA and
+ * galpy provide.  Uses: l = 2 / m = 2 power (triaxiality, bars), l = 1 lopsidedness and monopole drift over time; a
+ * potential without sqrt(N) sampling noise and without softening (rotation curves, escape speeds, tracer orbits).  The
+ * reference has no counterpart.  Inputs: scale radius a > 0 [m], centre c (fp64 [3]), nmax in [0, 31], lmax in [0, 15].
+ * For a body or point p, with d = p - c in fp64 (from the fp32 coordinates): r = |d|, s = r / a, xi = (s - 1)/(s + 1),
+ * cos theta = d_z / r, phi the azimuth of (d_x, d_y).
+ *   Phi~_nl(s) = - s^l (1+s)^-(2l+1) C_n^(2l+3/2)(xi)                      (Gegenbauer polynomial)
+ *   K_nl       = n(n+4l+3)/2 + (l+1)(2l+1)
+ *   A~_nl      = - 2^(8l+6) n! (n+2l+3/2) Gamma(2l+3/2)^2 / (4 pi K_nl Gamma(n+4l+3))
+ *   N_lm       = (2l+1) (l-m)! / (l+m)!
+ *   S_nlm      = (2 - delta_m0) A~_nl N_lm (1/a) sum_k (G m_k) Phi~_nl(s_k) P_l^m(cos theta_k) cos(m phi_k)
+ *   T_nlm      = the same with sin(m phi_k)                                 (T_nl0 = 0)
+ *   Phi(p)     = sum_{n<=nmax, l<=lmax, m<=l} Phi~_nl(s) P_l^m(cos theta) [S_nlm cos(m phi) + T_nlm sin(m phi)]
+ *   a(p)       = -grad Phi(p)
+ * P_l^m carries the Condon-Shortley phase (as scipy.special.lpmv); it cancels between coefficients and evaluation.  G m_k
+ * is the fp32 G*m fold of the force pass, so S and T are in m^2/s^2.  A Hernquist sphere of mass M and scale a has
+ * S_000 = GM/a and every other coefficient 0, and then Phi = -GM/(r + a).  Members: the bodies k < n_bodies with
+ * group[k] == label (group == NULL: every body); padding bodies never take part.  A body at r = 0 adds to l = 0 only
+ * (s^l = 0), without a NaN from its undefined angles.  A member at a non-finite position, or with a non-finite G*m,
+ * makes every S and every T with m > 0 NaN (T_nl0 stays 0); nothing is filtered.  Layout of S and T: packed
+ * [nmax+1][(lmax+1)(lmax+2)/2], index n*(lmax+1)(lmax+2)/2 + l(l+1)/2 + m.
+ * Evaluation: at r = 0 (the centre itself) Phi is the l = 0 sum and a = 0, since the l = 0 term has a cusp there whose
+ * direction is undefined; everywhere else, the z axis included, Phi and a are the formulas above, finite.
+ * Promises:
+ *  1. pure function: the coefficients depend only on the fp32 positions and G*m of the members, the member mask, nmax,
+ *     lmax, a and c.  Bit-identical on reruns, for any shard or rank count, straight after an asynchronous step of
+ *     either integrator or a graph-replayed one, and when non-members are relabelled; group == NULL is bit-identical to
+ *     a label array that puts every body in `label`;
+ *  2. truncation: the coefficients of (nmax', lmax') <= (nmax, lmax) are the matching entries of the larger call, bit
+ *     for bit (the summation order of a coefficient does not depend on nmax or lmax);
+ *  3. locality: Phi and a at a point depend only on the point, the coefficients, nmax, lmax, a and c: bit-identical
+ *     under any batching and whatever the other points of the call;
+ *  4. accuracy: fp64 recurrences (Gegenbauer in n, reduced associated Legendre in l) with host tables rounded once from
+ *     long double; every coefficient is within 1e-12 of its cancellation-free scale sum_k |term_k| of an exact
+ *     evaluation, and Phi and each component of a within 1e-12 of sum |term| at the point.
+ * Calling contract of the field section: both calls are ordered after a preceding asynchronous b200nb_step, join the
+ * device of the first local shard and change nothing in the state (positions, velocities, the stored accelerations, the
+ * leapfrog's a(x_n), the tracers, the external terms, cached step graphs).  Neither is collective:
+ * b200nb_scf_coefficients runs on the first local shard over its replicated body array, so every rank computes the same
+ * result on its own device; b200nb_scf_field is allowed before an upload.  Device scratch is grow-only, owned by the
+ * context, counted in b200nb_allocated_bytes and shared with the field calls.  With K = (nmax+1)(lmax+1)(lmax+2)/2
+ * (at most 4352), C = min(512, ceil(n_bodies / 64)) chunks and r(x) = x rounded up to a multiple of 256:
+ *   coefficients  r(12952) + r(8 K) + r(16 K) + r(16 K C) + r(4 n_bodies) [only with group]  bytes: at most 34 MiB of
+ *                 partial rows;
+ *   field         r(12952) + r(16 K) + 44 B per point of a batch of B = min(2^20, n_points rounded up to 256): at most
+ *                 44 MiB + 81 KiB.
+ * Kernel launches: two per coefficient call; one per batch of the field call.
+ * Errors: B200NB_ESTATE for coefficients before an upload; B200NB_EINVAL for nmax or lmax out of range, a not finite or
+ * <= 0, a NULL or non-finite centre, NULL S or T, and NULL point arrays with n_points > 0 (n_points == 0 is a no-op). */
+#define B200NB_SCF_NMAX 31
+#define B200NB_SCF_LMAX 15
+
+/* coefficients of the bodies with group[i] == label (group == NULL: all bodies); S, T packed [nmax+1][(lmax+1)(lmax+2)/2],
+ * index n*(lmax+1)(lmax+2)/2 + l(l+1)/2 + m */
+int b200nb_scf_coefficients(b200nb_ctx *ctx, uint32_t nmax, uint32_t lmax, double a, const double centre[3],
+                            const uint32_t *group, uint32_t label, double *S, double *T);
+/* Phi and a of an expansion at n_points fp32 points (host SoA), fp64 outputs, any output may be NULL */
+int b200nb_scf_field(b200nb_ctx *ctx, uint32_t nmax, uint32_t lmax, double a, const double centre[3], const double *S,
+                     const double *T, uint64_t n_points, const float *px, const float *py, const float *pz,
+                     double *ax, double *ay, double *az, double *phi);
+
 /* Joins every device and communication stream.  main.cpp:353-371 only synchronises the current device, so the glue
  * calls this when more than one device is in use. */
 int b200nb_sync(b200nb_ctx *ctx);

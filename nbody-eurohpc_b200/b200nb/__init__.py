@@ -22,7 +22,7 @@ __all__ = [
     "G_F32", "INTEGRATOR_MURB", "INTEGRATOR_LEAPFROG", "slice_length", "load_tab",
     "fof_groups", "NO_GROUP", "bound_groups", "component_budget", "COMPONENTS_MAX",
     "ExternalTerm", "EXTERNAL_MAX", "EXT_PLUMMER", "EXT_HERNQUIST", "EXT_NFW", "EXT_MIYAMOTO_NAGAI", "EXT_LOGARITHMIC",
-    "plummer", "hernquist", "nfw", "miyamoto_nagai", "logarithmic",
+    "plummer", "hernquist", "nfw", "miyamoto_nagai", "logarithmic", "SCF_NMAX", "SCF_LMAX",
 ]
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -32,6 +32,7 @@ INTEGRATOR_MURB, INTEGRATOR_LEAPFROG = 0, 1
 OK, EINVAL, ECUDA, ENCCL, ESTATE = 0, 1, 2, 3, 4
 NO_GROUP = 0xFFFFFFFF  # B200NB_NO_GROUP: a body with this label takes no part in the group calls
 COMPONENTS_MAX = 64    # n_comp of the component-field calls lies in [1, COMPONENTS_MAX]
+SCF_NMAX, SCF_LMAX = 31, 15  # B200NB_SCF_NMAX, B200NB_SCF_LMAX: the largest expansion of the basis-function calls
 _FP = POINTER(c_float)
 _UP = POINTER(c_uint)
 _DP = POINTER(c_double)
@@ -160,6 +161,8 @@ def lib() -> ctypes.CDLL:
         "b200nb_set_external": (c_int, [ctx, c_uint, POINTER(ExternalTerm)]),
         "b200nb_get_external": (c_int, [ctx, POINTER(ExternalTerm), POINTER(c_uint)]),
         "b200nb_external_field": (c_int, [ctx, c_uint64] + [_FP] * 3 + [_DP] * 4),
+        "b200nb_scf_coefficients": (c_int, [ctx, c_uint, c_uint, c_double, _DP, _UP, c_uint, _DP, _DP]),
+        "b200nb_scf_field": (c_int, [ctx, c_uint, c_uint, c_double, _DP, _DP, _DP, c_uint64] + [_FP] * 3 + [_DP] * 4),
         "b200nb_sync": (c_int, [ctx]),
         "b200nb_n_bodies": (c_uint64, [ctx]),
         "b200nb_n_local_gpus": (c_int, [ctx]),
@@ -252,6 +255,20 @@ class PinnedArrays:
             self.close()
         except Exception:
             pass
+
+
+def _scf_unpack(packed: np.ndarray, nmax: int, lmax: int) -> np.ndarray:
+    """the ABI's packed [nmax+1][(lmax+1)(lmax+2)/2] coefficients -> [nmax+1][lmax+1][lmax+1], zeros where m > l"""
+    P = packed.reshape(nmax + 1, -1)
+    out = np.zeros((nmax + 1, lmax + 1, lmax + 1))
+    for l in range(lmax + 1):
+        out[:, l, :l + 1] = P[:, l * (l + 1) // 2:l * (l + 1) // 2 + l + 1]
+    return out
+
+
+def _scf_pack(C: np.ndarray) -> np.ndarray:
+    """[nmax+1][lmax+1][lmax+1] -> the ABI's packed [nmax+1][(lmax+1)(lmax+2)/2] (entries with m > l are not read)"""
+    return np.ascontiguousarray(np.concatenate([C[:, l, :l + 1] for l in range(C.shape[1])], axis=1), np.float64)
 
 
 class Context:
@@ -611,6 +628,53 @@ class Context:
         out = [np.empty(m, dtype=np.float64) for _ in range(4)]
         self._check(self._L.b200nb_external_field(self._ctx, m, *[_p(a) for a in p], *[o.ctypes.data_as(_DP) for o in out]),
                     "b200nb_external_field")
+        return out[0], out[1], out[2], out[3]
+
+    @staticmethod
+    def _scf_args(nmax, lmax, a, centre) -> tuple[int, int, float, np.ndarray]:
+        """(nmax, lmax, a, centre) as the library reads them; ValueError unless nmax in [0, SCF_NMAX], lmax in
+        [0, SCF_LMAX], a finite and > 0 and the centre three finite numbers."""
+        for name, v, hi in (("nmax", nmax, SCF_NMAX), ("lmax", lmax, SCF_LMAX)):
+            if isinstance(v, bool) or not isinstance(v, (int, np.integer)) or not 0 <= int(v) <= hi:
+                raise ValueError(f"{name} must be an integer in [0, {hi}], got {v!r}")
+        if isinstance(a, bool) or not isinstance(a, (int, float, np.integer, np.floating)) or not (np.isfinite(a) and a > 0):
+            raise ValueError(f"a must be a finite number > 0, got {a!r}")
+        c = np.ascontiguousarray(centre, dtype=np.float64)
+        if c.shape != (3,) or not np.all(np.isfinite(c)):
+            raise ValueError(f"centre must be three finite numbers, got {centre!r}")
+        return int(nmax), int(lmax), float(a), c
+
+    def scf_coefficients(self, nmax, lmax, a, centre=(0.0, 0.0, 0.0), group=None, label=0) -> tuple[np.ndarray, np.ndarray]:
+        """Hernquist-Ostriker basis-function expansion of the bodies with group == label (group None: every body) about
+        `centre` with scale radius a (include/b200nb.h: b200nb_scf_coefficients).  Returns (S, T), float64[nmax+1, lmax+1,
+        lmax+1] in m^2/s^2, zero where m > l (gala's layout)."""
+        nmax, lmax, a, c = self._scf_args(nmax, lmax, a, centre)
+        g = None if group is None else self._labels(group)
+        if isinstance(label, bool) or not isinstance(label, (int, np.integer)) or not 0 <= int(label) <= NO_GROUP:
+            raise ValueError(f"label must be an integer in [0, 2^32 - 1], got {label!r}")
+        K = (nmax + 1) * (lmax + 1) * (lmax + 2) // 2
+        S, T = np.empty(K), np.empty(K)
+        self._check(self._L.b200nb_scf_coefficients(self._ctx, nmax, lmax, a, c.ctypes.data_as(_DP),
+                                                    None if g is None else g.ctypes.data_as(_UP), int(label),
+                                                    S.ctypes.data_as(_DP), T.ctypes.data_as(_DP)), "b200nb_scf_coefficients")
+        return _scf_unpack(S, nmax, lmax), _scf_unpack(T, nmax, lmax)
+
+    def scf_field(self, S, T, a, centre, px, py, pz) -> tuple[np.ndarray, np.ndarray, np.ndarray, np.ndarray]:
+        """Acceleration and potential of an expansion (S, T float64[nmax+1, lmax+1, lmax+1], as scf_coefficients returns
+        them) at fp32 points (include/b200nb.h: b200nb_scf_field).  Returns (ax, ay, az, phi), float64."""
+        S, T = np.asarray(S), np.asarray(T)
+        if S.ndim != 3 or S.shape != T.shape or S.shape[1] != S.shape[2] or S.dtype.kind != "f" or T.dtype.kind != "f":
+            raise ValueError(f"S and T must be float arrays of one shape (nmax+1, lmax+1, lmax+1), got {S.shape}, {T.shape}")
+        nmax, lmax, a, c = self._scf_args(S.shape[0] - 1, S.shape[1] - 1, a, centre)
+        p = [_f32(x) for x in (px, py, pz)]
+        if any(x.ndim != 1 for x in p) or len({x.shape for x in p}) != 1:
+            raise ValueError(f"expected three 1-D arrays of equal length, got {[x.shape for x in p]}")
+        m = p[0].shape[0]
+        out = [np.empty(m, dtype=np.float64) for _ in range(4)]
+        Sp, Tp = _scf_pack(S), _scf_pack(T)
+        self._check(self._L.b200nb_scf_field(self._ctx, nmax, lmax, a, c.ctypes.data_as(_DP), Sp.ctypes.data_as(_DP),
+                                             Tp.ctypes.data_as(_DP), m, *[_p(x) for x in p],
+                                             *[o.ctypes.data_as(_DP) for o in out]), "b200nb_scf_field")
         return out[0], out[1], out[2], out[3]
 
     def sync(self):

@@ -32,6 +32,7 @@
 #include "components_sm100.cuh"
 #include "integrate_sm100.cuh"
 #include "external_sm100.cuh"
+#include "scf_sm100.cuh"
 #include "plan.hpp"
 // The default force-kernel variant once more, as a cubin whose hot loop has been re-ordered after ptxas by
 // tools/sass_resched.py (same instructions, same registers, same arithmetic: bit-identical results, ~5 % faster; the
@@ -2123,6 +2124,177 @@ int b200nb_download_tracers(b200nb_ctx *c, float *qx, float *qy, float *qz, floa
 }
 
 uint64_t b200nb_n_tracers(const b200nb_ctx *c) { return c ? c->m_tracers : 0; }
+
+} // extern "C"
+
+// ------------------------------------------------------------------------------------------------ basis-function expansion
+namespace {
+
+size_t round256(size_t x) { return (x + 255) / 256 * 256; }
+
+// The recurrence tables of scf_sm100.cuh, in long double, each entry rounded once.
+void scf_tables(ScfTables &t)
+{
+    memset(&t, 0, sizeof t);
+    for (int l = 0; l <= SCF_LMAX; ++l) {
+        const long double alpha = 2.0L * l + 1.5L;
+        for (int n = 1; n <= SCF_NMAX; ++n) {
+            t.ga[l][n] = (double)(2.0L * (n + alpha - 1.0L) / n);
+            t.gb[l][n] = (double)((n + 2.0L * alpha - 2.0L) / n);
+        }
+    }
+    long double dfact = 1.0L; // (2m - 1)!!
+    for (int m = 0; m <= SCF_LMAX + 1; ++m) {
+        if (m > 0) dfact *= 2.0L * m - 1.0L;
+        t.qs[m] = (double)(m % 2 ? -dfact : dfact);
+        for (int l = m + 1; l <= SCF_LMAX + 1; ++l) {
+            t.qa[l][m] = (double)((2.0L * l - 1.0L) / (l - m));
+            t.qb[l][m] = (double)((l + m - 1.0L) / (l - m));
+        }
+    }
+}
+
+// F_nlm = (2 - delta_m0) A~_nl N_lm / a, packed as the coefficients (include/b200nb.h), in long double
+void scf_norms(uint32_t nmax, uint32_t lmax, double a, std::vector<double> &F)
+{
+    const uint32_t LM = (lmax + 1) * (lmax + 2) / 2;
+    F.assign((size_t)(nmax + 1) * LM, 0.0);
+    for (uint32_t n = 0; n <= nmax; ++n)
+        for (uint32_t l = 0; l <= lmax; ++l) {
+            const long double K = 0.5L * n * (n + 4.0L * l + 3.0L) + (l + 1.0L) * (2.0L * l + 1.0L);
+            const long double lg = (8.0L * l + 6.0L) * logl(2.0L) + lgammal(n + 1.0L) + logl(n + 2.0L * l + 1.5L) +
+                                   2.0L * lgammal(2.0L * l + 1.5L) - logl(4.0L * 3.14159265358979323846264338327950288L * K) -
+                                   lgammal(n + 4.0L * l + 3.0L);
+            const long double At = -expl(lg);
+            long double ratio = 1.0L; // (l - m)! / (l + m)!
+            for (uint32_t m = 0; m <= l; ++m) {
+                if (m > 0) ratio /= (long double)(l + m) * (long double)(l - m + 1);
+                F[(size_t)n * LM + l * (l + 1) / 2 + m] = (double)((m ? 2.0L : 1.0L) * At * (2.0L * l + 1.0L) * ratio / a);
+            }
+        }
+}
+
+int scf_check(b200nb_ctx *c, const char *what, uint32_t nmax, uint32_t lmax, double a, const double *centre)
+{
+    if (nmax > (uint32_t)SCF_NMAX || lmax > (uint32_t)SCF_LMAX)
+        return fail(c, B200NB_EINVAL, "%s: nmax = %u and lmax = %u must lie in [0, %d] and [0, %d]", what, nmax, lmax, SCF_NMAX,
+                    SCF_LMAX);
+    if (!(std::isfinite(a) && a > 0.0)) return fail(c, B200NB_EINVAL, "%s: a = %g must be finite and > 0", what, a);
+    if (!centre) return fail(c, B200NB_EINVAL, "%s: centre is NULL", what);
+    if (!(std::isfinite(centre[0]) && std::isfinite(centre[1]) && std::isfinite(centre[2])))
+        return fail(c, B200NB_EINVAL, "%s: non-finite centre", what);
+    return B200NB_OK;
+}
+
+} // namespace
+
+extern "C" {
+
+int b200nb_scf_coefficients(b200nb_ctx *c, uint32_t nmax, uint32_t lmax, double a, const double centre[3], const uint32_t *group,
+                            uint32_t label, double *S, double *T)
+{
+    if (!c) return B200NB_EINVAL;
+    if (int rc = scf_check(c, "scf_coefficients", nmax, lmax, a, centre)) return rc;
+    if (!S || !T) return fail(c, B200NB_EINVAL, "scf_coefficients: S or T is NULL");
+    if (!c->uploaded) return fail(c, B200NB_ESTATE, "scf_coefficients before upload");
+    DeviceGuard guard;
+    Shard &s = c->shards[0];
+    const uint32_t n = (uint32_t)c->n, K = (nmax + 1) * (lmax + 1) * (lmax + 2) / 2, n_chunks = scf_chunks(n);
+    ScfTables tab;
+    scf_tables(tab);
+    std::vector<double> F;
+    scf_norms(nmax, lmax, a, F);
+    // scratch: tables | F | [S | T] | partial rows | labels
+    const size_t o_f = round256(sizeof(ScfTables)), o_out = o_f + round256(8 * (size_t)K), o_part = o_out + round256(16 * (size_t)K),
+                 o_grp = o_part + round256((size_t)n_chunks * 16 * K), bytes = o_grp + (group ? round256(4 * (size_t)n) : 0);
+    if (int rc = query_scratch(c, s, bytes)) return rc;
+    CU(c, cudaSetDevice(s.device));
+    if (c->n_ranks > 1) // an asynchronous step may still be exchanging positions: the whole body array is read
+        if (int rc = wait_remote_positions(c, s)) return rc;
+    unsigned char *buf = s.query_buf;
+    CU(c, cudaMemcpyAsync(buf, &tab, sizeof tab, cudaMemcpyHostToDevice, s.s_compute));
+    CU(c, cudaMemcpyAsync(buf + o_f, F.data(), 8 * (size_t)K, cudaMemcpyHostToDevice, s.s_compute));
+    if (group) CU(c, cudaMemcpyAsync(buf + o_grp, group, 4 * (size_t)n, cudaMemcpyHostToDevice, s.s_compute));
+    ScfArgs A{};
+    A.bodies = s.bodies;
+    A.group = group ? reinterpret_cast<const uint32_t *>(buf + o_grp) : nullptr;
+    A.tab = reinterpret_cast<const ScfTables *>(buf);
+    A.partial = reinterpret_cast<double *>(buf + o_part);
+    A.label = label;
+    A.n = n;
+    A.chunk = (n + n_chunks - 1) / n_chunks;
+    A.nmax = nmax;
+    A.lmax = lmax;
+    A.K = K;
+    A.cx = centre[0]; A.cy = centre[1]; A.cz = centre[2];
+    A.a = a;
+    const size_t smem = scf_coef_smem(nmax, lmax);
+    CU(c, cudaFuncSetAttribute(scf_coef_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    scf_coef_kernel<<<n_chunks, SCF_THREADS, smem, s.s_compute>>>(A);
+    c->launches++;
+    CU(c, cudaGetLastError());
+    double *dout = reinterpret_cast<double *>(buf + o_out);
+    scf_reduce_kernel<<<(2 * K + 255) / 256, 256, 0, s.s_compute>>>(A.partial, reinterpret_cast<const double *>(buf + o_f), n_chunks,
+                                                                    K, lmax, dout);
+    c->launches++;
+    CU(c, cudaGetLastError());
+    CU(c, cudaMemcpyAsync(S, dout, 8 * (size_t)K, cudaMemcpyDeviceToHost, s.s_compute));
+    CU(c, cudaMemcpyAsync(T, dout + K, 8 * (size_t)K, cudaMemcpyDeviceToHost, s.s_compute));
+    CU(c, cudaStreamSynchronize(s.s_compute));
+    return B200NB_OK;
+}
+
+int b200nb_scf_field(b200nb_ctx *c, uint32_t nmax, uint32_t lmax, double a, const double centre[3], const double *S, const double *T,
+                     uint64_t n_points, const float *px, const float *py, const float *pz, double *ax, double *ay, double *az,
+                     double *phi)
+{
+    if (!c) return B200NB_EINVAL;
+    if (int rc = scf_check(c, "scf_field", nmax, lmax, a, centre)) return rc;
+    if (!S || !T) return fail(c, B200NB_EINVAL, "scf_field: S or T is NULL");
+    if (n_points == 0) return B200NB_OK;
+    if (!px || !py || !pz) return fail(c, B200NB_EINVAL, "scf_field: NULL point array");
+    DeviceGuard guard;
+    Shard &s = c->shards[0];
+    const uint32_t K = (nmax + 1) * (lmax + 1) * (lmax + 2) / 2;
+    const uint32_t cap = (uint32_t)std::min<uint64_t>(SCF_BATCH, (n_points + 255) / 256 * 256);
+    ScfTables tab;
+    scf_tables(tab);
+    // scratch: tables | [S | T] | [4][cap] outputs | [3][cap] points
+    const size_t o_coef = round256(sizeof(ScfTables)), o_out = o_coef + round256(16 * (size_t)K), o_pts = o_out + 32 * (size_t)cap;
+    if (int rc = query_scratch(c, s, o_pts + 12 * (size_t)cap)) return rc;
+    CU(c, cudaSetDevice(s.device));
+    unsigned char *buf = s.query_buf;
+    CU(c, cudaMemcpyAsync(buf, &tab, sizeof tab, cudaMemcpyHostToDevice, s.s_compute));
+    CU(c, cudaMemcpyAsync(buf + o_coef, S, 8 * (size_t)K, cudaMemcpyHostToDevice, s.s_compute));
+    CU(c, cudaMemcpyAsync(buf + o_coef + 8 * (size_t)K, T, 8 * (size_t)K, cudaMemcpyHostToDevice, s.s_compute));
+    double *dout = reinterpret_cast<double *>(buf + o_out);
+    float *dpts = reinterpret_cast<float *>(buf + o_pts);
+    const size_t smem = scf_field_smem(K);
+    CU(c, cudaFuncSetAttribute(scf_field_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const float *pts[3] = {px, py, pz};
+    double *out[4] = {ax, ay, az, phi};
+    for (uint64_t base = 0; base < n_points; base += cap) {
+        const uint32_t cnt = (uint32_t)std::min<uint64_t>(cap, n_points - base);
+        for (int k = 0; k < 3; ++k)
+            CU(c, cudaMemcpyAsync(dpts + (size_t)k * cap, pts[k] + base, (size_t)cnt * 4, cudaMemcpyHostToDevice, s.s_compute));
+        ScfFieldArgs A{};
+        A.coef = reinterpret_cast<const double *>(buf + o_coef);
+        A.tab = reinterpret_cast<const ScfTables *>(buf);
+        A.px = dpts; A.py = dpts + cap; A.pz = dpts + 2 * (size_t)cap;
+        A.out = dout;
+        A.count = cnt; A.stride = cap; A.nmax = nmax; A.lmax = lmax; A.K = K;
+        A.cx = centre[0]; A.cy = centre[1]; A.cz = centre[2];
+        A.a = a;
+        scf_field_kernel<<<(cnt + SCF_EVAL_THREADS - 1) / SCF_EVAL_THREADS, SCF_EVAL_THREADS, smem, s.s_compute>>>(A);
+        c->launches++;
+        CU(c, cudaGetLastError());
+        for (int k = 0; k < 4; ++k)
+            if (out[k])
+                CU(c, cudaMemcpyAsync(out[k] + base, dout + (size_t)k * cap, (size_t)cnt * 8, cudaMemcpyDeviceToHost, s.s_compute));
+    }
+    CU(c, cudaStreamSynchronize(s.s_compute));
+    return B200NB_OK;
+}
 
 } // extern "C"
 
