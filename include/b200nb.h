@@ -516,6 +516,46 @@ int b200nb_scf_field(b200nb_ctx *ctx, uint32_t nmax, uint32_t lmax, double a, co
                      const double *T, uint64_t n_points, const float *px, const float *py, const float *pz,
                      double *ax, double *ay, double *az, double *phi);
 
+/* ---- frozen expansion as an external potential -------------------------------------------------------------------
+ * A host taken from a simulation (triaxial, lopsided, barred) expanded once and frozen: the satellite, stream or tracers
+ * then move in it at O(N) per step, as gala, AGAMA and galpy run orbits in simulated haloes.  A context holds at most one
+ * expansion (nmax, lmax, a, centre, S, T) next to its 0 to B200NB_EXTERNAL_MAX analytic terms, with exactly the meaning,
+ * packed layout and limits of b200nb_scf_field; its Phi_scf and a_scf at an fp32 point are bit for bit what
+ * b200nb_scf_field returns there.  With an expansion the external field is, per component, in fp64:
+ *   e = fl(e_terms + a_scf),  Phi_ext = fl(Phi_terms + Phi_scf)
+ * where e_terms and Phi_terms are the sums of the analytic terms above (+0 without terms); the expansion is added last.
+ * Everything "external potential" states for the terms holds with this e and Phi_ext: the bodies' step rounds S + e once
+ * to fp32 (MUrB at q_n, the leapfrog's a(x_0) and closing kick at x_{n+1}); the stored accelerations include it;
+ * b200nb_integrate_host_accel adds nothing; tracers take a(p) = fp32(field sums + e(p)) at the same instants;
+ * b200nb_energy and METRIC_ENERGY add sum_i m_i Phi_ext(q_i); b200nb_external_field returns the total e and Phi_ext, bit
+ * for bit what the step uses.  The field, tidal, component, neighbour, friends-of-friends, group and SCF calls keep
+ * describing the bodies' own field.
+ * b200nb_set_external_scf installs or replaces the expansion; S == NULL and T == NULL removes it (the other arguments
+ * are then ignored).  Lifecycle as b200nb_set_external: allowed before the first upload, not collective (every rank
+ * passes the same expansion), joins the devices, drops the cached step graphs and invalidates the leapfrog's stored
+ * a(x_n) and tracer a(p).  b200nb_set_external and b200nb_set_external_scf do not affect each other.
+ * Cost: one extra kernel launch per local shard for every evaluation of e (each force pass of a step, each tracer pass
+ * of a shard with tracers, each energy or metrics call).  Without an expansion, whether or not one was ever set, a
+ * context makes the same launches and step graphs, holds the same b200nb_allocated_bytes and gives bit-identical results.
+ * Device memory, per local shard, counted in b200nb_allocated_bytes and freed on removal or b200nb_destroy, with
+ * K = (nmax+1)(lmax+1)(lmax+2)/2, r(x) = x rounded up to a multiple of 256, L = b200nb_slice_length and T the tracer
+ * slots per shard of "test particles":
+ *   r(12952) + r(16 K_max)   the tables and S | T, K_max the largest K set since the expansion was last removed
+ *                            (grow-only while an expansion is set; at most 82 688 bytes);
+ *   32 L                     fp64 (ax, ay, az, Phi) of each slot of the shard's body slice;
+ *   32 T                     with tracers, fp64 (ax, ay, az, Phi) of each tracer slot, allocated by whichever of
+ *                            b200nb_set_tracers and b200nb_set_external_scf comes second and freed by either.
+ * A failed allocation leaves the context with no expansion (B200NB_ECUDA), never with half of one; one in
+ * b200nb_set_tracers leaves it with no tracers.
+ * Errors (B200NB_EINVAL; the previous expansion stays in place): nmax or lmax out of range, a not finite or <= 0, a NULL
+ * or non-finite centre, exactly one of S and T NULL, a non-finite S or T entry, a T_nl0 != 0 (b200nb_scf_coefficients
+ * always returns +0 there). */
+int b200nb_set_external_scf(b200nb_ctx *ctx, uint32_t nmax, uint32_t lmax, double a, const double centre[3],
+                            const double *S, const double *T);
+/* *present = 0 or 1; when 1, fills nmax, lmax, a, centre and S and T (packed, K entries each), each where non-NULL */
+int b200nb_get_external_scf(const b200nb_ctx *ctx, uint32_t *present, uint32_t *nmax, uint32_t *lmax, double *a,
+                            double centre[3], double *S, double *T);
+
 /* Joins every device and communication stream.  main.cpp:353-371 only synchronises the current device, so the glue
  * calls this when more than one device is in use. */
 int b200nb_sync(b200nb_ctx *ctx);

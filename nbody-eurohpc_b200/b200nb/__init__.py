@@ -163,6 +163,9 @@ def lib() -> ctypes.CDLL:
         "b200nb_external_field": (c_int, [ctx, c_uint64] + [_FP] * 3 + [_DP] * 4),
         "b200nb_scf_coefficients": (c_int, [ctx, c_uint, c_uint, c_double, _DP, _UP, c_uint, _DP, _DP]),
         "b200nb_scf_field": (c_int, [ctx, c_uint, c_uint, c_double, _DP, _DP, _DP, c_uint64] + [_FP] * 3 + [_DP] * 4),
+        "b200nb_set_external_scf": (c_int, [ctx, c_uint, c_uint, c_double, _DP, _DP, _DP]),
+        "b200nb_get_external_scf": (c_int, [ctx, POINTER(c_uint), POINTER(c_uint), POINTER(c_uint), POINTER(c_double), _DP,
+                                            _DP, _DP]),
         "b200nb_sync": (c_int, [ctx]),
         "b200nb_n_bodies": (c_uint64, [ctx]),
         "b200nb_n_local_gpus": (c_int, [ctx]),
@@ -676,6 +679,50 @@ class Context:
                                              Tp.ctypes.data_as(_DP), m, *[_p(x) for x in p],
                                              *[o.ctypes.data_as(_DP) for o in out]), "b200nb_scf_field")
         return out[0], out[1], out[2], out[3]
+
+    @staticmethod
+    def _external_scf_args(S, T, a, centre) -> tuple[int, int, float, np.ndarray, np.ndarray, np.ndarray]:
+        """(nmax, lmax, a, centre, packed S, packed T) as b200nb_set_external_scf reads them; ValueError for a bad shape,
+        nmax or lmax out of range, a or the centre (as scf_field), a non-finite entry or T[n, l, 0] != 0."""
+        if S is None or T is None:
+            raise ValueError("S and T must both be given (or both None to remove the expansion)")
+        S, T = np.asarray(S), np.asarray(T)
+        if S.ndim != 3 or S.shape != T.shape or S.shape[1] != S.shape[2] or S.dtype.kind != "f" or T.dtype.kind != "f":
+            raise ValueError(f"S and T must be float arrays of one shape (nmax+1, lmax+1, lmax+1), got {S.shape}, {T.shape}")
+        nmax, lmax, a, c = Context._scf_args(S.shape[0] - 1, S.shape[1] - 1, a, centre)
+        Sp, Tp = _scf_pack(S), _scf_pack(T)
+        if not (np.all(np.isfinite(Sp)) and np.all(np.isfinite(Tp))):
+            raise ValueError("S and T must be finite where m <= l")
+        if np.any(T[:, :, 0] != 0):
+            raise ValueError("T[n, l, 0] must be 0 (scf_coefficients returns 0 there)")
+        return nmax, lmax, a, c, Sp, Tp
+
+    def set_external_scf(self, S, T=None, a=None, centre=(0.0, 0.0, 0.0)):
+        """Installs (or replaces) a frozen basis-function expansion as part of the external potential (include/b200nb.h:
+        b200nb_set_external_scf).  S, T float64[nmax+1, lmax+1, lmax+1] as scf_coefficients returns them, scale radius a,
+        centre.  set_external_scf(None) removes it; the analytic terms of set_external are not affected."""
+        if S is None and T is None:
+            self._check(self._L.b200nb_set_external_scf(self._ctx, 0, 0, 0.0, None, None, None), "b200nb_set_external_scf")
+            return
+        nmax, lmax, a, c, Sp, Tp = self._external_scf_args(S, T, a, centre)
+        self._check(self._L.b200nb_set_external_scf(self._ctx, nmax, lmax, a, c.ctypes.data_as(_DP), Sp.ctypes.data_as(_DP),
+                                                    Tp.ctypes.data_as(_DP)), "b200nb_set_external_scf")
+
+    @property
+    def external_scf(self):
+        """None, or the expansion as set: (S, T, a, centre), S and T float64[nmax+1, lmax+1, lmax+1], centre a tuple."""
+        present, nmax, lmax, a = c_uint(), c_uint(), c_uint(), c_double()
+        c = np.zeros(3)
+        self._check(self._L.b200nb_get_external_scf(self._ctx, byref(present), byref(nmax), byref(lmax), byref(a),
+                                                    c.ctypes.data_as(_DP), None, None), "b200nb_get_external_scf")
+        if not present.value:
+            return None
+        K = (nmax.value + 1) * (lmax.value + 1) * (lmax.value + 2) // 2
+        S, T = np.empty(K), np.empty(K)
+        self._check(self._L.b200nb_get_external_scf(self._ctx, byref(present), None, None, None, None, S.ctypes.data_as(_DP),
+                                                    T.ctypes.data_as(_DP)), "b200nb_get_external_scf")
+        return (_scf_unpack(S, nmax.value, lmax.value), _scf_unpack(T, nmax.value, lmax.value), a.value,
+                tuple(float(x) for x in c))
 
     def sync(self):
         self._check(self._L.b200nb_sync(self._ctx), "b200nb_sync")

@@ -176,6 +176,11 @@ struct Shard {
     float *tr = nullptr, *tr_part = nullptr;
     uint32_t tr_local = 0;
     uint64_t tr_bytes = 0;
+    // the external expansion (b200nb_set_external_scf): ext_coef = tables | [S | T] (grow-only, ext_coef_bytes), and the
+    // [4][L] and [4][tr_T] fp64 rows (ax, ay, az, phi) ext_total_kernel writes for the slice and the tracers before use
+    unsigned char *ext_coef = nullptr;
+    uint64_t ext_coef_bytes = 0;
+    double *ext_body = nullptr, *ext_tr = nullptr;
     ncclComm_t comm = nullptr;
     CUmodule resched_mod = nullptr;   // the re-ordered cubin of the default variant on this device (nullptr: not in use)
     CUfunction resched_fn = nullptr;
@@ -227,6 +232,13 @@ struct b200nb_ctx {
     uint32_t tr_cap = 0;
     bool tr_acc_valid = false;
     ExtTerms ext{}; // the external potential (b200nb_set_external); ext.n == 0: none
+    // the external expansion (b200nb_set_external_scf) as set, for b200nb_get_external_scf; on == false: none
+    struct {
+        bool on = false;
+        uint32_t nmax = 0, lmax = 0, K = 0;
+        double a = 0.0, centre[3] = {};
+        std::vector<double> coef; // [S | T], K each
+    } scf;
     uint64_t launches = 0;
     std::string err;
 };
@@ -713,9 +725,36 @@ int enqueue_force(b200nb_ctx *c)
     return B200NB_OK;
 }
 
+size_t round256(size_t x) { return (x + 255) / 256 * 256; }
+
+// ext_total_kernel over `count` points of `pts` into out = [4][stride], on the shard's compute stream: one launch
+template <class Points>
+int enqueue_ext_total(b200nb_ctx *c, Shard &s, const Points &pts, uint32_t count, uint32_t stride, double *out)
+{
+    ExtScf E{};
+    E.tab = reinterpret_cast<const ScfTables *>(s.ext_coef);
+    E.coef = reinterpret_cast<const double *>(s.ext_coef + round256(sizeof(ScfTables)));
+    E.nmax = c->scf.nmax; E.lmax = c->scf.lmax; E.K = c->scf.K;
+    E.cx = c->scf.centre[0]; E.cy = c->scf.centre[1]; E.cz = c->scf.centre[2];
+    E.a = c->scf.a;
+    ext_total_kernel<Points><<<(count + SCF_EVAL_THREADS - 1) / SCF_EVAL_THREADS, SCF_EVAL_THREADS, scf_field_smem(E.K), s.s_compute>>>(
+        c->ext, E, pts, count, stride, out);
+    c->launches++;
+    CU(c, cudaGetLastError());
+    return B200NB_OK;
+}
+
+// the total external field at the shard's own bodies, into s.ext_body (the current positions of `bodies`)
+int enqueue_ext_total_bodies(b200nb_ctx *c, Shard &s)
+{
+    return enqueue_ext_total(c, s, BlockedPoints{s.bodies, (uint64_t)s.rank * c->L}, s.n_local, (uint32_t)c->L, s.ext_body);
+}
+
 int enqueue_integrate(b200nb_ctx *c, int mode, float dt)
 {
     const bool moves = mode == IM_MURB || mode == IM_MURB_STORED || mode == IM_LF_KICK_DRIFT;
+    // the modes that sum partial rows add e: with an expansion it is evaluated by one ext_total_kernel launch first
+    const bool field = c->scf.on && (mode == IM_MURB || mode == IM_REDUCE_ONLY || mode == IM_LF_KICK);
     const bool push = c->p2p && moves;
     for (auto &s : c->shards) {
         CU(c, cudaSetDevice(s.device));
@@ -743,10 +782,14 @@ int enqueue_integrate(b200nb_ctx *c, int mode, float dt)
             a.sk[1] = SkRows{(uint64_t)n_itiles * nbr, c->sk_grid, nbr, c->sk_rows_own};
         }
         // caller-supplied accelerations (IM_MURB_STORED) already are the whole acceleration: no terms added
-        if (c->ext.n > 0 && mode != IM_MURB_STORED)
-            integrate_kernel<true><<<(s.n_local + 255) / 256, 256, 0, s.s_compute>>>(a, c->ext);
-        else
-            integrate_kernel<false><<<(s.n_local + 255) / 256, 256, 0, s.s_compute>>>(a, c->ext);
+        if (field) {
+            if (int rc = enqueue_ext_total_bodies(c, s)) return rc;
+            integrate_kernel<true, true><<<(s.n_local + 255) / 256, 256, 0, s.s_compute>>>(a, c->ext, s.ext_body);
+        } else if (c->ext.n > 0 && mode != IM_MURB_STORED) {
+            integrate_kernel<true><<<(s.n_local + 255) / 256, 256, 0, s.s_compute>>>(a, c->ext, nullptr);
+        } else {
+            integrate_kernel<false><<<(s.n_local + 255) / 256, 256, 0, s.s_compute>>>(a, c->ext, nullptr);
+        }
         c->launches++;
         CU(c, cudaGetLastError());
     }
@@ -947,9 +990,55 @@ void nb_launch(bool self, const NbArgs &a, uint32_t k, uint32_t *idx, float *dis
 // Device bytes of one shard's tracer set (include/b200nb.h states the same formula)
 uint64_t tracer_bytes(uint64_t T, uint32_t cap, uint32_t S) { return 36 * T + 16 * (uint64_t)S * cap; }
 
+// the expansion's [4][tr_T] tracer rows of every shard (callers have joined the streams)
+void free_ext_tracers(b200nb_ctx *c)
+{
+    for (auto &s : c->shards) {
+        if (!s.ext_tr) continue;
+        cudaSetDevice(s.device);
+        cudaFree(s.ext_tr);
+        s.ext_tr = nullptr;
+        s.bytes -= 32 * c->tr_T;
+    }
+}
+
+// with an expansion and tracers: the [4][tr_T] tracer rows of every shard that lacks them
+cudaError_t alloc_ext_tracers(b200nb_ctx *c)
+{
+    for (auto &s : c->shards) {
+        if (s.ext_tr) continue;
+        cudaError_t e = cudaSetDevice(s.device);
+        if (e == cudaSuccess) e = cudaMalloc((void **)&s.ext_tr, 32 * c->tr_T);
+        if (e != cudaSuccess) { s.ext_tr = nullptr; (void)cudaGetLastError(); return e; }
+        s.bytes += 32 * c->tr_T;
+    }
+    return cudaSuccess;
+}
+
+// the context holds no expansion afterwards (callers have joined the streams)
+void free_ext_scf(b200nb_ctx *c)
+{
+    free_ext_tracers(c);
+    for (auto &s : c->shards) {
+        if (s.ext_coef || s.ext_body) {
+            cudaSetDevice(s.device);
+            cudaFree(s.ext_coef);
+            cudaFree(s.ext_body);
+        }
+        if (s.ext_body) s.bytes -= 32 * c->L;
+        s.bytes -= s.ext_coef_bytes;
+        s.ext_coef = nullptr;
+        s.ext_body = nullptr;
+        s.ext_coef_bytes = 0;
+    }
+    c->scf.on = false;
+    c->scf.coef.clear();
+}
+
 // the context holds no tracers afterwards (callers have joined the streams)
 void free_tracers(b200nb_ctx *c)
 {
+    free_ext_tracers(c);
     for (auto &s : c->shards) {
         if (s.tr || s.tr_part) {
             cudaSetDevice(s.device);
@@ -977,6 +1066,10 @@ int enqueue_tracer_pass(b200nb_ctx *c, int mode, float dt)
         CU(c, cudaSetDevice(s.device));
         if (c->n_ranks > 1)
             if (int rc = wait_remote_positions(c, s)) return rc;
+        if (c->scf.on) // the total external field at every tracer of the shard, before any batch moves one
+            if (int rc = enqueue_ext_total(c, s, SoaPoints{s.tr, s.tr + c->tr_T, s.tr + 2 * c->tr_T}, s.tr_local,
+                                           (uint32_t)c->tr_T, s.ext_tr))
+                return rc;
         for (uint32_t base = 0; base < s.tr_local; base += c->tr_cap) {
             const uint32_t cnt = std::min(c->tr_cap, s.tr_local - base);
             FieldArgs a{};
@@ -992,10 +1085,12 @@ int enqueue_tracer_pass(b200nb_ctx *c, int mode, float dt)
             TracerArgs u{};
             u.partial = s.tr_part; u.n_chunks = S; u.stride = c->tr_cap; u.count = cnt;
             u.tr = s.tr + base; u.T = c->tr_T; u.dt = dt; u.mode = mode;
-            if (c->ext.n > 0)
-                tracer_update_kernel<true><<<(cnt + 255) / 256, 256, 0, s.s_compute>>>(u, c->ext);
+            if (c->scf.on)
+                tracer_update_kernel<true, true><<<(cnt + 255) / 256, 256, 0, s.s_compute>>>(u, c->ext, s.ext_tr + base);
+            else if (c->ext.n > 0)
+                tracer_update_kernel<true><<<(cnt + 255) / 256, 256, 0, s.s_compute>>>(u, c->ext, nullptr);
             else
-                tracer_update_kernel<false><<<(cnt + 255) / 256, 256, 0, s.s_compute>>>(u, c->ext);
+                tracer_update_kernel<false><<<(cnt + 255) / 256, 256, 0, s.s_compute>>>(u, c->ext, nullptr);
             c->launches += 2;
             CU(c, cudaGetLastError());
         }
@@ -1097,6 +1192,7 @@ void b200nb_destroy(b200nb_ctx *c)
         cudaFree(s.bodies); cudaFree(s.bodies_next); cudaFree(s.vel); cudaFree(s.acc); cudaFree(s.mass); cudaFree(s.partial); cudaFree(s.stage); cudaFree(s.stage_full);
         cudaFree(s.energy_blocks); cudaFree(s.energy_out); cudaFree(s.l2_scratch); cudaFree(s.query_buf);
         cudaFree(s.tr); cudaFree(s.tr_part);
+        cudaFree(s.ext_coef); cudaFree(s.ext_body); cudaFree(s.ext_tr);
         for (auto t : s.timer) if (t) cudaEventDestroy(t);
         if (s.ev_integrated) cudaEventDestroy(s.ev_integrated);
         if (s.ev_gathered) cudaEventDestroy(s.ev_gathered);
@@ -1402,10 +1498,12 @@ static int metric_sums(b200nb_ctx *c, double *raw)
         const uint32_t nb = (s.n_local + ENERGY_THREADS - 1) / ENERGY_THREADS;
         double part[MR_COUNT];
         if (nb > 0) {
-            auto energy = c->ext.n > 0 ? energy_kernel<true> : energy_kernel<false>;
+            if (c->scf.on)
+                if (int rc = enqueue_ext_total_bodies(c, s)) return rc;
+            auto energy = c->scf.on ? energy_kernel<true, true> : c->ext.n > 0 ? energy_kernel<true> : energy_kernel<false>;
             energy<<<nb, ENERGY_THREADS, 0, s.s_compute>>>(s.bodies, s.vel, s.mass, (uint32_t)c->L, s.n_local,
                                                           (uint64_t)s.rank * c->L, c->nblk_total, c->soft2,
-                                                          s.energy_blocks, c->ext);
+                                                          s.energy_blocks, c->ext, s.ext_body);
             energy_final_kernel<<<MR_COUNT, 256, 0, s.s_compute>>>(s.energy_blocks, nb, s.energy_out);
             c->launches += 2;
             CU(c, cudaGetLastError());
@@ -1991,6 +2089,13 @@ int b200nb_set_tracers(b200nb_ctx *c, uint64_t n_tracers, const float *qx, const
     c->m_tracers = n_tracers;
     c->tr_T = T;
     c->tr_cap = cap;
+    if (c->scf.on) { // the expansion's tracer rows; without them, no tracers at all
+        const cudaError_t e = alloc_ext_tracers(c);
+        if (e != cudaSuccess) {
+            free_tracers(c);
+            return fail(c, B200NB_ECUDA, "set_tracers: %s", cudaGetErrorString(e));
+        }
+    }
     return B200NB_OK;
 }
 
@@ -2069,10 +2174,14 @@ int b200nb_external_field(b200nb_ctx *c, uint64_t n_points, const float *px, con
         const uint32_t cnt = (uint32_t)std::min<uint64_t>(cap, n_points - base);
         for (int k = 0; k < 3; ++k)
             CU(c, cudaMemcpyAsync(dpts + (size_t)k * cap, pts[k] + base, (size_t)cnt * 4, cudaMemcpyHostToDevice, s.s_compute));
-        external_field_kernel<<<(cnt + 255) / 256, 256, 0, s.s_compute>>>(c->ext, dpts, dpts + cap, dpts + 2 * (size_t)cap,
-                                                                          cnt, cap, dout);
-        c->launches++;
-        CU(c, cudaGetLastError());
+        if (c->scf.on) {
+            if (int rc = enqueue_ext_total(c, s, SoaPoints{dpts, dpts + cap, dpts + 2 * (size_t)cap}, cnt, cap, dout)) return rc;
+        } else {
+            external_field_kernel<<<(cnt + 255) / 256, 256, 0, s.s_compute>>>(c->ext, dpts, dpts + cap, dpts + 2 * (size_t)cap,
+                                                                              cnt, cap, dout);
+            c->launches++;
+            CU(c, cudaGetLastError());
+        }
         for (int k = 0; k < 4; ++k)
             if (out[k])
                 CU(c, cudaMemcpyAsync(out[k] + base, dout + (size_t)k * cap, (size_t)cnt * 8, cudaMemcpyDeviceToHost, s.s_compute));
@@ -2129,8 +2238,6 @@ uint64_t b200nb_n_tracers(const b200nb_ctx *c) { return c ? c->m_tracers : 0; }
 
 // ------------------------------------------------------------------------------------------------ basis-function expansion
 namespace {
-
-size_t round256(size_t x) { return (x + 255) / 256 * 256; }
 
 // The recurrence tables of scf_sm100.cuh, in long double, each entry rounded once.
 void scf_tables(ScfTables &t)
@@ -2293,6 +2400,99 @@ int b200nb_scf_field(b200nb_ctx *c, uint32_t nmax, uint32_t lmax, double a, cons
                 CU(c, cudaMemcpyAsync(out[k] + base, dout + (size_t)k * cap, (size_t)cnt * 8, cudaMemcpyDeviceToHost, s.s_compute));
     }
     CU(c, cudaStreamSynchronize(s.s_compute));
+    return B200NB_OK;
+}
+
+// ------------------------------------------------------------------------------------------------ external expansion
+int b200nb_set_external_scf(b200nb_ctx *c, uint32_t nmax, uint32_t lmax, double a, const double centre[3], const double *S,
+                            const double *T)
+{
+    if (!c) return B200NB_EINVAL;
+    const bool remove = !S && !T;
+    uint32_t K = 0;
+    if (!remove) {
+        if (!S || !T) return fail(c, B200NB_EINVAL, "set_external_scf: one of S and T is NULL");
+        if (int rc = scf_check(c, "set_external_scf", nmax, lmax, a, centre)) return rc;
+        const uint32_t LM = (lmax + 1) * (lmax + 2) / 2;
+        K = (nmax + 1) * LM;
+        for (uint32_t k = 0; k < K; ++k)
+            if (!std::isfinite(S[k]) || !std::isfinite(T[k]))
+                return fail(c, B200NB_EINVAL, "set_external_scf: non-finite S or T entry at packed index %u", k);
+        for (uint32_t n = 0; n <= nmax; ++n)
+            for (uint32_t l = 0; l <= lmax; ++l)
+                if (T[n * LM + l * (l + 1) / 2] != 0.0)
+                    return fail(c, B200NB_EINVAL, "set_external_scf: T[n=%u, l=%u, m=0] = %g must be 0", n, l,
+                                T[n * LM + l * (l + 1) / 2]);
+    }
+    DeviceGuard guard;
+    // steps in flight read the old coefficients, and captured step graphs bake in their buffers
+    if (int rc = sync_all(c)) return rc;
+    for (auto &g : c->graphs)
+        if (g.exec) cudaGraphExecDestroy(g.exec);
+    c->graphs.clear();
+    c->acc_valid = false; // the leapfrog's a(x_n) and a(p) were taken in the old field
+    c->tr_acc_valid = false;
+    if (remove) {
+        free_ext_scf(c);
+        return B200NB_OK;
+    }
+    ScfTables tab;
+    scf_tables(tab);
+    const size_t o_coef = round256(sizeof(ScfTables)), need = o_coef + round256(16 * (size_t)K);
+    const int smem_max = (int)scf_field_smem((SCF_NMAX + 1) * (SCF_LMAX + 1) * (SCF_LMAX + 2) / 2);
+    for (auto &s : c->shards) {
+        cudaError_t e = cudaSetDevice(s.device);
+        if (e == cudaSuccess && s.ext_coef_bytes < need) { // grow-only
+            cudaFree(s.ext_coef);
+            s.bytes -= s.ext_coef_bytes;
+            s.ext_coef = nullptr;
+            s.ext_coef_bytes = 0;
+            e = cudaMalloc((void **)&s.ext_coef, need);
+            if (e == cudaSuccess) { s.ext_coef_bytes = need; s.bytes += need; } else s.ext_coef = nullptr;
+        }
+        if (e == cudaSuccess && !s.ext_body) {
+            e = cudaMalloc((void **)&s.ext_body, 32 * c->L);
+            if (e == cudaSuccess) s.bytes += 32 * c->L; else s.ext_body = nullptr;
+        }
+        if (e == cudaSuccess)
+            e = cudaFuncSetAttribute(ext_total_kernel<BlockedPoints>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
+        if (e == cudaSuccess)
+            e = cudaFuncSetAttribute(ext_total_kernel<SoaPoints>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(s.ext_coef, &tab, sizeof tab, cudaMemcpyHostToDevice, s.s_compute);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(s.ext_coef + o_coef, S, 8 * (size_t)K, cudaMemcpyHostToDevice, s.s_compute);
+        if (e == cudaSuccess)
+            e = cudaMemcpyAsync(s.ext_coef + o_coef + 8 * (size_t)K, T, 8 * (size_t)K, cudaMemcpyHostToDevice, s.s_compute);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(s.s_compute); // S and T are borrowed for the call
+        if (e == cudaSuccess && c->m_tracers > 0) e = alloc_ext_tracers(c);
+        if (e != cudaSuccess) { // never half set: no expansion at all
+            (void)cudaGetLastError();
+            sync_all(c);
+            free_ext_scf(c);
+            return fail(c, B200NB_ECUDA, "set_external_scf: %s", cudaGetErrorString(e));
+        }
+    }
+    c->scf.on = true;
+    c->scf.nmax = nmax; c->scf.lmax = lmax; c->scf.K = K;
+    c->scf.a = a;
+    for (int k = 0; k < 3; ++k) c->scf.centre[k] = centre[k];
+    c->scf.coef.assign(S, S + K);
+    c->scf.coef.insert(c->scf.coef.end(), T, T + K);
+    return B200NB_OK;
+}
+
+int b200nb_get_external_scf(const b200nb_ctx *c, uint32_t *present, uint32_t *nmax, uint32_t *lmax, double *a, double centre[3],
+                            double *S, double *T)
+{
+    if (!c || !present) return B200NB_EINVAL;
+    *present = c->scf.on ? 1u : 0u;
+    if (!c->scf.on) return B200NB_OK;
+    const uint32_t K = c->scf.K;
+    if (nmax) *nmax = c->scf.nmax;
+    if (lmax) *lmax = c->scf.lmax;
+    if (a) *a = c->scf.a;
+    if (centre) for (int k = 0; k < 3; ++k) centre[k] = c->scf.centre[k];
+    if (S) memcpy(S, c->scf.coef.data(), 8 * (size_t)K);
+    if (T) memcpy(T, c->scf.coef.data() + K, 8 * (size_t)K);
     return B200NB_OK;
 }
 

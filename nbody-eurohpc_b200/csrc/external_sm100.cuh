@@ -2,6 +2,8 @@
 //
 // Every kernel that applies the terms (integrate_kernel, tracer_update_kernel, energy_kernel, external_field_kernel)
 // calls ext_eval, so the e and Phi_ext a step uses at an fp32 point are exactly what b200nb_external_field returns there.
+// With a frozen expansion (b200nb_set_external_scf) ext_total_kernel below adds scf_eval's field to ext_eval's, and the
+// <true, true> forms of those kernels read its output instead of calling ext_eval.
 // The terms travel by value as a __grid_constant__ kernel parameter: no device memory, and a captured step graph bakes
 // them in like any other argument (b200nb_set_external drops the cached graphs).
 //
@@ -27,6 +29,7 @@
 #include <cstddef>
 #include <cstdint>
 #include "../../include/b200nb.h"
+#include "scf_sm100.cuh"
 
 static_assert(sizeof(b200nb_external_term) == 56, "b200nb_external_term is 56 bytes");
 static_assert(offsetof(b200nb_external_term, gm) == 8 && offsetof(b200nb_external_term, a) == 16 &&
@@ -120,6 +123,66 @@ __global__ void __launch_bounds__(256) external_field_kernel(const __grid_consta
     double a[3], phi;
     ext_eval(e, px[i], py[i], pz[i], a, &phi);
     out[i] = a[0]; out[stride + i] = a[1]; out[2 * (size_t)stride + i] = a[2]; out[3 * (size_t)stride + i] = phi;
+}
+
+// ---------------------------------------------------------------------------------------------- external expansion
+// The context's frozen basis-function expansion (b200nb_set_external_scf) on the device: the tables and [S | T] packed
+// as b200nb_scf_field reads them, in the shard's coefficient block.
+struct ExtScf {
+    const ScfTables *tab;
+    const double *coef;
+    uint32_t nmax, lmax, K;
+    double cx, cy, cz, a;
+};
+
+// Point loaders of ext_total_kernel: bodies [first, first + count) of the blocked body array, or SoA coordinate arrays.
+struct BlockedPoints {
+    const float *bodies;
+    uint64_t first;
+    __device__ __forceinline__ void operator()(uint32_t i, float &x, float &y, float &z) const
+    {
+        const uint64_t g = first + i; // AoSoA-128: x | y | z | G*m per block of 128 bodies
+        const float *b = bodies + g / 128 * 512 + g % 128;
+        x = b[0]; y = b[128]; z = b[256];
+    }
+};
+struct SoaPoints {
+    const float *px, *py, *pz;
+    __device__ __forceinline__ void operator()(uint32_t i, float &x, float &y, float &z) const
+    {
+        x = px[i]; y = py[i]; z = pz[i];
+    }
+};
+
+// The total external field with an expansion: e = fl(e_terms + a_scf), Phi_ext = fl(Phi_terms + Phi_scf), per component,
+// e_terms and Phi_terms from ext_eval (+0 without terms), a_scf and Phi_scf from scf_eval.  out = [4][stride] doubles
+// (ax, ay, az, phi), read by b200nb_external_field and by the <true, true> forms of the step's consumers.  The tables
+// and [S | T] are staged in shared memory as scf_field_kernel stages them: scf_field_smem(K) bytes.
+template <class Points>
+__global__ void __launch_bounds__(SCF_EVAL_THREADS) ext_total_kernel(const __grid_constant__ ExtTerms ext, const ExtScf E,
+                                                                     const Points pts, uint32_t count, uint32_t stride,
+                                                                     double *__restrict__ out)
+{
+    extern __shared__ double smem[];
+    ScfTables &tab = *reinterpret_cast<ScfTables *>(smem);
+    double *S = smem + sizeof(ScfTables) / sizeof(double), *T = S + E.K;
+    {
+        const double *src = reinterpret_cast<const double *>(E.tab);
+        for (uint32_t e = threadIdx.x; e < sizeof(ScfTables) / sizeof(double); e += blockDim.x) smem[e] = src[e];
+        for (uint32_t e = threadIdx.x; e < 2 * E.K; e += blockDim.x) S[e] = E.coef[e];
+    }
+    __syncthreads();
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= count) return;
+    float x, y, z;
+    pts(i, x, y, z);
+    double e[3], phi, s[3], sphi;
+    ext_eval(ext, x, y, z, e, &phi);
+    scf_eval(tab, S, T, E, x, y, z, s, &sphi);
+    out[i] = __dadd_rn(e[0], s[0]);
+    out[stride + i] = __dadd_rn(e[1], s[1]);
+    out[2 * (size_t)stride + i] = __dadd_rn(e[2], s[2]);
+    out[3 * (size_t)stride + i] = __dadd_rn(phi, sphi);
 }
 
 } // namespace b200nb

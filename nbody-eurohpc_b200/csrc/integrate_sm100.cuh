@@ -52,9 +52,12 @@ struct IntegrateArgs {
 };
 
 // EXT: the fp64 sum is rounded together with the external acceleration at the body's current position (include/b200nb.h,
-// "external potential"); <false> ignores `ext` and is the kernel without terms.
-template <bool EXT>
-__global__ void __launch_bounds__(256) integrate_kernel(const IntegrateArgs a, const __grid_constant__ ExtTerms ext)
+// "external potential"); <false> ignores `ext` and `ef` and is the kernel without terms.  FIELD (with an expansion):
+// e is read from ef = [4][L], the total external field ext_total_kernel has just written for the slice, instead of
+// evaluated from `ext`; it is added at the same place.
+template <bool EXT, bool FIELD = false>
+__global__ void __launch_bounds__(256) integrate_kernel(const IntegrateArgs a, const __grid_constant__ ExtTerms ext,
+                                                        const double *__restrict__ ef)
 {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= a.n_local) return;
@@ -85,9 +88,14 @@ __global__ void __launch_bounds__(256) integrate_kernel(const IntegrateArgs a, c
             }
         }
         if constexpr (EXT) {
-            const size_t g = a.first + i;
-            double e[3], phi;
-            ext_eval(ext, a.bodies[blk_index(g, 0)], a.bodies[blk_index(g, 1)], a.bodies[blk_index(g, 2)], e, &phi);
+            double e[3];
+            if constexpr (FIELD) {
+                e[0] = ef[i]; e[1] = ef[L + i]; e[2] = ef[2 * L + i];
+            } else {
+                const size_t g = a.first + i;
+                double phi;
+                ext_eval(ext, a.bodies[blk_index(g, 0)], a.bodies[blk_index(g, 1)], a.bodies[blk_index(g, 2)], e, &phi);
+            }
             sx = __dadd_rn(sx, e[0]); sy = __dadd_rn(sy, e[1]); sz = __dadd_rn(sz, e[2]);
         }
         ax = (float)sx; ay = (float)sy; az = (float)sz;
@@ -200,14 +208,16 @@ __device__ __forceinline__ float rsqrt_nr(float d)
     return y * fmaf(-0.5f * d, y * y, 1.5f);
 }
 
-// block_out[row * n_blocks + block].  EXT: the energy row adds m_i Phi_ext(q_i); <false> ignores `ext`.
-template <bool EXT>
+// block_out[row * n_blocks + block].  EXT: the energy row adds m_i Phi_ext(q_i); <false> ignores `ext` and `ef`.
+// FIELD: Phi_ext is row 3 of ef = [4][L], written by ext_total_kernel for the slice (see integrate_kernel).
+template <bool EXT, bool FIELD = false>
 __global__ void __launch_bounds__(ENERGY_THREADS) energy_kernel(const float *__restrict__ bodies,
                                                                 const float *__restrict__ vel,
                                                                 const float *__restrict__ mass, uint32_t L,
                                                                 uint32_t n_local, uint64_t first, uint32_t nblk_total,
                                                                 float soft2, double *__restrict__ block_out,
-                                                                const __grid_constant__ ExtTerms ext)
+                                                                const __grid_constant__ ExtTerms ext,
+                                                                const double *__restrict__ ef)
 {
     __shared__ __align__(16) float tile[BLK_FLOATS];
     __shared__ double warp_sums[MR_COUNT][ENERGY_THREADS / 32];
@@ -244,8 +254,13 @@ __global__ void __launch_bounds__(ENERGY_THREADS) energy_kernel(const float *__r
         const double w = m * (pot - self);
         r[MR_ENERGY] = 0.5 * m * v2 - 0.5 * w;
         if constexpr (EXT) {
-            double e[3], phi;
-            ext_eval(ext, xi, yi, zi, e, &phi);
+            double phi;
+            if constexpr (FIELD) {
+                phi = ef[3 * (size_t)L + i];
+            } else {
+                double e[3];
+                ext_eval(ext, xi, yi, zi, e, &phi);
+            }
             r[MR_ENERGY] = __dadd_rn(r[MR_ENERGY], __dmul_rn(m, phi));
         }
         r[MR_LX] = m * (y * vz - z * vy);

@@ -21,7 +21,8 @@
 // F_nlm = (2 - delta_m0) A~_nl N_lm / a from the host.  Hence the "sub-block" promise: (nmax', lmax') <= (nmax, lmax) gives
 // the matching entries bit for bit.
 //
-// Evaluation (scf_field_kernel): one thread per point, S, T and the tables in shared memory.  For each m it runs the l
+// Evaluation (scf_eval, called by scf_field_kernel and by external_sm100.cuh's ext_total_kernel): one thread per point,
+// S, T and the tables in shared memory.  For each m it runs the l
 // recurrences of Q_l^m and Q_l^(m+1), for each (l, m) the n recurrence of C_n and of dC_n/dxi (the recurrence
 // differentiated), and dots them with S and T.  The gradient is assembled in Cartesian form:
 //   grad Phi = (dPhi/ds / a) u + (V - u (u . V)) / r,  u = d / r,
@@ -241,20 +242,17 @@ struct ScfFieldArgs {
     double cx, cy, cz, a;
 };
 
-__global__ void __launch_bounds__(SCF_EVAL_THREADS) scf_field_kernel(const ScfFieldArgs A)
+// Phi and a = -grad Phi of the expansion (S, T packed, tab the tables) at the fp32 point p: the one evaluator of
+// b200nb_scf_field and of the step's external expansion (ext_total_kernel), so both give the same bits at a point.
+// E is the kernel's argument struct (nmax, lmax, a, cx, cy, cz), read where the arithmetic uses it as scf_field_kernel
+// always did.  Where ptxas would be free to fuse either product of a two-product sum and has been seen to choose
+// differently between callers, the operation is written out: those are the choices scf_field_kernel compiled to
+// before scf_eval existed, so b200nb_scf_field keeps its bits.
+template <class E>
+__device__ __forceinline__ void scf_eval(const ScfTables &tab, const double *S, const double *T, const E &A, float px, float py,
+                                         float pz, double acc[3], double *phi_out)
 {
-    extern __shared__ double smem[];
-    ScfTables &tab = *reinterpret_cast<ScfTables *>(smem);
-    double *S = smem + sizeof(ScfTables) / sizeof(double), *T = S + A.K;
-    {
-        const double *src = reinterpret_cast<const double *>(A.tab);
-        for (uint32_t e = threadIdx.x; e < sizeof(ScfTables) / sizeof(double); e += blockDim.x) smem[e] = src[e];
-        for (uint32_t e = threadIdx.x; e < 2 * A.K; e += blockDim.x) S[e] = A.coef[e];
-    }
-    __syncthreads();
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= A.count) return;
-    const ScfGeom g = scf_geom(A.px[i], A.py[i], A.pz[i], A.cx, A.cy, A.cz, A.a);
+    const ScfGeom g = scf_geom(px, py, pz, A.cx, A.cy, A.cz, A.a);
     const uint32_t L1 = A.lmax + 1, LM = L1 * (L1 + 1) / 2;
     const double q = 1.0 / (1.0 + g.s), t = g.s * q * q, dxi = 2.0 * q * q; // dxi / ds
     double phi = 0.0, gs = 0.0, vx = 0.0, vy = 0.0, vz = 0.0;
@@ -298,8 +296,8 @@ __global__ void __launch_bounds__(SCF_EVAL_THREADS) scf_field_kernel(const ScfFi
             vz -= qb * (rs * cm + rt * sm);
         }
         cm1 = cm; sm1 = sm;
-        const double c2 = cm * g.wr - sm * g.wi;
-        sm = cm * g.wi + sm * g.wr;
+        const double c2 = __fma_rn(cm, g.wr, -__dmul_rn(sm, g.wi));
+        sm = __fma_rn(sm, g.wr, __dmul_rn(cm, g.wi));
         cm = c2;
         Pm *= t;
     }
@@ -310,7 +308,26 @@ __global__ void __launch_bounds__(SCF_EVAL_THREADS) scf_field_kernel(const ScfFi
         ay = -(k * g.wi + (vy - g.wi * uv) / g.r);
         az = -(k * g.x + (vz - g.x * uv) / g.r);
     }
-    A.out[i] = ax; A.out[A.stride + i] = ay; A.out[2 * (size_t)A.stride + i] = az; A.out[3 * (size_t)A.stride + i] = phi;
+    acc[0] = ax; acc[1] = ay; acc[2] = az;
+    *phi_out = phi;
+}
+
+__global__ void __launch_bounds__(SCF_EVAL_THREADS) scf_field_kernel(const ScfFieldArgs A)
+{
+    extern __shared__ double smem[];
+    ScfTables &tab = *reinterpret_cast<ScfTables *>(smem);
+    double *S = smem + sizeof(ScfTables) / sizeof(double), *T = S + A.K;
+    {
+        const double *src = reinterpret_cast<const double *>(A.tab);
+        for (uint32_t e = threadIdx.x; e < sizeof(ScfTables) / sizeof(double); e += blockDim.x) smem[e] = src[e];
+        for (uint32_t e = threadIdx.x; e < 2 * A.K; e += blockDim.x) S[e] = A.coef[e];
+    }
+    __syncthreads();
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= A.count) return;
+    double acc[3], phi;
+    scf_eval(tab, S, T, A, A.px[i], A.py[i], A.pz[i], acc, &phi);
+    A.out[i] = acc[0]; A.out[A.stride + i] = acc[1]; A.out[2 * (size_t)A.stride + i] = acc[2]; A.out[3 * (size_t)A.stride + i] = phi;
 }
 
 } // namespace b200nb

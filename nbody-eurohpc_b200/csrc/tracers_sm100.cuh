@@ -33,16 +33,24 @@ struct TracerArgs {
 
 // after each field_kernel batch: fixed-order fp64 sum, rounded once, then the update.  EXT: the sum is rounded together
 // with the external acceleration at the tracer's current position, as integrate_kernel<true> does for the bodies.
-template <bool EXT>
-__global__ void __launch_bounds__(256) tracer_update_kernel(const TracerArgs a, const __grid_constant__ ExtTerms ext)
+// FIELD (with an expansion): e is read from ef = [4][T] rows starting at the batch's first tracer, written by
+// ext_total_kernel for the shard's tracers before the pass, instead of evaluated from `ext`.
+template <bool EXT, bool FIELD = false>
+__global__ void __launch_bounds__(256) tracer_update_kernel(const TracerArgs a, const __grid_constant__ ExtTerms ext,
+                                                            const double *__restrict__ ef)
 {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= a.count) return;
     double s[3];
     field_sum_rows<3>(a.partial, a.n_chunks, a.stride, i, s);
     if constexpr (EXT) {
-        double e[3], phi;
-        ext_eval(ext, a.tr[i], a.tr[a.T + i], a.tr[2 * a.T + i], e, &phi);
+        double e[3];
+        if constexpr (FIELD) {
+            e[0] = ef[i]; e[1] = ef[a.T + i]; e[2] = ef[2 * a.T + i];
+        } else {
+            double phi;
+            ext_eval(ext, a.tr[i], a.tr[a.T + i], a.tr[2 * a.T + i], e, &phi);
+        }
         s[0] = __dadd_rn(s[0], e[0]); s[1] = __dadd_rn(s[1], e[1]); s[2] = __dadd_rn(s[2], e[2]);
     }
     const float ax = (float)s[0], ay = (float)s[1], az = (float)s[2];
